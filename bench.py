@@ -2,6 +2,7 @@
 """bench.py -- SAC updates/s at BipedalWalker shape (BASELINE.json configs[1]) on N B200s.
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload bipedal|population|donkey|dp] [--no-extras]
+                    [--dump-outputs DIR]
 
 A "step" is one full SAC gradient update (ring gather + target + 2 critic steps + actor step + temperature step
 + Polyak; reference: SAC.training_step, sac/agent.py:302-327) on synthetic transitions (SURVEY section 8d).
@@ -18,13 +19,17 @@ The two modes that DO shard ride along in `extra` of the same line (default work
 1024 InvertedPendulum-shape agents with 100000-row rings partitioned over the ranks, no collective -- and `extra.dp` --
 BipedalWalker shape at global batch 65536 split over the ranks, two NCCL all-reduces per update, with the in-run checks
 that the replicas stay bit-identical and within 2e-5 of the single-rank result, and the all-reduce share of the update.
-Timing: W warm-up steps, then >= 5 repeats of exactly K steps (until >= 0.5 s are timed); the median repeat is reported.
+Timing: W warm-up steps, then exactly K timed steps in up to 5 repeats of near-equal length; the median repeat's time per
+step is reported.
+--dump-outputs DIR: after the timed steps, what the timed path computed in its last step goes to DIR/<name>.npy (see
+dump_outputs). The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
 import json
 import os
+import re
 import subprocess
 import sys
 import threading
@@ -273,20 +278,20 @@ class Runner:
         return steps * self.world                                    # replicas: one independent agent per rank
 
 
-def timed(runner, steps, warmup, barrier, dist, world, min_seconds=0.5, min_repeats=5, max_repeats=200):
-    """W warm-up steps, then R >= 5 repeats of EXACTLY `steps` steps (until >= 0.5 s have been timed), each repeat bracketed by
-    barrier + synchronize on both sides and timed with CUDA events on the launching stream; per repeat the MAX over ranks;
-    the MEDIAN repeat is reported."""
+def timed(runner, steps, warmup, barrier, dist, world, max_repeats=5):
+    """W warm-up steps, then EXACTLY `steps` steps split into min(5, steps) repeats of near-equal length, each repeat bracketed
+    by barrier + synchronize on both sides and timed with CUDA events on the launching stream; per repeat the MAX over ranks.
+    Returns the MEDIAN repeat's ms per step and every repeat's (steps, ms)."""
     import torch
     runner.run(warmup)
     barrier()
+    n = min(max_repeats, steps)
     reps = []
-    total = 0.0
-    while len(reps) < min_repeats or (total < min_seconds * 1000.0 and len(reps) < max_repeats):
+    for k in [steps // n + (i < steps % n) for i in range(n)]:
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         ev0.record()
-        runner.run(steps)
+        runner.run(k)
         ev1.record()
         barrier()
         ms = ev0.elapsed_time(ev1)
@@ -294,9 +299,39 @@ def timed(runner, steps, warmup, barrier, dist, world, min_seconds=0.5, min_repe
             t = torch.tensor([ms], device="cuda")
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        reps.append(ms)
-        total += ms
-    return float(np.median(reps)), reps
+        reps.append((k, ms))
+    return float(np.median([ms / k for k, ms in reps])), reps
+
+
+DUMP_TENSORS = re.compile(r"(pi|q1|q2|q1t|q2t)\.[Wb]\d+|out\.(y|logpi|q1|q2)|scal\.(log_alpha|alpha)")
+
+
+def dump_outputs(runner, out_dir, max_agents=16, max_bytes=64 << 20):
+    """What the last update left for its caller, one DIR/<name>.npy per array: every network's weights and biases (pi, q1, q2)
+    and the target copies (q1t, q2t) as float32, the temperature (scal.alpha, scal.log_alpha) as float64, the per-row outputs
+    of the batch (out.y Bellman target, out.logpi, out.q1, out.q2) and the update's metrics (metrics.<key>, float64).
+    A population writes a fixed, seeded sample of `max_agents` of this rank's agents, stacked on a leading axis."""
+    import torch
+    eng = runner.eng
+    torch.cuda.synchronize()
+    agents = [0]
+    if eng.n_agents > 1:
+        agents = sorted(np.random.default_rng(0).choice(eng.n_agents, min(max_agents, eng.n_agents), replace=False).tolist())
+
+    def stack(vals):
+        return vals[0] if eng.n_agents == 1 else np.stack(vals)
+
+    arrays = {name: stack([eng.view(name, a).cpu().numpy() for a in agents]) for name in eng.layout if DUMP_TENSORS.fullmatch(name)}
+    if eng.n_agents > 1:
+        arrays["agents"] = np.asarray(agents, np.float64)
+    metrics = [eng.metrics(a) for a in agents]
+    for key in metrics[0]:
+        arrays[f"metrics.{key}"] = stack([np.float64(m[key]) for m in metrics])
+    total = sum(v.nbytes for v in arrays.values())
+    assert total <= max_bytes, f"output dump of {total} bytes exceeds {max_bytes}"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(v))
 
 
 def dp_checks(runner, dist, world, rank):
@@ -332,7 +367,7 @@ def dp_checks(runner, dist, world, rank):
     return out
 
 
-def measure(name, args, rank, world, local_rank, barrier, dist, steps, warmup, with_clocks):
+def measure(name, args, rank, world, local_rank, barrier, dist, steps, warmup, with_clocks, dump_dir=None):
     import torch
     runner = Runner(name, rank, world, args.chunk)
     w, eng = runner.w, runner.eng
@@ -345,7 +380,9 @@ def measure(name, args, rank, world, local_rank, barrier, dist, steps, warmup, w
         clocks.start()
     l0 = eng.launch_count()
     ms, reps = timed(runner, steps, warmup, barrier, dist, world)
-    launches_per_repeat = (eng.launch_count() - l0) / len(reps)
+    launches = eng.launch_count() - l0
+    if dump_dir and rank == 0:                                       # before anything below runs more updates
+        dump_outputs(runner, dump_dir)
     if runner.dp is not None and world > 1:                           # share of the update spent inside the two all-reduces
         runner.dp.time_exchange = True
         barrier()
@@ -364,23 +401,24 @@ def measure(name, args, rank, world, local_rank, barrier, dist, steps, warmup, w
                             "update and the parameter-sized passes: dW split reduction, Adam, Polyak)")
     clk = None
     if clocks is not None:
-        if sum(reps) < 1500:                                         # a longer stretch for the clock sampler (outside the timed region)
-            runner.run(int(min(50000, 1500 / max(ms / steps, 1e-3))))
+        if sum(t for _, t in reps) < 1500:                           # a longer stretch for the clock sampler (outside the timed region)
+            runner.run(int(min(50000, 1500 / max(ms, 1e-3))))
             torch.cuda.synchronize()
         clk = clocks.stop()
     m = eng.metrics()
     assert m["nonfinite"] == 0 and np.isfinite(m["q1_loss"]), f"non-finite update: {m}"
-    value = runner.units(steps) / (ms / 1000.0)
+    value = runner.units(1) / (ms / 1000.0)
     tc_on, _, tc_launches = eng.tensor_core()
     path = "tensor-core" if tc_on else eng.path()[0]
     gx, gy, smem = eng.grid()
-    res = {"value": value, "unit": "agent-updates/s" if w["n_agents"] > 1 else "updates/s", "ms_per_step": ms / steps, "steps": steps,
-           "repeats": len(reps), "ms_per_step_min": min(reps) / steps, "ms_per_step_max": max(reps) / steps, "scaling": runner.scaling,
-           "path": path, "gpu_launches_per_step": launches_per_repeat / steps, "agents_per_gpu": runner.n_local,
+    per_step = [t / k for k, t in reps]
+    res = {"value": value, "unit": "agent-updates/s" if w["n_agents"] > 1 else "updates/s", "ms_per_step": ms, "steps": steps,
+           "repeats": len(reps), "ms_per_step_min": min(per_step), "ms_per_step_max": max(per_step), "scaling": runner.scaling,
+           "path": path, "gpu_launches_per_step": launches / steps, "agents_per_gpu": runner.n_local,
            "workload": w["label"], "grid": [gx, gy], "smem_bytes": smem, "tc_kernel_launches": int(tc_launches),
            "l2": L2_NOTE[name].format(agents=runner.n_local, gb=runner.n_local * (w["fill"] * (2 * w["obs"] + w["act"] + 2) * 4 + 9.0e6) / 1e9),
            "final_metrics": {k: m[k] for k in ("q1_loss", "policy_loss", "alpha", "updates")}, **extra}
-    return runner, res, clk, launches_per_repeat * len(reps)
+    return runner, res, clk, launches
 
 
 def roofline_of(name, res, world, pk):
@@ -473,7 +511,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the population / data-parallel legs of the default run")
     ap.add_argument("--e2e-steps", type=int, default=0, help="0 = clamp(steps, 200, 2000)")
     ap.add_argument("--chunk", type=int, default=1000, help="updates per kernel launch in the device-resident loop")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -509,7 +552,8 @@ def main():
         torch.cuda.synchronize()
 
     # ---- headline workload: device-resident throughput, then the same metric through the public API -----------------------
-    runner, res, clk, launches = measure(args.workload, args, rank, world, local_rank, barrier, dist, args.steps, W, True)
+    runner, res, clk, launches = measure(args.workload, args, rank, world, local_rank, barrier, dist, args.steps, W, True,
+                                         args.dump_outputs)
     e2e = None
     if runner.agent is not None:
         e2e = e2e_through_public_api(runner.agent, w, args, W, world, barrier, dist)
@@ -520,7 +564,7 @@ def main():
     # population of 1024 agents partitioned over the ranks (no collective); global batch 65536 split over the ranks (2 all-reduces)
     extras = {}
     if args.workload == "bipedal" and not args.no_extras:
-        for name, k, wu in (("population", 10, 3), ("dp", 50, 10)):
+        for name, k, wu in (("population", 60, 3), ("dp", 250, 10)):          # about 0.5 s timed each on one B200
             r2, x, _, _ = measure(name, args, rank, world, local_rank, barrier, dist, k, wu, False)
             del r2
             torch.cuda.empty_cache()

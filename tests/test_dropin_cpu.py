@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 PKG = os.path.join(ROOT, "soft-actor-critic_b200")
 SHIM = os.path.join(HERE, "gym_shim")
-REF = "/root/reference"
+REF = os.environ.get("SAC_REFERENCE_DIR", "")       # a checkout of ignaschuemer7/soft-actor-critic; tests needing it skip without
 
 
 @pytest.fixture()
@@ -59,13 +59,14 @@ def test_sb3_param_mapping(shim):
     assert get_sb3_sac_params(OneDPointMassReachEnv(), cfg, 0)["ent_coef"] == cfg["sac"]["alpha"]
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "sac", "envs.py")), reason="reference checkout not present")
+@pytest.mark.skipif(not REF or not os.path.exists(os.path.join(REF, "sac", "envs.py")),
+                    reason="reference checkout not present (set SAC_REFERENCE_DIR)")
 @pytest.mark.parametrize("name,kwargs", [("ConstantRewardEnv", {}), ("ConstantRewardEnv", {"reward": -2.5, "max_steps": 3}),
                                          ("QuadraticActionRewardEnv", {}), ("QuadraticActionRewardEnv", {"target": -0.3, "max_steps": 2}),
                                          ("RandomObsBinaryRewardEnv", {}), ("RandomObsBinaryRewardEnv", {"obs_dim": 7, "max_steps": 4}),
                                          ("OneDPointMassReachEnv", {}), ("OneDPointMassReachEnv", {"goal_pos": -0.4, "max_steps": 9, "dt": 0.5})])
 def test_probe_envs_behave_like_the_reference(shim, name, kwargs):
-    """Same spaces, observations, rewards, terminated/truncated flags and info dicts as /root/reference/sac/envs.py on the
+    """Same spaces, observations, rewards, terminated/truncated flags and info dicts as the reference's sac/envs.py on the
     same seeds and action sequences."""
     spec = importlib.util.spec_from_file_location("_reference_envs", os.path.join(REF, "sac", "envs.py"))
     ref_mod = importlib.util.module_from_spec(spec)
@@ -89,9 +90,10 @@ def test_probe_envs_behave_like_the_reference(shim, name, kwargs):
             done = ra[2] or ra[3]
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "main.py")), reason="reference checkout not present")
+@pytest.mark.skipif(not REF or not os.path.exists(os.path.join(REF, "main.py")),
+                    reason="reference checkout not present (set SAC_REFERENCE_DIR)")
 def test_unmodified_reference_main_reaches_the_agent_constructor(tmp_path):
-    """`python /root/reference/main.py --config <yaml>` with this package first on PYTHONPATH: the YAML loads, every import
+    """The reference's `python main.py --config <yaml>` with this package first on PYTHONPATH: the YAML loads, every import
     resolves to this repo, the named probe environment is built, and the run stops exactly where this repo must stop on a
     GPU-less host -- SAC(...) refusing a non-CUDA / absent device (no CPU fallback). On the B200 box the same flow runs to
     'Final average return:' (tests/test_gpu_dropin.py)."""

@@ -1,6 +1,6 @@
 """-m gpu, needs >= 2 GPUs (skipped otherwise): the multi-GPU modes on REAL ranks -- one process per GPU launched with
 torch.distributed.run, NCCL all-reduces over NVLink -- where tests/test_gpu_multi.py emulates the ranks on one GPU.
-Run on the pod with `gpurun --gpus 2 -- python -m pytest tests/test_gpu_dist.py -m gpu`."""
+Run on a machine with two or more GPUs: `python -m pytest tests/test_gpu_dist.py -m gpu`."""
 import os
 import subprocess
 import sys

@@ -1,6 +1,6 @@
-"""oracle/donkey_obs.py against the REAL DonkeyVAEEnv methods of the reference (imported here when /root/reference exists;
-the class needs the simulator only in __init__, so the two methods are called on a bare instance carrying just the fields
-they read)."""
+"""oracle/donkey_obs.py against the REAL DonkeyVAEEnv methods of the reference (imported here when SAC_REFERENCE_DIR names a
+checkout of it; the class needs the simulator only in __init__, so the two methods are called on a bare instance carrying just
+the fields they read)."""
 import importlib.util
 import os
 import sys
@@ -9,10 +9,11 @@ import types
 import numpy as np
 import pytest
 
-REF = "/root/reference/DonkeyCarEnv/donkey_gym/envs/vae_env.py"
+REF_DIR = os.environ.get("SAC_REFERENCE_DIR", "")
+REF = os.path.join(REF_DIR, "DonkeyCarEnv", "donkey_gym", "envs", "vae_env.py")
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference checkout not present")
+@pytest.mark.skipif(not REF_DIR or not os.path.exists(REF), reason="reference checkout not present (set SAC_REFERENCE_DIR)")
 @pytest.mark.parametrize("z,n_hist,n_stack", [(32, 20, 3), (32, 20, 1), (8, 3, 4)])
 def test_oracle_matches_reference_postprocessing(z, n_hist, n_stack, monkeypatch):
     from oracle.donkey_obs import DonkeyObsOracle

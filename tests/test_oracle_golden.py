@@ -18,6 +18,17 @@ LARGE = ["bipedal", "pendulum128"]
 # round 2: BASELINE configs 3 / 4 / 5 themselves, K = 10, runs continued from reference-written checkpoints
 ROUND2 = ["cfg3_pendulum256", "cfg4_donkey", "cfg4_donkey_elu", "cfg4_donkey_obs216", "cfg5_b2048", "cfg5_b65536", "bipedal_k10",
           "ckpt_tiny_auto", "ckpt_pendulum128"]
+# The golden files were recorded with torch on 8 CPU threads. torch's reductions and MKL's GEMMs split their work by the
+# thread count, so the same ops give the same bits only at the same count (12 threads, or 1, already differ in the last bit).
+RECORDING_THREADS = 8
+
+
+@pytest.fixture(autouse=True)
+def recording_threads():
+    n = torch.get_num_threads()
+    torch.set_num_threads(RECORDING_THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 def _port_from_golden(g):
