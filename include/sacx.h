@@ -259,6 +259,41 @@ int sacx_debug_profile(sacx_agent_t h, int32_t n_steps, uint64_t* out_host, int6
 /* number of kernels this handle has launched since create (bench.py's gpu_launches) */
 int64_t sacx_launch_count(sacx_agent_t h);
 
+/* ---------------------------------------------------------------- prioritized experience replay (Schaul et al., 2016)
+ * A sum/min tree of fan-out 32 over the slots of a single-agent ring; the handle owns its device memory.
+ *   priority of a written row  p = (|delta| + eps)^alpha; transitions pushed since the tree last looked get p_max (the
+ *                              largest priority ever assigned, initially 1), applied lazily from the ring header's push count
+ *   sampling                   stratified proportional: row k draws u = (k + U_k) / B * sum(p) and takes the first slot whose
+ *                              inclusive prefix sum exceeds u (duplicates allowed; never an empty slot)
+ *   importance weight          w = (p / p_min)^(-beta), p_min over the stored transitions, so w in (0, 1]
+ * Every call is one cooperative kernel on the attached agent's stream (else the ring's); no call synchronises except
+ * sacx_per_priorities with p_max != NULL and sacx_per_load_priorities. Tree nodes are recomputed from their children in a fixed
+ * order (no atomic accumulation): results are bit-reproducible. */
+typedef struct sacx_per_s* sacx_per_t;
+/* max_batch: the largest B of sacx_per_sample and of an attached agent's batch. SACX_ERR_INVALID for alpha < 0, beta0 outside [0, 1],
+ * beta_steps < 0, eps <= 0 or a ring with n_agents > 1. */
+int sacx_per_create(sacx_ring_t ring, float alpha, float beta0, int64_t beta_steps, float eps, int32_t max_batch, sacx_per_t* out);
+int sacx_per_destroy(sacx_per_t per);
+/* B logical indices (idx_dev, the idx_dev format of sacx_update: position in the deque, 0 = oldest) and weights w_dev at exponent
+ * beta. u_dev [B] in [0, 1) or NULL -> device Philox keyed by (seed, agent 0, counter, k), a stream of its own. */
+int sacx_per_sample(sacx_per_t per, int32_t B, float beta, const float* u_dev /* nullable */, uint64_t seed, uint64_t counter,
+                    int64_t* idx_dev, float* w_dev);
+/* new priorities (|delta_dev[k]| + eps)^alpha for logical indices of the most recent sample; out-of-range indices are ignored,
+ * a slot named twice takes the row with the highest k, slots overwritten by pushes since keep p_max */
+int sacx_per_update_priorities(sacx_per_t per, const int64_t* idx_dev, const float* delta_dev, int32_t B);
+/* leaves_dev [capacity] (by ring slot, 0 = empty; nullable) and p_max (nullable; synchronises) after applying pending writes */
+int sacx_per_priorities(sacx_per_t per, float* leaves_dev, float* p_max);
+/* exact resume: replace the leaves (by ring slot) and p_max, rebuild the tree; the ring image must be loaded first */
+int sacx_per_load_priorities(sacx_per_t per, const float* leaves_dev, float p_max);
+/* With a tree attached (NULL detaches), sacx_update(h, NULL, eps1, eps2, n) runs n x (tree launch: write-back of the previous
+ * update's rows from its q1 / q2 / y, delta = (|q1 - y| + |q2 - y|) / 2, new pushes, sample of this batch with beta(t) = min(1,
+ * beta0 + (1 - beta0) t / beta_steps) at the agent's update counter t -> fused update with critic loss (1/B) sum w (q - y)^2,
+ * n_steps = 1); the last write-back is applied by the next tree launch or by any other launch on the agent. The actor and
+ * temperature losses stay unweighted. SACX_ERR_INVALID: n_agents > 1, dp_world > 1, a tree of another ring, max_batch below
+ * batch_size. With a tree attached, sacx_update with idx_dev != NULL, sacx_update_host*, and sacx_update_staged are refused; the
+ * per-phase entry points (sacx_critic_step, ...) stay unweighted. */
+int sacx_agent_attach_per(sacx_agent_t h, sacx_per_t per);
+
 #ifdef __cplusplus
 }
 #endif

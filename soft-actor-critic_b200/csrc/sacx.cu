@@ -11,6 +11,7 @@
 #include <vector>
 
 #include "sacx_engine.cuh"
+#include "sacx_per.cuh"
 
 namespace sacx {
 
@@ -103,8 +104,77 @@ struct Ring {
   }
 };
 
+// ------------------------------------------------------------------------------------------ prioritized replay tree
+// Host side of sacx_per.cuh: owns the tree's device memory (the agent arena is untouched) and issues per_refresh_kernel.
+// Every call is one cooperative launch on the attached agent's stream (else the ring's). The write-back of an agent update
+// is deferred into the next launch (the next update's sample, or a read of the priorities); every launch that can overwrite
+// the arena's per-row q / y flushes it first (engine_launch, engine_launch_rp).
+struct Per {
+  Ring* ring = nullptr;
+  Engine* agent = nullptr;
+  float alpha = 0.6f, eps = 1e-6f;
+  double beta0 = 0.4;
+  i64 beta_steps = 0;
+  int max_batch = 0, depth = 0, grid_max = 1;
+  i64 nodes[PER_MAX_LEVELS + 1] = {};
+  i64 internal = 0;                    // internal nodes over all levels
+  float* d_leaf = nullptr;
+  float* d_tree = nullptr;             // sums of levels 1..depth, then mins
+  unsigned* d_mark = nullptr;
+  unsigned long long* d_win = nullptr;
+  PerState* d_st = nullptr;
+  i64* d_idx = nullptr; float* d_w = nullptr; i64* d_slots = nullptr;   // [max_batch]: the agent update's batch
+  unsigned epoch = 0;
+  i64 seen_hint = 0;                   // host view of PerState::seen (sizes the grid only)
+  bool rebuild = true;                 // internal nodes not valid yet (create, load_priorities)
+  int pend_n = 0;                      // deferred write-back: rows of the last agent update
+  const float *pend_q1 = nullptr, *pend_q2 = nullptr, *pend_y = nullptr;
+
+  cudaStream_t stream() const { return agent ? agent->stream : ring->stream; }
+
+  PerArgs base() {
+    PerArgs a;
+    memset(&a, 0, sizeof a);
+    a.leaf = d_leaf;
+    i64 off = 0;
+    for (int l = 1; l <= depth; ++l) {
+      a.sum[l] = d_tree + off; a.mn[l] = d_tree + internal + off; a.mark[l] = d_mark + off;
+      off += nodes[l];
+    }
+    for (int l = 0; l <= depth; ++l) a.nodes[l] = nodes[l];
+    a.depth = depth; a.win = d_win; a.st = d_st; a.hdr = reinterpret_cast<const RingMeta*>(ring->block(0)); a.cap = ring->cap;
+    a.alpha = alpha; a.eps = eps; a.beta0 = beta0; a.beta_steps = beta_steps;
+    if (pend_n) {
+      a.wb_n = pend_n; a.wb_slots = d_slots; a.wb_q1 = pend_q1; a.wb_q2 = pend_q2; a.wb_y = pend_y;
+    }
+    return a;
+  }
+  int run(PerArgs& a) {
+    int rc = ring->flush();
+    if (rc) return rc;
+    if (ring->stream != stream()) SACX_CUDA(cudaStreamSynchronize(ring->stream));
+    const i64 pushes = ring->pushes[0], n_new = pushes - seen_hint;
+    const bool full = rebuild || n_new < 0 || n_new >= ring->cap;
+    const i64 work = full ? ring->cap : std::max<i64>(a.B, a.wb_n + n_new);
+    a.rebuild = rebuild ? 1 : 0;
+    a.epoch = ++epoch;
+    // one warp per row / touched leaf: the sampler's walk and the propagation are chains of dependent L2 reads, so the
+    // rows run side by side rather than one after another on fewer warps (B 256: 32 CTAs)
+    const int blocks = (int)std::max<i64>(1, std::min<i64>(grid_max, (work + 7) / 8));
+    void* args[] = {(void*)&a};
+    SACX_CUDA(cudaLaunchCooperativeKernel((const void*)per_refresh_kernel, dim3(blocks), dim3(256), args, 0, stream()));
+    if (agent) ++agent->launches;
+    seen_hint = pushes; rebuild = false; pend_n = 0;
+    return SACX_OK;
+  }
+  int flush() { PerArgs a = base(); return run(a); }
+};
+
 // ------------------------------------------------------------------------------------------ engine runtime
+static int per_flush_pending(Engine* e) { return (e->per && e->per->pend_n) ? e->per->flush() : SACX_OK; }
+
 static int engine_launch(Engine* e, int plan_id, int pb, int pe, int n_steps, const RunArgs& proto, bool per_phase) {
+  { int rc = per_flush_pending(e); if (rc) return rc; }
   const Plan& hp = e->h_plans[plan_id];
   if (pe < 0) pe = hp.n_phases;
   RunArgs a = proto;
@@ -215,6 +285,7 @@ static int engine_launch(Engine* e, int plan_id, int pb, int pe, int n_steps, co
 // Row-parallel launch: n_groups x 8 CTAs, cooperative (all CTAs co-resident: grid and group barriers spin).
 
 static int engine_launch_rp(Engine* e, int n_steps, const RunArgs& proto) {
+  { int rc = per_flush_pending(e); if (rc) return rc; }
   RunArgs a = proto;
   a.arena = e->arena; a.agent_stride = e->stride; a.scal_off = e->scal_off; a.hp = e->hp;
   a.n_agents = 1; a.barrier = e->d_barrier; a.ctas_per_agent = e->rp_grid; a.barrier_mode = e->rp_barrier_mode;
@@ -562,6 +633,7 @@ using namespace sacx;
 
 struct sacx_ring_s { Ring r; };
 struct sacx_agent_s { Engine e; };
+struct sacx_per_s { Per p; };
 
 extern "C" {
 
@@ -993,6 +1065,7 @@ int sacx_agent_create(const sacx_config* cfg, float* arena_dev, sacx_agent_t* ou
 int sacx_agent_destroy(sacx_agent_t h) {
   if (!h) return SACX_OK;
   Engine& e = h->e;
+  if (e.per) { e.per->flush(); e.per->agent = nullptr; }     // the pending write-back reads this arena
   cudaStreamSynchronize(e.stream);
   if (e.own_arena && e.arena) cudaFree(e.arena);
   if (e.d_plans) cudaFree(e.d_plans);
@@ -1116,6 +1189,26 @@ static int do_update(sacx_agent_t h, const int64_t* idx, const float* e1, const 
   if (rc) return rc;
   RunArgs a;
   memset(&a, 0, sizeof a);
+  if (e.per) {
+    // prioritized replay: per update, one tree launch (deferred write-back of the previous update + new pushes + sample of
+    // this batch and its weights), then the update itself with n_steps = 1; this update's write-back is left pending
+    if (idx) return fail(SACX_ERR_INVALID, "update: a prioritized replay tree is attached; it samples the batch (pass idx = NULL)");
+    if (staged) return fail(SACX_ERR_INVALID, "sacx_update_staged does not support prioritized replay");
+    Per& p = *e.per;
+    const i64 nba = (i64)e.cfg.batch_size * e.cfg.act_dim;
+    for (int s = 0; s < n_steps; ++s) {
+      PerArgs pa = p.base();
+      pa.B = e.cfg.batch_size; pa.scal = reinterpret_cast<const AgentScalars*>(e.arena + e.scal_off);
+      pa.out_idx = p.d_idx; pa.out_w = p.d_w; pa.out_slots = p.d_slots;
+      if ((rc = p.run(pa))) return rc;
+      a.idx_ext = p.d_idx; a.w_ext = p.d_w;
+      a.eps1_ext = e1 ? e1 + s * nba : nullptr; a.eps2_ext = e2 ? e2 + s * nba : nullptr;
+      if ((rc = e.rp ? engine_launch_rp(&e, 1, a) : engine_launch(&e, PLAN_FUSED, 0, -1, 1, a, false))) return rc;
+      p.pend_n = e.cfg.batch_size;
+      p.pend_q1 = e.arena + e.b_q[0]; p.pend_q2 = e.arena + e.b_q[1]; p.pend_y = e.arena + e.b_y;
+    }
+    return SACX_OK;
+  }
   a.idx_ext = (const i64*)idx; a.eps1_ext = e1; a.eps2_ext = e2;
   if (e.rp && !staged) return engine_launch_rp(&e, n_steps, a);
   return engine_launch(&e, PLAN_FUSED, 0, -1, n_steps, a, staged);
@@ -1271,6 +1364,7 @@ static int host_update_collect(Engine& e, int slot, sacx_metrics* out) {
 
 int sacx_update_host(sacx_agent_t h, const int64_t* idx, const float* e1, const float* e2, int32_t n_steps, sacx_metrics* m) {
   if (!h || n_steps <= 0) return fail(SACX_ERR_INVALID, "update_host: bad arguments");
+  if (h->e.per) return fail(SACX_ERR_INVALID, "update_host: not available with prioritized replay (use sacx_update)");
   Engine& e = h->e;
   const int slot = (int)(e.host_calls++ & 1);
   int rc = host_update_submit(e, slot, idx, e1, e2, n_steps);
@@ -1281,6 +1375,7 @@ int sacx_update_host(sacx_agent_t h, const int64_t* idx, const float* e1, const 
 int sacx_update_host_pipelined(sacx_agent_t h, const int64_t* idx, const float* e1, const float* e2, int32_t n_steps,
                                sacx_metrics* prev_metrics, int32_t* have_prev) {
   if (!h || n_steps <= 0) return fail(SACX_ERR_INVALID, "update_host_pipelined: bad arguments");
+  if (h->e.per) return fail(SACX_ERR_INVALID, "update_host_pipelined: not available with prioritized replay (use sacx_update)");
   Engine& e = h->e;
   const int slot = (int)(e.host_calls++ & 1);
   int rc = host_update_submit(e, slot, idx, e1, e2, n_steps);
@@ -1521,5 +1616,135 @@ int sacx_sync(sacx_agent_t h) {
 }
 
 int64_t sacx_launch_count(sacx_agent_t h) { return h ? h->e.launches + (h->e.ring ? h->e.ring->launches : 0) : 0; }
+
+// ---------------------------------------------------------------------------------------- prioritized replay
+int sacx_per_create(sacx_ring_t ring, float alpha, float beta0, int64_t beta_steps, float eps, int32_t max_batch, sacx_per_t* out) {
+  if (!ring || !out) return fail(SACX_ERR_INVALID, "per_create: null argument");
+  if (!(alpha >= 0.f) || !(beta0 >= 0.f && beta0 <= 1.f) || beta_steps < 0 || !(eps > 0.f) || !std::isfinite(alpha) || !std::isfinite(eps) ||
+      max_batch <= 0)
+    return fail(SACX_ERR_INVALID, "per_create: need alpha >= 0, 0 <= beta0 <= 1, beta_steps >= 0, eps > 0, max_batch > 0");
+  Ring& r = ring->r;
+  if (r.n_agents != 1) return fail(SACX_ERR_INVALID, "per_create: prioritized replay needs a single-agent ring");
+  sacx_per_s* h = new sacx_per_s();
+  Per& p = h->p;
+  p.ring = &r; p.alpha = alpha; p.beta0 = beta0; p.beta_steps = beta_steps; p.eps = eps; p.max_batch = max_batch;
+  p.nodes[0] = r.cap;
+  do {
+    ++p.depth;
+    p.nodes[p.depth] = (p.nodes[p.depth - 1] + PER_FANOUT - 1) / PER_FANOUT;
+    p.internal += p.nodes[p.depth];
+  } while (p.nodes[p.depth] > 1);
+  int rc = SACX_OK;
+  auto bad = [&](cudaError_t ce) { if (ce == cudaSuccess) return false; rc = fail(SACX_ERR_CUDA, cudaGetErrorString(ce)); return true; };
+  int dev = 0, sms = 0, per_sm = 0;
+  PerState st;
+  memset(&st, 0, sizeof st);
+  const float one = 1.f;
+  memcpy(&st.pmax_bits, &one, 4);
+  if (bad(cudaGetDevice(&dev)) || bad(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) ||
+      bad(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, per_refresh_kernel, 256, 0)) ||
+      bad(cudaMalloc((void**)&p.d_leaf, (size_t)r.cap * 4)) || bad(cudaMalloc((void**)&p.d_tree, (size_t)p.internal * 8)) ||
+      bad(cudaMalloc((void**)&p.d_mark, (size_t)p.internal * 4)) || bad(cudaMalloc((void**)&p.d_win, (size_t)r.cap * 8)) ||
+      bad(cudaMalloc((void**)&p.d_st, sizeof(PerState))) || bad(cudaMalloc((void**)&p.d_idx, (size_t)max_batch * 8)) ||
+      bad(cudaMalloc((void**)&p.d_w, (size_t)max_batch * 4)) || bad(cudaMalloc((void**)&p.d_slots, (size_t)max_batch * 8)) ||
+      bad(cudaMemset(p.d_leaf, 0, (size_t)r.cap * 4)) || bad(cudaMemset(p.d_mark, 0, (size_t)p.internal * 4)) ||
+      bad(cudaMemset(p.d_win, 0, (size_t)r.cap * 8)) || bad(cudaMemcpy(p.d_st, &st, sizeof st, cudaMemcpyHostToDevice))) {
+    sacx_per_destroy(h);
+    return rc;
+  }
+  p.grid_max = std::max(1, per_sm * sms);
+  *out = h;
+  return SACX_OK;
+}
+
+int sacx_per_destroy(sacx_per_t h) {
+  if (!h) return SACX_OK;
+  Per& p = h->p;
+  if (p.agent) { p.flush(); p.agent->per = nullptr; p.agent = nullptr; }
+  cudaStreamSynchronize(p.stream());
+  cudaFree(p.d_leaf); cudaFree(p.d_tree); cudaFree(p.d_mark); cudaFree(p.d_win); cudaFree(p.d_st);
+  cudaFree(p.d_idx); cudaFree(p.d_w); cudaFree(p.d_slots);
+  delete h;
+  return SACX_OK;
+}
+
+int sacx_per_sample(sacx_per_t h, int32_t B, float beta, const float* u_dev, uint64_t seed, uint64_t counter, int64_t* idx_dev,
+                    float* w_dev) {
+  if (!h || B <= 0 || !idx_dev || !w_dev) return fail(SACX_ERR_INVALID, "per_sample: bad arguments");
+  Per& p = h->p;
+  if (B > p.max_batch) return fail(SACX_ERR_INVALID, "per_sample: B exceeds the tree's max_batch");
+  if (!(beta >= 0.f && beta <= 1.f)) return fail(SACX_ERR_INVALID, "per_sample: beta must be in [0, 1]");
+  if (p.ring->len(0) < 1) return fail(SACX_ERR_UNDERFILLED, "per_sample: the replay buffer is empty");
+  PerArgs a = p.base();
+  a.B = B; a.beta = beta; a.u_ext = u_dev; a.seed = seed; a.counter = counter; a.agent = 0;
+  a.out_idx = (i64*)idx_dev; a.out_w = w_dev; a.out_slots = p.d_slots;
+  return p.run(a);
+}
+
+int sacx_per_update_priorities(sacx_per_t h, const int64_t* idx_dev, const float* delta_dev, int32_t B) {
+  if (!h || !idx_dev || !delta_dev || B <= 0) return fail(SACX_ERR_INVALID, "per_update_priorities: bad arguments");
+  Per& p = h->p;
+  int rc = p.pend_n ? p.flush() : SACX_OK;
+  if (rc) return rc;
+  PerArgs a = p.base();
+  a.wb_n = B; a.wb_idx = (const i64*)idx_dev; a.wb_delta = delta_dev;
+  return p.run(a);
+}
+
+int sacx_per_priorities(sacx_per_t h, float* leaves_dev, float* p_max) {
+  if (!h) return fail(SACX_ERR_INVALID, "null tree");
+  Per& p = h->p;
+  int rc = p.flush();
+  if (rc) return rc;
+  if (leaves_dev) SACX_CUDA(cudaMemcpyAsync(leaves_dev, p.d_leaf, (size_t)p.ring->cap * 4, cudaMemcpyDeviceToDevice, p.stream()));
+  if (p_max) {
+    PerState st;
+    SACX_CUDA(cudaMemcpyAsync(&st, p.d_st, sizeof st, cudaMemcpyDeviceToHost, p.stream()));
+    SACX_CUDA(cudaStreamSynchronize(p.stream()));
+    memcpy(p_max, &st.pmax_bits, 4);
+  }
+  return SACX_OK;
+}
+
+int sacx_per_load_priorities(sacx_per_t h, const float* leaves_dev, float p_max) {
+  if (!h || !leaves_dev || !(p_max > 0.f) || !std::isfinite(p_max)) return fail(SACX_ERR_INVALID, "per_load_priorities: bad arguments");
+  Per& p = h->p;
+  p.pend_n = 0;                                        // priorities of the run being replaced
+  int rc = p.ring->flush();
+  if (rc) return rc;
+  SACX_CUDA(cudaStreamSynchronize(p.ring->stream));
+  const i64 pushes = p.ring->pushes[0], cap = p.ring->cap;
+  PerState st;
+  memset(&st, 0, sizeof st);
+  st.seen = pushes; st.sample_oldest = pushes > cap ? pushes % cap : 0;
+  memcpy(&st.pmax_bits, &p_max, 4);
+  SACX_CUDA(cudaMemcpyAsync(p.d_leaf, leaves_dev, (size_t)cap * 4, cudaMemcpyDeviceToDevice, p.stream()));
+  SACX_CUDA(cudaMemcpyAsync(p.d_st, &st, sizeof st, cudaMemcpyHostToDevice, p.stream()));
+  SACX_CUDA(cudaStreamSynchronize(p.stream()));
+  p.seen_hint = pushes;
+  p.rebuild = true;
+  return p.flush();
+}
+
+int sacx_agent_attach_per(sacx_agent_t h, sacx_per_t per) {
+  if (!h) return fail(SACX_ERR_INVALID, "null agent");
+  Engine& e = h->e;
+  if (per) {
+    Per& p = per->p;
+    if (e.cfg.n_agents != 1 || e.cfg.dp_world > 1)
+      return fail(SACX_ERR_INVALID, "prioritized replay supports a single agent without data parallelism");
+    if (e.ring != p.ring) return fail(SACX_ERR_INVALID, "attach_per: the tree belongs to a different ring than the agent's");
+    if (p.max_batch < e.cfg.batch_size) return fail(SACX_ERR_INVALID, "attach_per: the tree's max_batch is below the batch size");
+    if (p.agent && p.agent != &e) return fail(SACX_ERR_INVALID, "attach_per: the tree is attached to another agent");
+  }
+  if (e.per && e.per != (per ? &per->p : nullptr)) {
+    int rc = e.per->flush();
+    if (rc) return rc;
+    e.per->agent = nullptr;
+  }
+  e.per = per ? &per->p : nullptr;
+  if (per) per->p.agent = &e;
+  return SACX_OK;
+}
 
 }  // extern "C"

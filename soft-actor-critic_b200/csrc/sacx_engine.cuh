@@ -45,6 +45,7 @@ enum PlanId { PLAN_FUSED = 0, PLAN_SAMPLE, PLAN_TARGET, PLAN_CRITIC, PLAN_CRITIC
               PLAN_ALPHA, PLAN_POLYAK, PLAN_APPLY_Q, PLAN_APPLY_Q_POLYAK, PLAN_APPLY_PI, PLAN_FUSED_NOGATHER, PLAN_ALPHA_APPLY, PLAN_RP, N_PLANS };
 
 struct Ring;
+struct Per;
 
 struct Engine {
   sacx_config cfg;
@@ -90,6 +91,7 @@ struct Engine {
   bool pipelined_pending = false;
   cudaStream_t stream = 0;
   Ring* ring = nullptr;
+  Per* per = nullptr;                     // prioritized replay tree (sacx_agent_attach_per), or null: uniform sampling
   long long launches = 0;
   unsigned long long act_calls = 0;
   Hyper hp;

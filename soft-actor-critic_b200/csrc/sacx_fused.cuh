@@ -30,6 +30,7 @@ struct FusedCtx {
   const AgentScalars* scal;
   const Hyper* hp;
   float* xsm;
+  const float* w_ext;             // RunArgs::w_ext
 };
 
 __device__ __forceinline__ float sum_parts(const float* __restrict__ p, int n_part, i64 stride) {
@@ -51,7 +52,7 @@ __device__ __forceinline__ float sum_parts8(const float* __restrict__ p, int n_p
 // GEN_CRITIC slots: o[2..3]=target-critic shares [tn][B]  o[4..5]=target output biases  o[6]=r o[7]=d o[8]=logpi' o[9]=y out
 //   o[10..11]=tq out  o[12]=this critic's shares  o[13]=its output bias  o[14]=q out  o[15]=dout out (ld 4)  o[16]=lossrow out
 //   o[17]=W_L of this critic   i[2]=number of shares  i[3]=critic index
-struct CriticRow { float y, tq1, tq2, q, dout, diff; };
+struct CriticRow { float y, tq1, tq2, q, dout, diff, w; };
 // all 8 lanes of the row call this (shuffles inside); every lane returns the full result
 __device__ __forceinline__ CriticRow critic_row_scalars(const Op& op, const FusedCtx& c, int m, int j8, bool ok) {
   const Hyper& hp = *c.hp;
@@ -74,7 +75,8 @@ __device__ __forceinline__ CriticRow critic_row_scalars(const Op& op, const Fuse
   const float z = sq + bq;
   r.q = act_fwd(op.act_out, z);
   r.diff = r.q - r.y;
-  r.dout = (2.f * r.diff / (float)hp.B_global) * act_dz2(op.act_out, z, r.q);     // d mse / d q through the output activation
+  r.w = (c.w_ext && ok) ? __ldcg(c.w_ext + m) : 1.f;       // importance weight (prioritized replay); 1 multiplies exactly
+  r.dout = (2.f * (r.w * r.diff) / (float)hp.B_global) * act_dz2(op.act_out, z, r.q);     // d mse / d q through the output activation
   return r;
 }
 
@@ -98,7 +100,7 @@ __device__ __forceinline__ void gen_prologue(const Op& op, const FusedCtx& c, in
         if (op.i[3] == 0) { base[op.o[9] + m] = cr.y; base[op.o[10] + m] = cr.tq1; base[op.o[11] + m] = cr.tq2; }
         base[op.o[14] + m] = cr.q;
         base[op.o[15] + (i64)m * 4] = cr.dout;
-        base[op.o[16] + m] = cr.diff * cr.diff;
+        base[op.o[16] + m] = cr.w * (cr.diff * cr.diff);
       }
     } else {
       // GEN_ACTORQ: o[2..3]=shares of Q1,Q2(s, a~pi)  o[4..5]=output biases  o[8]=logpi  o[10..11]=q out  o[16]=policy loss rows

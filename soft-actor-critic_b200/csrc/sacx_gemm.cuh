@@ -59,6 +59,7 @@ struct EpiCtx {
   const Hyper* hp;
   unsigned long long* t;        // optional intra-tile timestamps (profiling aid), 8 slots
   float* xsm;                   // extra shared memory of the fused paths (XSM_FLOATS)
+  const float* w_ext;           // RunArgs::w_ext (critic loss weights)
 };
 // (intra-tile timestamps for tools/phase_profile.py: debug library only, like the row-parallel kernel's event trace)
 #ifdef SACX_DEBUG_HOOKS
@@ -402,7 +403,7 @@ __device__ __noinline__ void gemm_tile_impl(const Op& op, const EpiCtx& ctx, int
   const bool bias_tile = BSUM && (tn == 0) && (op.pb >= 0);
   const int nk = (K + GEMM_BK - 1) / GEMM_BK;
   SACX_TSTAMP(0);
-  const FusedCtx fc{ctx.base, ctx.scal, ctx.hp, ctx.xsm};
+  const FusedCtx fc{ctx.base, ctx.scal, ctx.hp, ctx.xsm, ctx.w_ext};
   const bool gen = (MODE == 1) && (op.mode != GEN_NONE);
   const bool part = (MODE <= 1) && (op.i[4] != 0);
   if (part) part_stage(op, fc, n0, BN);

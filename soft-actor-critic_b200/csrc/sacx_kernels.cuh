@@ -79,8 +79,8 @@ __global__ void __launch_bounds__(256, 1) sacx_run_kernel(const Plan* __restrict
     AgentScalars* scal = reinterpret_cast<AgentScalars*>(base + args.scal_off);
     RowCtx rc{base, scal, &sargs, agent, 0, wsm + warp * 4 * SACX_MAX_ACT, gsm, C::SMEM_FLOATS, nullptr};
     rc.gcache = gcache + warp * GCACHE_WORDS;
-    EpiCtx ec{base, scal, &sargs.hp, nullptr, gsm + C::SMEM_FLOATS};
-    const FusedCtx fcx{base, scal, &sargs.hp, gsm + C::SMEM_FLOATS};
+    EpiCtx ec{base, scal, &sargs.hp, nullptr, gsm + C::SMEM_FLOATS, sargs.w_ext};
+    const FusedCtx fcx{base, scal, &sargs.hp, gsm + C::SMEM_FLOATS, sargs.w_ext};
     const bool last_agent = (agent + (int)gridDim.y >= args.n_agents);
     for (int step = 0; step < args.n_steps; ++step) {
       rc.step = step;

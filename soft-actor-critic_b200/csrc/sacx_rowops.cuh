@@ -303,12 +303,13 @@ __device__ __forceinline__ void tile_q_tail(const Op& op, const RowCtx& c, int t
   }
   if (op.mode & 2) {
     if (!(op.mode & 1)) y = c.args->y_ext ? c.args->y_ext[row] : __ldcg(base + op.o[9] + row);
+    const float w = c.args->w_ext ? __ldcg(c.args->w_ext + row) : 1.f;     // importance weight; 1 multiplies exactly
 #pragma unroll
     for (int cc = 0; cc < 2; ++cc) {
       const float z = __ldcg(base + op.o[2 + cc] + row), q = act_fwd(op.act_out, z), diff = q - y;
       base[op.o[2 + cc] + row] = q;
-      base[op.o[10 + cc] + (i64)row * 4] = (2.f * diff / (float)hp.B_global) * act_dz2(op.act_out, z, q);
-      base[op.o[12 + cc] + row] = diff * diff;
+      base[op.o[10 + cc] + (i64)row * 4] = (2.f * (w * diff) / (float)hp.B_global) * act_dz2(op.act_out, z, q);
+      base[op.o[12 + cc] + row] = w * (diff * diff);
     }
   }
   if (op.mode & 4) {
@@ -381,7 +382,7 @@ __device__ __noinline__ void tile_q_row(const Op& op, const RowCtx& c, int tile)
   const bool aux_is_h = do_c && (op.o[14] == op.o[12]);
   RowReg ht[2], hc[2], ac[2];
   // scalars of this row travel together with the staged weights (no dependent L2 round trip after the barrier)
-  float bt[2] = {0.f, 0.f}, bc_[2] = {0.f, 0.f}, alpha = 0.f, r_ = 0.f, d_ = 0.f, lp2_ = 0.f, y_in = 0.f;
+  float bt[2] = {0.f, 0.f}, bc_[2] = {0.f, 0.f}, alpha = 0.f, r_ = 0.f, d_ = 0.f, lp2_ = 0.f, y_in = 0.f, w_in = 1.f;
   if (in) {
     if (do_t) {
       bt[0] = __ldcg(base + op.o[4]); bt[1] = __ldcg(base + op.o[5]);
@@ -392,6 +393,7 @@ __device__ __noinline__ void tile_q_row(const Op& op, const RowCtx& c, int tile)
       bc_[0] = __ldcg(base + op.o[18]); bc_[1] = __ldcg(base + op.o[19]);
       if (c.args->y_ext) y_in = c.args->y_ext[row];
       else if (!do_t) y_in = __ldcg(base + op.o[9] + row);
+      if (c.args->w_ext) w_in = __ldcg(c.args->w_ext + row);
     }
   }
   if (staged) {
@@ -446,12 +448,12 @@ __device__ __noinline__ void tile_q_row(const Op& op, const RowCtx& c, int tile)
       const float z = warp_sum(part) + bc_[n];
       const float q = act_fwd(op.act_out, z);
       const float diff = q - y;
-      // d mse / d q = 2 (q - y) / B; through the output activation
-      const float dout = (2.f * diff / (float)hp.B_global) * act_dz2(op.act_out, z, q);
+      // d mse / d q = 2 w (q - y) / B (w: importance weight, 1 without prioritized replay); through the output activation
+      const float dout = (2.f * (w_in * diff) / (float)hp.B_global) * act_dz2(op.act_out, z, q);
       if (lane == 0) {
         base[op.o[20 + n] + row] = q;
         base[op.o[22 + n] + (i64)row * 4] = dout;
-        base[op.o[26 + n] + row] = diff * diff;
+        base[op.o[26 + n] + row] = w_in * (diff * diff);
       }
       float* dl = base + op.o[24 + n] + (i64)row * ld;
       if (fast) {

@@ -682,7 +682,9 @@ __device__ __forceinline__ void rp_load_wl(const RpCtx& c, float4 (&wl)[2]) {
   for (int cc = 0; cc < 2; ++cc) wl[cc] = __ldcg(reinterpret_cast<const float4*>(c.base + c.P->q_WL[cc] + k));
 }
 
-// soft Bellman target (agent.py:195-211) and the critics' loss gradient (agent.py:213-236) for the row block
+// soft Bellman target (agent.py:195-211) and the critics' loss gradient (agent.py:213-236) for the row block.
+// WEIGHTED: per-row importance weights of prioritized replay (RunArgs::w_ext); the uniform instantiation has no weight load.
+template <bool WEIGHTED>
 __device__ __noinline__ void rp_target_critic(const RpCtx& c) {
   const Hyper& hp = c.args->hp;
   const RpProgram& P = *c.P;
@@ -704,15 +706,17 @@ __device__ __noinline__ void rp_target_critic(const RpCtx& c) {
     const float sq[2] = {rp_add_parts(pq[0]), rp_add_parts(pq[1])};
     const float tq[2] = {act_fwd(P.act_oq, st[0] + bt[0]), act_fwd(P.act_oq, st[1] + bt[1])};
     const float y = R.r[mm] + (__ldcg(&c.scal->gamma) * (1.f - R.d[mm])) * (fminf(tq[0], tq[1]) - alpha * R.lp2[mm]);
+    const float wr = (WEIGHTED && ok) ? __ldcg(c.args->w_ext + row) : 1.f;
     if (w0 && ok) { c.base[P.b_y + row] = y; c.base[P.b_tq[0] + row] = tq[0]; c.base[P.b_tq[1] + row] = tq[1]; }
 #pragma unroll
     for (int cc = 0; cc < 2; ++cc) {
       const float z = sq[cc] + bq[cc];
       const float q = act_fwd(P.act_oq, z);
       const float diff = q - y;
-      const float dout = (2.f * diff / (float)hp.B_global) * act_dz2(P.act_oq, z, q);
+      // importance weight w (prioritized replay): loss w diff^2, gradient 2 w diff / B; w = 1 multiplies exactly
+      const float dout = (2.f * (wr * diff) / (float)hp.B_global) * act_dz2(P.act_oq, z, q);
       R.coef[cc][mm] = ok ? dout : 0.f;
-      if (w0 && ok) { c.base[P.b_q[cc] + row] = q; c.base[P.b_dout[cc] + (i64)row * 4] = dout; c.base[P.b_loss[cc] + row] = diff * diff; }
+      if (w0 && ok) { c.base[P.b_q[cc] + row] = q; c.base[P.b_dout[cc] + (i64)row * 4] = dout; c.base[P.b_loss[cc] + row] = wr * (diff * diff); }
     }
   }
   RP_TRACE(2902);
@@ -1142,7 +1146,7 @@ __device__ __forceinline__ void rp_run_steps(const RpCtx& c, int s0, int s1, RpS
     switch (st.row_op) {
       case RPR_GATHER: rp_gather(c, *c.L, c.slots); break;
       case RPR_PI_HEADS: rp_pi_heads(c); break;
-      case RPR_TARGET_CRITIC: rp_target_critic(c); break;
+      case RPR_TARGET_CRITIC: if (c.args->w_ext) rp_target_critic<true>(c); else rp_target_critic<false>(c); break;
       case RPR_RELOAD: rp_reload(c); break;
       case RPR_ACTOR_Q: rp_actor_q(c); break;
       case RPR_PI_BWD: rp_pi_bwd(c); break;

@@ -114,6 +114,7 @@ struct RunArgs {
   const float* eps2_ext;
   const float* y_ext;        // staged critic step: external y [B] or null
   const float* lp_ext;       // staged alpha step: external logpi [B] or null
+  const float* w_ext;        // per-row weights of the critic loss [B] (prioritized replay; launches of one update only) or null
   int n_steps, n_agents;
   int phase_begin, phase_end;
   int ctas_per_agent;

@@ -86,6 +86,13 @@ SYMBOLS = {
     "sacx_ring_resync": (C.c_int, [_P]),
     "sacx_index_filter": (_I32, [C.c_char_p, _I32, _U64, _I32, _P, _I32, _I32]),
     "sacx_ring_sample_indices": (C.c_int, [_P, _I32, _U64, _U64, _I32, _P]),
+    "sacx_per_create": (C.c_int, [_P, _F, _F, _I64, _F, _I32, C.POINTER(_P)]),
+    "sacx_per_destroy": (C.c_int, [_P]),
+    "sacx_per_sample": (C.c_int, [_P, _I32, _F, _P, _U64, _U64, _P, _P]),
+    "sacx_per_update_priorities": (C.c_int, [_P, _P, _P, _I32]),
+    "sacx_per_priorities": (C.c_int, [_P, _P, C.POINTER(_F)]),
+    "sacx_per_load_priorities": (C.c_int, [_P, _P, _F]),
+    "sacx_agent_attach_per": (C.c_int, [_P, _P]),
     "sacx_obs_create": (C.c_int, [_I32, _I32, _I32, _I32, C.POINTER(_P)]),
     "sacx_obs_destroy": (C.c_int, [_P]),
     "sacx_obs_dim": (_I32, [_P]),
@@ -186,6 +193,35 @@ def ptr(t) -> Optional[int]:
     if hasattr(t, "data_ptr"):
         return t.data_ptr()
     return t.ctypes.data
+
+
+PER_DEFAULTS = {"alpha": 0.6, "beta": 0.4, "beta_steps": 0, "eps": 1e-6}
+
+
+def per_config(config: dict) -> Optional[dict]:
+    """``buffer.prioritized`` of a YAML config, validated and completed with the defaults; None when absent or null (uniform
+    sampling). Needs no device. ValueError for a bad range or a combination prioritized replay does not support."""
+    p = (config.get("buffer") or {}).get("prioritized")
+    if p is None:
+        return None
+    if not isinstance(p, dict):
+        raise ValueError("buffer.prioritized must be a mapping {alpha, beta, beta_steps, eps} or null")
+    unknown = set(p) - set(PER_DEFAULTS)
+    if unknown:
+        raise ValueError(f"buffer.prioritized: unknown keys {sorted(unknown)}")
+    out = dict(PER_DEFAULTS, **p)
+    alpha, beta, beta_steps, eps = float(out["alpha"]), float(out["beta"]), out["beta_steps"], float(out["eps"])
+    if not alpha >= 0.0 or alpha != alpha or alpha == float("inf"):
+        raise ValueError("buffer.prioritized.alpha must be a finite number >= 0")
+    if not 0.0 <= beta <= 1.0:
+        raise ValueError("buffer.prioritized.beta must be in [0, 1]")
+    if isinstance(beta_steps, bool) or int(beta_steps) != beta_steps or int(beta_steps) < 0:
+        raise ValueError("buffer.prioritized.beta_steps must be an integer >= 0")
+    if not eps > 0.0 or eps == float("inf"):
+        raise ValueError("buffer.prioritized.eps must be a finite number > 0")
+    if (config.get("train") or {}).get("rng", "device") == "host":
+        raise ValueError("buffer.prioritized needs train.rng: device (the tree samples on the device)")
+    return {"alpha": alpha, "beta": beta, "beta_steps": int(beta_steps), "eps": eps}
 
 
 def make_config(obs_dim: int, act_dim: int, config: dict, n_agents: int = 1, ctas_per_agent: int = 0,

@@ -17,6 +17,9 @@ Optional config keys (all default so that every reference YAML loads unchanged):
   ``train.rng``: ``"device"`` (default; Feistel index sampling + Philox normals inside the kernel) or
   ``"host"`` (reference streams: indices from Python's global ``random``, normals from torch's CPU
   generator -- bit-identical index stream, used by the parity tests and the e2e benchmark).
+  ``buffer.prioritized``: ``{alpha: 0.6, beta: 0.4, beta_steps: 0, eps: 1e-6}`` (missing keys take these defaults) turns on
+  prioritized experience replay on the device (``PrioritizedReplayBuffer``; single agent, ``train.rng: device``); absent or
+  null keeps uniform sampling.
 """
 from __future__ import annotations
 
@@ -31,9 +34,10 @@ import numpy as np
 import torch
 import torch.optim as optim
 
+from . import _engine as E
 from .engine import UpdateEngine
 from .models import PolicyNetwork, QNetwork
-from .replay_buffer import ReplayBuffer, Transition
+from .replay_buffer import PrioritizedReplayBuffer, ReplayBuffer, Transition
 
 try:  # progress bars are optional plumbing
     from tqdm import tqdm
@@ -133,8 +137,15 @@ class SAC:
             raise ValueError("train.rng must be 'device' or 'host'")
         seed = config["train"]["seed"]
         pn, qn = config["policy_net"], config["q_net"]
+        self.per = E.per_config(config)            # buffer.prioritized: None -> uniform sampling
 
-        self.replay_buffer = ReplayBuffer(config["buffer"]["capacity"], self.obs_size, self.action_size, device=self.device)
+        if self.per is None:
+            self.replay_buffer = ReplayBuffer(config["buffer"]["capacity"], self.obs_size, self.action_size, device=self.device)
+        else:
+            self.replay_buffer = PrioritizedReplayBuffer(
+                config["buffer"]["capacity"], self.obs_size, self.action_size, device=self.device, alpha=self.per["alpha"],
+                beta=self.per["beta"], beta_steps=self.per["beta_steps"], eps=self.per["eps"],
+                max_batch=config["train"]["batch_size"], seed=seed)
 
         # networks: same constructor calls and seeds as the reference (policy/Q1: seed, Q2: seed+1)
         self.policy_net = PolicyNetwork(self.obs_size, self.action_size, pn["hidden_sizes"], log_std_min=pn["log_std_min"],
@@ -147,6 +158,8 @@ class SAC:
 
         self.engine = UpdateEngine(self.obs_size, self.action_size, config, device=self.device)
         self.engine.attach_ring(self.replay_buffer)
+        if self.per is not None:
+            self.engine.attach_per(self.replay_buffer)
         views = self._views = self.engine.views()
         self.policy_net.bind_to_views(views, "pi")
         self.q_net1.bind_to_views(views, "q1")
@@ -243,7 +256,7 @@ class SAC:
 
     def sample_batch(self) -> Transition:
         """reference: agent.py:166-193 -- float32 device tensors for a ``random.sample`` index draw."""
-        return self.replay_buffer.sample_tensors(self.config["train"]["batch_size"])
+        return ReplayBuffer.sample_tensors(self.replay_buffer, self.config["train"]["batch_size"])
 
     # ------------------------------------------------------------------ acting
     def select_action(self, state: Any, deterministic: bool = False) -> Any:
@@ -495,6 +508,9 @@ class SAC:
             "torch_rng": torch.get_rng_state(),
             "numpy_rng": np.random.get_state(),
         }
+        if self.per is not None:                   # prioritized replay: priorities by ring slot and p_max
+            leaves, p_max = self.replay_buffer.slot_priorities()
+            snap["per"] = {"leaves": leaves.cpu(), "p_max": p_max}
         torch.save(snap, filepath)
 
     def load_snapshot(self, filepath: str) -> None:
@@ -504,6 +520,8 @@ class SAC:
             raise ValueError("not a sacx snapshot")
         if int(snap["seed"]) != int(self.config["train"]["seed"]):
             raise ValueError("snapshot was taken with train.seed=%d: build the agent from the same config to resume" % snap["seed"])
+        if self.per is not None and snap.get("per") is None:
+            raise ValueError("snapshot has no replay priorities: it was taken without buffer.prioritized")
         eng = self.engine
         eng.sync()
         head = snap["arena_head"]
@@ -518,6 +536,8 @@ class SAC:
                 self.replay_buffer._allocate(int(od), int(ad))
                 self.engine.attach_ring(self.replay_buffer)
             self.replay_buffer.load_image(snap["ring"])
+        if self.per is not None:
+            self.replay_buffer.load_slot_priorities(snap["per"]["leaves"], snap["per"]["p_max"])
         random.setstate(snap["python_random"])
         torch.set_rng_state(snap["torch_rng"])
         np.random.set_state(snap["numpy_rng"])

@@ -45,6 +45,7 @@ class UpdateEngine:
         self.layout: Dict[str, Tuple[int, int, int, int, int]] = {
             d.name.decode(): (int(d.offset), int(d.rows), int(d.cols), int(d.ld), int(d.dtype)) for d in descs}
         self.ring = None
+        self.per = None
         self._stream = None
         self._metrics = E.SacxMetrics()
 
@@ -90,6 +91,11 @@ class UpdateEngine:
         self.ring = ring
         E.check(self.lib.sacx_agent_attach_ring(self.h, ring.handle if ring is not None else None))
         self._stream = None
+
+    def attach_per(self, buf) -> None:
+        """Prioritized replay: ``buf`` a PrioritizedReplayBuffer (the attached ring's), or None for uniform sampling."""
+        E.check(self.lib.sacx_agent_attach_per(self.h, buf.per_handle if buf is not None else None))
+        self.per = buf
 
     def reset_state(self) -> None:
         self._sync_stream()

@@ -18,6 +18,7 @@ from typing import Dict, List, Optional, Sequence, Tuple
 import numpy as np
 import torch
 
+from . import _engine as E
 from .engine import UpdateEngine
 from .models import PolicyNetwork, QNetwork
 from .replay_buffer import ReplayBuffer
@@ -47,6 +48,8 @@ def _dist():
 class SACPopulation:
     def __init__(self, obs_dim: int, act_dim: int, config: dict, n_agents: int, seeds: Optional[Sequence[int]] = None,
                  device=None, rank: Optional[int] = None, world: Optional[int] = None, reference_init: bool = True):
+        if E.per_config(config) is not None:
+            raise ValueError("buffer.prioritized is not supported by SACPopulation")
         d = _dist()
         self.world = world if world is not None else (d.get_world_size() if d else 1)
         self.rank = rank if rank is not None else (d.get_rank() if d else 0)
@@ -220,6 +223,8 @@ class DataParallelSAC:
 
     def __init__(self, obs_dim: int, act_dim: int, config: dict, global_batch: int, device=None,
                  rank: Optional[int] = None, world: Optional[int] = None):
+        if E.per_config(config) is not None:
+            raise ValueError("buffer.prioritized is not supported by DataParallelSAC")
         d = _dist()
         self.world = world if world is not None else (d.get_world_size() if d else 1)
         self.rank = rank if rank is not None else (d.get_rank() if d else 0)

@@ -247,3 +247,90 @@ class ReplayBuffer:
     def flush(self) -> None:
         if self._h is not None:
             E.check(self._lib.sacx_ring_flush(self._h))
+
+
+class PrioritizedReplayBuffer(ReplayBuffer):
+    """Prioritized experience replay (Schaul et al., 2016) on the device ring: a sum/min tree over the ring's slots
+    (``sacx_per_*``), proportional stratified sampling, importance weights ``w = (p / p_min)^-beta`` and priorities
+    ``p = (|td| + eps)^alpha``. New transitions enter with the largest priority assigned so far (initially 1).
+
+    ``sample_tensors(B, beta=None)`` returns ``(Transition, weights, indices)``: device tensors, ``indices`` are logical
+    positions (0 = oldest) to hand back to ``update_priorities(indices, td_abs)``. Draws are keyed by ``seed`` and a call
+    counter. Attached to a SAC agent (``buffer.prioritized``), the agent's own updates sample and refresh the tree on the
+    device. ``sample`` and ``draw_indices`` stay the uniform stream of ``ReplayBuffer``."""
+
+    def __init__(self, capacity: int, obs_dim: Optional[int] = None, act_dim: Optional[int] = None,
+                 device: Optional[str] = None, alpha: float = 0.6, beta: float = 0.4, beta_steps: int = 0, eps: float = 1e-6,
+                 max_batch: int = 65536, seed: int = 0):
+        cfg = E.per_config({"buffer": {"prioritized": {"alpha": alpha, "beta": beta, "beta_steps": beta_steps, "eps": eps}}})
+        self.alpha, self.beta, self.beta_steps, self.eps = cfg["alpha"], cfg["beta"], cfg["beta_steps"], cfg["eps"]
+        self.max_batch, self.seed, self._draws = int(max_batch), int(seed), 0
+        self._per = None
+        super().__init__(capacity, obs_dim, act_dim, device=device)
+
+    def _allocate(self, obs_dim: int, act_dim: int) -> None:
+        super()._allocate(obs_dim, act_dim)
+        h = C.c_void_p()
+        E.check(self._lib.sacx_per_create(self._h, self.alpha, self.beta, self.beta_steps, self.eps, self.max_batch, C.byref(h)))
+        self._per = h
+
+    @property
+    def per_handle(self):
+        return self._per
+
+    def __del__(self):
+        try:
+            if self._per is not None:
+                self._lib.sacx_per_destroy(self._per)
+                self._per = None
+        except Exception:
+            pass
+        super().__del__()
+
+    def sample_tensors(self, batch_size: int, beta: Optional[float] = None):
+        self._require(batch_size)
+        beta = self.beta if beta is None else float(beta)
+        kw = dict(device=self.device)
+        idx = torch.empty(batch_size, dtype=torch.int64, **kw)
+        w = torch.empty(batch_size, dtype=torch.float32, **kw)
+        E.check(self._lib.sacx_per_sample(self._per, int(batch_size), beta, None, self.seed, self._draws, idx.data_ptr(), w.data_ptr()))
+        self._draws += 1
+        return ReplayBuffer.sample_tensors(self, batch_size, idx), w, idx
+
+    def sample_with_uniforms(self, u: torch.Tensor, beta: Optional[float] = None):
+        """Indices and weights for given stratum offsets ``u`` in [0, 1) (row k draws (k + u_k) / B of the total priority)."""
+        u = u.to(device=self.device, dtype=torch.float32).contiguous().reshape(-1)
+        B = u.shape[0]
+        beta = self.beta if beta is None else float(beta)
+        idx = torch.empty(B, dtype=torch.int64, device=self.device)
+        w = torch.empty(B, dtype=torch.float32, device=self.device)
+        E.check(self._lib.sacx_per_sample(self._per, B, beta, u.data_ptr(), 0, 0, idx.data_ptr(), w.data_ptr()))
+        return idx, w
+
+    def update_priorities(self, indices, td_abs) -> None:
+        idx = torch.as_tensor(indices).to(device=self.device, dtype=torch.int64).contiguous().reshape(-1)
+        td = torch.as_tensor(td_abs).to(device=self.device, dtype=torch.float32).contiguous().reshape(-1)
+        if idx.shape != td.shape:
+            raise ValueError("indices and td_abs differ in length")
+        if idx.numel():
+            E.check(self._lib.sacx_per_update_priorities(self._per, idx.data_ptr(), td.data_ptr(), idx.numel()))
+
+    def slot_priorities(self):
+        """(priorities by ring slot [capacity], 0 = empty slot; p_max), pending writes applied."""
+        leaves = torch.empty(self.capacity, dtype=torch.float32, device=self.device)
+        pm = C.c_float()
+        E.check(self._lib.sacx_per_priorities(self._per, leaves.data_ptr(), C.byref(pm)))
+        return leaves, float(pm.value)
+
+    def priorities(self) -> torch.Tensor:
+        """Priority of every stored transition in logical order (0 = oldest), a device tensor of length len(self)."""
+        leaves, _ = self.slot_priorities()
+        n, pushes = len(self), int(self._lib.sacx_ring_pushes(self._h, 0))
+        oldest = (pushes - self.capacity) % self.capacity if pushes > self.capacity else 0
+        return leaves[(oldest + torch.arange(n, device=self.device)) % self.capacity]
+
+    def load_slot_priorities(self, leaves: torch.Tensor, p_max: float) -> None:
+        leaves = leaves.to(device=self.device, dtype=torch.float32).contiguous()
+        if leaves.numel() != self.capacity:
+            raise ValueError("priority image does not match this buffer's capacity")
+        E.check(self._lib.sacx_per_load_priorities(self._per, leaves.data_ptr(), float(p_max)))
