@@ -513,6 +513,11 @@ __device__ __forceinline__ void rp_gather_rows(const RpCtx& c, const i64* __rest
     xs2[mm * ldx + col] = 0.f; xpi[mm * ldx + col] = 0.f;
   }
   const bool ok = w0 && slot >= 0;
+  // the row's arena destinations, formed before the first store: the compiler cannot tell a store through a float pointer
+  // from the program table or the context, and reloaded their fields after every store of the scatter
+  const i64 grow = (i64)row * P.gldx;
+  float* const gsa = c.base + P.x_sa + grow, *const gpi = c.base + P.x_pi + grow, *const gs2 = c.base + P.x_s2 + grow;
+  float* const gr = c.base + P.b_r + row, *const gd = c.base + P.b_d + row;
 #pragma unroll
   for (int u = 0; u < MAXE; ++u) {
     const int col = c0 + 16 * u;
@@ -520,19 +525,19 @@ __device__ __forceinline__ void rp_gather_rows(const RpCtx& c, const i64* __rest
       const float x = v[u];
       if (col < O) {
         xsa[mm * ldx + col] = x; xpi[mm * ldx + col] = x;
-        if (ok) { c.base[P.x_sa + (i64)row * P.gldx + col] = x; c.base[P.x_pi + (i64)row * P.gldx + col] = x; }
+        if (ok) { gsa[col] = x; gpi[col] = x; }
       } else if (col < 2 * O) {
         xs2[mm * ldx + col - O] = x;
-        if (ok) c.base[P.x_s2 + (i64)row * P.gldx + col - O] = x;
+        if (ok) gs2[col - O] = x;
       } else if (col < 2 * O + A) {
         xsa[mm * ldx + col - O] = x;                       // action columns sit behind the state in X_sa
-        if (ok) c.base[P.x_sa + (i64)row * P.gldx + col - O] = x;
+        if (ok) gsa[col - O] = x;
       } else if (col == 2 * O + A) {
         R.r[mm] = x;
-        if (ok) c.base[P.b_r + row] = x;
+        if (ok) *gr = x;
       } else {
         R.d[mm] = x;
-        if (ok) c.base[P.b_d + row] = x;
+        if (ok) *gd = x;
       }
     }
   }
@@ -659,18 +664,22 @@ __device__ __forceinline__ void rp_delta_critics(const RpCtx& c, const float4 (&
   const int tid = threadIdx.x, H = P.Hq, NS = H / RP_CS, n0g = c.rank * NS, B = c.args->hp.B;
   const int cpr = H >> 2, k = (tid % cpr) << 2, m0 = tid / cpr, mstep = 256 / cpr;
   const bool mine = store && k >= n0g && k < n0g + NS;
+  // loop operands in registers before the first store (see rp_gather_rows): the rows then cost shared-memory round trips only
+  const int lda = P.lda, act = P.act_q, ld = P.ld_hq, nrows = min(RP_RB, B - c.row0);
 #pragma unroll
   for (int cc = 0; cc < 2; ++cc) {
     float* ab = smem_raw + P.sm_abuf + P.ab_q[cc] * P.abuf_floats;
+    float* const dq = c.base + P.dq_last[cc] + (i64)c.row0 * ld + k;
+    const float* const coef = R.coef[cc];
     const float4 w = wl[cc];
     for (int mm = m0; mm < RP_RB; mm += mstep) {
-      float4* p = reinterpret_cast<float4*>(ab + mm * P.lda + k);
+      float4* p = reinterpret_cast<float4*>(ab + mm * lda + k);
       const float4 h = *p;
-      const float co = R.coef[cc][mm];
-      const float4 dv = make_float4(co * w.x * act_dz(P.act_q, h.x), co * w.y * act_dz(P.act_q, h.y), co * w.z * act_dz(P.act_q, h.z),
-                                    co * w.w * act_dz(P.act_q, h.w));
+      const float co = coef[mm];
+      const float4 dv = make_float4(co * w.x * act_dz(act, h.x), co * w.y * act_dz(act, h.y), co * w.z * act_dz(act, h.z),
+                                    co * w.w * act_dz(act, h.w));
       *p = dv;
-      if (mine && c.row0 + mm < B) *reinterpret_cast<float4*>(c.base + P.dq_last[cc] + (i64)(c.row0 + mm) * P.ld_hq + k) = dv;
+      if (mine && mm < nrows) *reinterpret_cast<float4*>(dq + (i64)mm * ld) = dv;
     }
     RP_TRACE(2910 + cc);
   }
@@ -854,6 +863,9 @@ __device__ __forceinline__ void rp_pi_bwd_impl(const RpCtx& c) {
   __syncthreads();
   float* ab = smem_raw + P.sm_abuf + P.ab_pi * P.abuf_floats;
   const bool mine = k >= n0g && k < n0g + NS;
+  // loop operands in registers before the first store (see rp_gather_rows)
+  const int lda = P.lda, act = P.act_pi, ld = P.ld_hpi, nrows = min(RP_RB, B - c.row0);
+  float* const dp = c.base + P.dp_last + (i64)c.row0 * ld + k;
   for (int mm = m0; mm < RP_RB; mm += mstep) {
     float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
@@ -863,11 +875,11 @@ __device__ __forceinline__ void rp_pi_bwd_impl(const RpCtx& c) {
         s.x = fmaf(gj, wl[j].x, s.x); s.y = fmaf(gj, wl[j].y, s.y); s.z = fmaf(gj, wl[j].z, s.z); s.w = fmaf(gj, wl[j].w, s.w);
       }
     }
-    float4* p = reinterpret_cast<float4*>(ab + mm * P.lda + k);
+    float4* p = reinterpret_cast<float4*>(ab + mm * lda + k);
     const float4 h = *p;
-    const float4 dv = make_float4(s.x * act_dz(P.act_pi, h.x), s.y * act_dz(P.act_pi, h.y), s.z * act_dz(P.act_pi, h.z), s.w * act_dz(P.act_pi, h.w));
+    const float4 dv = make_float4(s.x * act_dz(act, h.x), s.y * act_dz(act, h.y), s.z * act_dz(act, h.z), s.w * act_dz(act, h.w));
     *p = dv;
-    if (mine && c.row0 + mm < B) *reinterpret_cast<float4*>(c.base + P.dp_last + (i64)(c.row0 + mm) * P.ld_hpi + k) = dv;
+    if (mine && mm < nrows) *reinterpret_cast<float4*>(dp + (i64)mm * ld) = dv;
   }
   __syncthreads();
 }
