@@ -523,7 +523,8 @@ static int engine_setup_rp_tma(Engine* e) {
   void* fn = nullptr;
   cudaDriverEntryPointQueryResult qres;
   const bool have = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) == cudaSuccess && fn;
-  std::vector<CUtensorMap> maps(P.n_jobs + 2 * plan.n_ops);
+  const int nj = 2 * P.n_jobs;                                   // job j: map 2j, and 2j + 1 for the second slice of a pair
+  std::vector<CUtensorMap> maps(nj + 2 * plan.n_ops);
   memset(maps.data(), 0, sizeof(CUtensorMap) * maps.size());
   bool ok = have;
   for (int j = 0; ok && j < P.n_jobs; ++j) {
@@ -534,8 +535,10 @@ static int engine_setup_rp_tma(Engine* e) {
     box[0] = 32; box[1] = 32;                                   // 32 x 32 tiles (4 KB), one per warp
     if (!jb.bkm) { dims[0] = jb.K; dims[1] = jb.N; }            // W [N][K]: 32 rows n x 32 k
     else { dims[0] = jb.N; dims[1] = jb.K; }                    // W [K][N]: 32 rows k x 32 columns n
-    ok = ((TcEncodeFn)fn)(&maps[j], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, e->arena + jb.w, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    for (int h = 0; ok && h <= (jb.pair && jb.w2_off > 0 ? 1 : 0); ++h)
+      ok = ((TcEncodeFn)fn)(&maps[h ? jb.map2 : jb.map], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, e->arena + (h ? jb.w2 : jb.w), dims, strides, box, estr,
+                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
   }
   if (!ok) { for (int j = 0; j < P.n_jobs; ++j) P.jobs[j].tma = 0; cudaGetLastError(); }
   // dW operands: dy [batch][M] and x [batch][N], boxes of 64 batch rows x 32 columns
@@ -549,11 +552,11 @@ static int engine_setup_rp_tma(Engine* e) {
     for (int w = 0; ok_dw && w < 2; ++w) {
       cuuint64_t dims[2] = {(cuuint64_t)(w ? o.N : o.M), (cuuint64_t)o.K}, strides[1] = {(cuuint64_t)(w ? o.b_sk : o.a_sk) * 4};
       cuuint32_t box[2] = {32, (cuuint32_t)RP_DW_CHUNK}, estr[2] = {1, 1};
-      ok_dw = ((TcEncodeFn)fn)(&maps[P.n_jobs + 2 * k + w], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, e->arena + (w ? o.b : o.a), dims, strides, box, estr,
+      ok_dw = ((TcEncodeFn)fn)(&maps[nj + 2 * k + w], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, e->arena + (w ? o.b : o.a), dims, strides, box, estr,
                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
     }
-    if (ok_dw) { o.i[2] = P.n_jobs + 2 * k + 1; o.i[3] = P.n_jobs + 2 * k + 2; }
+    if (ok_dw) { o.i[2] = nj + 2 * k + 1; o.i[3] = nj + 2 * k + 2; }
   }
   if (!ok_dw) { for (int k = 0; k < plan.n_ops; ++k) { plan.ops[k].i[2] = 0; plan.ops[k].i[3] = 0; } cudaGetLastError(); }
   // one-row output layers (the critics' heads) as 128-column vector tiles (rp_dw_vec_tile) instead of 32 x 32 tiles with one valid

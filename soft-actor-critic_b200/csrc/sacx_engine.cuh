@@ -845,24 +845,60 @@ struct Engine {
     memset(&P, 0, sizeof P);
     const int O = cfg.obs_dim, A = cfg.act_dim, Lq = q1.L(), Lp = pi.L();
     bool overflow = false;
-    int wmax = 0;
+    // wmax: floats of the widest weight slice (sizes the slots); red: floats of the k-group reduction buffer.
+    // wcap: a pair with two slices runs as one job only if both fit in a slot sized for single slices (set by a first pass)
+    int wmax = 0, red = 0, wcap = 0;
     auto step = [&](int row_op) {
       if (P.n_steps_a + P.n_steps_c >= RP_MAX_STEPS) { overflow = true; return; }
       RpStep& st = P.steps[P.n_steps_a + P.n_steps_c];
       st.row_op = row_op; st.job0 = P.n_jobs; st.njobs = 0; st.load0 = P.n_loads; st.nloads = 0;
     };
     auto cur = [&]() -> RpStep& { return P.steps[P.n_steps_a + P.n_steps_c]; };
+    // TMA-staged slice (sacx_rowpar.cuh): 32 columns per CTA, rows the tensor map can address
+    auto tma_ok = [&](const RpJob& j, i64 w) { return rp_tma && j.N / RP_CS == 32 && (j.w_ld % 4) == 0 && (w % 4) == 0 && j.K <= 256; };
+    auto slice_floats = [&](const RpJob& j, bool tma) {
+      const int NS = j.N / RP_CS;
+      if (tma) return j.bkm ? j.K * 32 : ((j.K + 31) / 32) * 1024;
+      return j.bkm ? j.K * NS : NS * (j.Kp + 4);
+    };
+    // two slices of a pair: a TMA-staged second slice starts at a 1 KB granule (swizzled tiles) behind the first, placed so that
+    // the cp.async layout fits as well (the slices fall back to it when a tensor map cannot be encoded); a cp.async-only slice
+    // needs 16-byte alignment only
+    auto pair_w2_off = [&](const RpJob& j, bool tma) {
+      if (!tma) return (slice_floats(j, false) + 3) & ~3;
+      return (std::max(slice_floats(j, true), slice_floats(j, false)) + 255) & ~255;
+    };
     auto add_job = [&](const RpJob& j) {
       if (P.n_jobs >= RP_MAX_JOBS) { overflow = true; return; }
       const int NS = j.N / RP_CS;
       RpJob jj = j;
-      // TMA-staged slice (sacx_rowpar.cuh): 32 columns per CTA, rows the tensor map can address; map index = job index
-      jj.tma = (rp_tma && NS == 32 && (j.w_ld % 4) == 0 && (j.w % 4) == 0 && j.K <= 256) ? 1 : 0;
-      jj.map = P.n_jobs;
+      const bool sep = j.pair && j.w2 != j.w;
+      jj.tma = (tma_ok(j, j.w) && (!sep || tma_ok(j, j.w2))) ? 1 : 0;
+      jj.map = 2 * P.n_jobs; jj.map2 = 2 * P.n_jobs + 1;      // tensor maps of the two halves' slices
+      jj.w2_off = sep ? pair_w2_off(j, jj.tma) : 0;
       P.jobs[P.n_jobs++] = jj; cur().njobs++;
-      const int cp_floats = j.bkm ? j.K * NS : NS * (j.Kp + 4);
-      const int tma_floats = j.bkm ? j.K * 32 : ((j.K + 31) / 32) * 1024;
-      wmax = std::max(wmax, jj.tma ? tma_floats : cp_floats);
+      wmax = std::max(wmax, jj.w2_off + (sep ? jj.w2_off : slice_floats(j, jj.tma)));
+      red = std::max(red, (1 + j.pair) * (64 / NS) * RP_RB * (NS + 8));      // k-groups (8 warps x 8 columns / NS) x [16][NS + 8]
+    };
+    // two independent forward jobs of the same shape as one pair job (fewer fixed per-job costs: waits, barriers, issue,
+    // reduction and epilogue). Either the weight slice is shared (pi(s') / pi(s): W, bias and head weights are the policy's), or
+    // each half has its own slice and bias and no projection (the critics' first layers: never the last hidden layer).
+    // Pairing shortens the job sequence, and rp_run_steps issues job j + 2's operands when job j starts. A backward job's
+    // aux operand (the saved activations of layer l - 1) must therefore come from a job at least three positions earlier.
+    // That holds because the last hidden layer, whose backward job follows right after, carries the head projection and
+    // so never pairs with its twin: its two single jobs keep that distance for the layer in front of it.
+    auto add_pair = [&](const RpJob& a, const RpJob& b) {
+      const bool shared = a.w == b.w && a.bias == b.bias && a.proj_w == b.proj_w;
+      bool ok = wcap > 0 && !a.bkm && !b.bkm && a.K == b.K && a.N == b.N && a.act == b.act && a.w_ld == b.w_ld &&
+                a.out_ld == b.out_ld && a.proj_J == b.proj_J && (shared || a.proj_J == 0);
+      if (ok && !shared) {
+        const bool tma = tma_ok(a, a.w) && tma_ok(a, b.w);
+        ok = 2 * pair_w2_off(a, tma) <= wcap && (!tma || 2 * ((a.K + 31) / 32) <= 8);      // (one TMA tile per warp)
+      }
+      if (!ok) { add_job(a); add_job(b); return; }
+      RpJob j = a;
+      j.pair = 1; j.a_src2 = b.a_src; j.out2 = b.out; j.proj_slot2 = b.proj_slot; j.w2 = b.w; j.bias2 = b.bias;
+      add_job(j);
     };
     auto add_load = [&](i64 off, int ld, int K, int abuf) {
       if (P.n_loads >= RP_MAX_LOADS) { overflow = true; return; }
@@ -889,86 +925,90 @@ struct Engine {
       return j;
     };
     const i64 tsh = T0 - q1.begin;
-    // ---------------- phase A: pi(s'), pi(s), Q(s,a) forward; target critics; Bellman target; critics' backward
-    step(RPR_GATHER);
-    add_job(fwd(pi, 0, 0, RPS_XS2, a_pit, RPP_PI_T));
-    add_job(fwd(pi, 0, 0, RPS_XSA, a_pia, RPP_PI_A));
-    for (int c = 0; c < 2; ++c) add_job(fwd(c ? q2 : q1, 0, 0, RPS_XSA, a_q[c], RPP_Q1 + c));
-    P.n_steps_a++;
-    for (int l = 1; l < std::max(Lp, Lq); ++l) {
-      step(RPR_NONE);
-      if (l < Lp) {
-        add_load(a_pit.h[l - 1], a_pit.ld[l - 1], pi.dims[l], 0); add_job(fwd(pi, l, 0, 0, a_pit, RPP_PI_T));
-        add_load(a_pia.h[l - 1], a_pia.ld[l - 1], pi.dims[l], 1); add_job(fwd(pi, l, 0, 1, a_pia, RPP_PI_A));
-      }
-      if (l < Lq)
-        for (int c = 0; c < 2; ++c) {
-          add_load(a_q[c].h[l - 1], a_q[c].ld[l - 1], q1.dims[l], 2 + c);
-          add_job(fwd(c ? q2 : q1, l, 0, 2 + c, a_q[c], RPP_Q1 + c));
+    auto emit = [&]() {
+      // ---------------- phase A: pi(s'), pi(s), Q(s,a) forward; target critics; Bellman target; critics' backward
+      step(RPR_GATHER);
+      add_pair(fwd(pi, 0, 0, RPS_XS2, a_pit, RPP_PI_T), fwd(pi, 0, 0, RPS_XSA, a_pia, RPP_PI_A));
+      add_pair(fwd(q1, 0, 0, RPS_XSA, a_q[0], RPP_Q1), fwd(q2, 0, 0, RPS_XSA, a_q[1], RPP_Q2));
+      P.n_steps_a++;
+      for (int l = 1; l < std::max(Lp, Lq); ++l) {
+        step(RPR_NONE);
+        if (l < Lp) {
+          add_load(a_pit.h[l - 1], a_pit.ld[l - 1], pi.dims[l], 0);
+          add_load(a_pia.h[l - 1], a_pia.ld[l - 1], pi.dims[l], 1);
+          add_pair(fwd(pi, l, 0, 0, a_pit, RPP_PI_T), fwd(pi, l, 0, 1, a_pia, RPP_PI_A));
         }
-      P.n_steps_a++;
-    }
-    step(RPR_PI_HEADS);
-    for (int c = 0; c < 2; ++c) add_job(fwd(c ? q2 : q1, 0, tsh, RPS_XS2, a_qt[c], RPP_QT1 + c));
-    P.n_steps_a++;
-    for (int l = 1; l < Lq; ++l) {
-      step(RPR_NONE);
-      for (int c = 0; c < 2; ++c) {
-        add_load(a_qt[c].h[l - 1], a_qt[c].ld[l - 1], q1.dims[l], c);
-        add_job(fwd(c ? q2 : q1, l, tsh, c, a_qt[c], RPP_QT1 + c));
+        if (l < Lq) {
+          for (int c = 0; c < 2; ++c) add_load(a_q[c].h[l - 1], a_q[c].ld[l - 1], q1.dims[l], 2 + c);
+          add_pair(fwd(q1, l, 0, 2, a_q[0], RPP_Q1), fwd(q2, l, 0, 3, a_q[1], RPP_Q2));
+        }
+        P.n_steps_a++;
       }
+      step(RPR_PI_HEADS);
+      add_pair(fwd(q1, 0, tsh, RPS_XS2, a_qt[0], RPP_QT1), fwd(q2, 0, tsh, RPS_XS2, a_qt[1], RPP_QT2));
       P.n_steps_a++;
-    }
-    step(RPR_TARGET_CRITIC);
-    for (int c = 0; c < 2; ++c) {
-      add_load(a_q[c].h[Lq - 1], a_q[c].ld[Lq - 1], q1.dims[Lq], 2 + c);
-      add_job(bwd(c ? q2 : q1, Lq - 1, 2 + c, a_q[c], d_q[c], -1));
-    }
-    P.n_steps_a++;
-    for (int l = Lq - 2; l >= 1; --l) {
-      step(RPR_NONE);
+      for (int l = 1; l < Lq; ++l) {
+        step(RPR_NONE);
+        for (int c = 0; c < 2; ++c) add_load(a_qt[c].h[l - 1], a_qt[c].ld[l - 1], q1.dims[l], c);
+        add_pair(fwd(q1, l, tsh, 0, a_qt[0], RPP_QT1), fwd(q2, l, tsh, 1, a_qt[1], RPP_QT2));
+        P.n_steps_a++;
+      }
+      step(RPR_TARGET_CRITIC);
       for (int c = 0; c < 2; ++c) {
-        add_load(d_q[c][l], rup4(q1.dims[l + 1]), q1.dims[l + 1], c);
-        add_job(bwd(c ? q2 : q1, l, c, a_q[c], d_q[c], -1));
+        add_load(a_q[c].h[Lq - 1], a_q[c].ld[Lq - 1], q1.dims[Lq], 2 + c);
+        add_job(bwd(c ? q2 : q1, Lq - 1, 2 + c, a_q[c], d_q[c], -1));
       }
       P.n_steps_a++;
-    }
-    // ---------------- phase C: critics on (s, a~pi), routed dQ back to the action, policy backward
-    step(RPR_RELOAD);
-    for (int c = 0; c < 2; ++c) add_job(fwd(c ? q2 : q1, 0, 0, RPS_XPI, a_q[c], RPP_Q1 + c));
-    P.n_steps_c++;
-    for (int l = 1; l < Lq; ++l) {
-      step(RPR_NONE);
+      for (int l = Lq - 2; l >= 1; --l) {
+        step(RPR_NONE);
+        for (int c = 0; c < 2; ++c) {
+          add_load(d_q[c][l], rup4(q1.dims[l + 1]), q1.dims[l + 1], c);
+          add_job(bwd(c ? q2 : q1, l, c, a_q[c], d_q[c], -1));
+        }
+        P.n_steps_a++;
+      }
+      // ---------------- phase C: critics on (s, a~pi), routed dQ back to the action, policy backward
+      step(RPR_RELOAD);
+      add_pair(fwd(q1, 0, 0, RPS_XPI, a_q[0], RPP_Q1), fwd(q2, 0, 0, RPS_XPI, a_q[1], RPP_Q2));
+      P.n_steps_c++;
+      for (int l = 1; l < Lq; ++l) {
+        step(RPR_NONE);
+        for (int c = 0; c < 2; ++c) add_load(a_q[c].h[l - 1], a_q[c].ld[l - 1], q1.dims[l], c);
+        add_pair(fwd(q1, l, 0, 0, a_q[0], RPP_Q1), fwd(q2, l, 0, 1, a_q[1], RPP_Q2));
+        P.n_steps_c++;
+      }
+      step(RPR_ACTOR_Q);
       for (int c = 0; c < 2; ++c) {
-        add_load(a_q[c].h[l - 1], a_q[c].ld[l - 1], q1.dims[l], c);
-        add_job(fwd(c ? q2 : q1, l, 0, c, a_q[c], RPP_Q1 + c));
+        add_load(a_q[c].h[Lq - 1], a_q[c].ld[Lq - 1], q1.dims[Lq], 2 + c);
+        add_job(bwd(c ? q2 : q1, Lq - 1, 2 + c, a_q[c], d_q[c], Lq - 1 == 1 ? RPP_DA1 + c : -1));
       }
       P.n_steps_c++;
-    }
-    step(RPR_ACTOR_Q);
-    for (int c = 0; c < 2; ++c) {
-      add_load(a_q[c].h[Lq - 1], a_q[c].ld[Lq - 1], q1.dims[Lq], 2 + c);
-      add_job(bwd(c ? q2 : q1, Lq - 1, 2 + c, a_q[c], d_q[c], Lq - 1 == 1 ? RPP_DA1 + c : -1));
-    }
-    P.n_steps_c++;
-    for (int l = Lq - 2; l >= 1; --l) {
-      step(RPR_NONE);
-      for (int c = 0; c < 2; ++c) {
-        add_load(d_q[c][l], rup4(q1.dims[l + 1]), q1.dims[l + 1], c);
-        add_job(bwd(c ? q2 : q1, l, c, a_q[c], d_q[c], l == 1 ? RPP_DA1 + c : -1));
+      for (int l = Lq - 2; l >= 1; --l) {
+        step(RPR_NONE);
+        for (int c = 0; c < 2; ++c) {
+          add_load(d_q[c][l], rup4(q1.dims[l + 1]), q1.dims[l + 1], c);
+          add_job(bwd(c ? q2 : q1, l, c, a_q[c], d_q[c], l == 1 ? RPP_DA1 + c : -1));
+        }
+        P.n_steps_c++;
       }
+      step(RPR_PI_BWD);
+      add_load(a_pia.h[Lp - 1], a_pia.ld[Lp - 1], pi.dims[Lp], 0);
+      add_job(bwd(pi, Lp - 1, 0, a_pia, d_p, -1));
       P.n_steps_c++;
-    }
-    step(RPR_PI_BWD);
-    add_load(a_pia.h[Lp - 1], a_pia.ld[Lp - 1], pi.dims[Lp], 0);
-    add_job(bwd(pi, Lp - 1, 0, a_pia, d_p, -1));
-    P.n_steps_c++;
-    for (int l = Lp - 2; l >= 1; --l) {
-      step(RPR_NONE);
-      add_load(d_p[l], rup4(pi.dims[l + 1]), pi.dims[l + 1], 1);
-      add_job(bwd(pi, l, 1, a_pia, d_p, -1));
-      P.n_steps_c++;
-    }
+      for (int l = Lp - 2; l >= 1; --l) {
+        step(RPR_NONE);
+        add_load(d_p[l], rup4(pi.dims[l + 1]), pi.dims[l + 1], 1);
+        add_job(bwd(pi, l, 1, a_pia, d_p, -1));
+        P.n_steps_c++;
+      }
+    };
+    // first pass with single jobs only: the widest single slice sizes the slots, and a pair with two slices runs as one job
+    // only if they fit in one of those slots
+    emit();
+    wcap = wmax;
+    P.n_steps_a = P.n_steps_c = P.n_jobs = P.n_loads = 0;
+    wmax = red = 0; overflow = false;
+    emit();
     if (overflow) { rp_why = "program tables too small"; return false; }
     // ---------------- geometry, row-op operands
     P.O = O; P.A = A; P.Hq = q1.dims[Lq]; P.Hpi = pi.dims[Lp]; P.ld_hq = rup4(P.Hq); P.ld_hpi = rup4(P.Hpi);
@@ -996,7 +1036,7 @@ struct Engine {
     P.sm_xbuf = off; off += 3 * RP_RB * P.ldx;
     off = (off + 255) & ~255;
     P.sm_wslot = off; off += RP_NWSLOT * P.wslot_floats;
-    P.sm_red = off; off += RP_RED;
+    P.sm_red = off; off += red;
     P.sm_otile = off; P.sm_pw = off;
     off = std::max(off, WSM_FLOATS + CfgSmall::SMEM_FLOATS);
     off = std::max(off, RP_DW_SMEM);      // the dW tiles alias the same region

@@ -31,7 +31,6 @@ constexpr int RP_RB = 16;                        // rows per row block
 constexpr int RP_HMAX = 256;                     // widest hidden layer
 constexpr int RP_NABUF = 4;                      // full-row activation buffers [16][lda], lda = widest hidden + 4 (== 4 mod 32)
 constexpr int RP_NWSLOT = 3;                     // weight slots (forward slice [N/8][K+4] / backward [K][N/8])
-constexpr int RP_RED = 2048;
 constexpr int RP_MAXA = 8;                       // action dimension handled by the row ops
 constexpr int RP_MAX_GROUPS = 32;
 constexpr int RP_MAX_JOBS = 40, RP_MAX_STEPS = 28, RP_MAX_LOADS = 48, RP_MAX_DW_OPS = 16;
@@ -51,6 +50,11 @@ struct RpJob {
   int proj_J, proj_slot, proj_sj, proj_sn;      // projection of the output slice onto J weight vectors (0: none)
   int tma, map;            // tma = 1: the weight slice arrives by TMA (tensor map `map`, 128B-swizzled tiles) instead of cp.async
   i64 w, bias, out, aux, proj_w;                // arena offsets (-1: unused)
+  // pair = 1: a second, independent forward GEMM of the same shape rides in this job (pi(s') / pi(s), Q1 / Q2): its own input
+  // rows (a_src2), output, projection slot and -- when w2_off > 0 -- its own weight slice (at slot + w2_off, tensor map map2)
+  // and bias (epilogue operand + 32). Each half keeps the single job's k-groups and summation order: same bits.
+  int pair, a_src2, proj_slot2, map2, w2_off, pad_p;
+  i64 w2, bias2, out2;
 };
 struct RpLoad { i64 off; int ld, K, abuf, pad; };
 struct RpStep { int row_op, job0, njobs, load0, nloads, pad0, pad1, pad2; };
@@ -217,24 +221,29 @@ __device__ __forceinline__ void rp_issue_job(const RpJob& jb, float* __restrict_
   float* pws = slot + P.wslot_floats - 512;
   const int J = jb.proj_J, cl = jb.ns_log2 - 2;            // chunks per NS-wide row = NS / 4 = 1 << cl
   const int B = c.args->hp.B;
+  const bool sep = jb.pair && jb.w2_off > 0;               // a pair with a second weight slice (and bias) of its own
   if (jb.tma) {
     if (lane == 0) {
       // one 32 x 32 tile (4 KB) per warp: the issue cost (~100 cycles per tile on the TMA queue) is spread over the warps.
       // The slot was last READ with ordinary loads, all complete before the caller's barrier -- the usual consumer-release /
       // producer-acquire pattern of TMA pipelines, no proxy fence (it would also wait for the cp.async copies in flight).
       uint64_t* bar = c.wbar + slot_idx;
-      const int slabs = (jb.K + 31) >> 5;                  // K <= 256: at most 8
-      if (warp < slabs) {
-        const char* map = reinterpret_cast<const char*>(c.args->rp_maps) + (size_t)jb.map * 128;
+      const int slabs = (jb.K + 31) >> 5;                  // K <= 256: at most 8 (a pair with two slices: 2 x slabs <= 8)
+      if (warp < (sep ? 2 * slabs : slabs)) {
+        const bool h = warp >= slabs;                      // second slice of a pair: tiles at slot + w2_off
+        const int wt = h ? warp - slabs : warp;
+        const char* map = reinterpret_cast<const char*>(c.args->rp_maps) + (size_t)(h ? jb.map2 : jb.map) * 128;
+        float* dst = slot + (h ? jb.w2_off : 0) + wt * 1024;
         rp_mbar_expect_tx(bar, 4096u);
-        if (!jb.bkm) rp_tma_load(slot + warp * 1024, map, bar, 32 * warp, n0g);
-        else rp_tma_load(slot + warp * 1024, map, bar, n0g, 32 * warp);
+        if (!jb.bkm) rp_tma_load(dst, map, bar, 32 * wt, n0g);
+        else rp_tma_load(dst, map, bar, n0g, 32 * wt);
       } else {
         asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"((uint32_t)__cvta_generic_to_shared(bar)) : "memory");
       }
     }
     if (!jb.bkm) {
       if (tid < (1 << cl)) cp_async16(eps + (tid << 2), base + jb.bias + n0g + (tid << 2), 16);
+      else if (sep && tid >= 32 && tid < 32 + (1 << cl)) cp_async16(eps + 32 + ((tid - 32) << 2), base + jb.bias2 + n0g + ((tid - 32) << 2), 16);
     } else if (tid < (RP_RB << cl)) {
       const int m = tid >> cl, cc = (tid & ((1 << cl) - 1)) << 2;
       const bool ok = c.row0 + m < B;
@@ -242,24 +251,30 @@ __device__ __forceinline__ void rp_issue_job(const RpJob& jb, float* __restrict_
     }
   } else if (!jb.bkm) {
     const int ldw = jb.Kp + 4;
-    const bool vec = ((jb.K & 3) == 0) && ((jb.w & 3) == 0) && ((jb.w_ld & 3) == 0);
-    if (vec) {
-      const int cpr = jb.Kp >> 2;            // 16-byte chunks per row (the last one may be zero padding)
-      for (int n = warp; n < NS; n += 8) {
-        const float* src = W + (i64)(n0g + n) * jb.w_ld;
-        float* dst = slot + n * ldw;
-        for (int ch = lane; ch < cpr; ch += 32) {
-          const int k = ch << 2;
-          if (k < jb.K) cp_async16(dst + k, src + k, 16);
-          else *reinterpret_cast<float4*>(dst + k) = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int h = 0; h <= (int)sep; ++h) {
+      const i64 wo = h ? jb.w2 : jb.w;
+      const float* __restrict__ Wh = base + wo;
+      float* sl = slot + (h ? jb.w2_off : 0);
+      const bool vec = ((jb.K & 3) == 0) && ((wo & 3) == 0) && ((jb.w_ld & 3) == 0);
+      if (vec) {
+        const int cpr = jb.Kp >> 2;            // 16-byte chunks per row (the last one may be zero padding)
+        for (int n = warp; n < NS; n += 8) {
+          const float* src = Wh + (i64)(n0g + n) * jb.w_ld;
+          float* dst = sl + n * ldw;
+          for (int ch = lane; ch < cpr; ch += 32) {
+            const int k = ch << 2;
+            if (k < jb.K) cp_async16(dst + k, src + k, 16);
+            else *reinterpret_cast<float4*>(dst + k) = make_float4(0.f, 0.f, 0.f, 0.f);
+          }
         }
+      } else {
+        for (int n = warp; n < NS; n += 8)
+          for (int k = lane; k < jb.Kp; k += 32)
+            sl[n * ldw + k] = (k < jb.K) ? __ldcg(Wh + (i64)(n0g + n) * jb.w_ld + k) : 0.f;
       }
-    } else {
-      for (int n = warp; n < NS; n += 8)
-        for (int k = lane; k < jb.Kp; k += 32)
-          slot[n * ldw + k] = (k < jb.K) ? __ldcg(W + (i64)(n0g + n) * jb.w_ld + k) : 0.f;
     }
     if (tid < (1 << cl)) cp_async16(eps + (tid << 2), base + jb.bias + n0g + (tid << 2), 16);
+    else if (sep && tid >= 32 && tid < 32 + (1 << cl)) cp_async16(eps + 32 + ((tid - 32) << 2), base + jb.bias2 + n0g + ((tid - 32) << 2), 16);
   } else {
     // [K][NS], 8-column groups XOR-swizzled by the row so that the (k = t, n = g) fragment reads hit 32 banks
     const int sh = 5 - jb.ns_log2;
@@ -396,65 +411,78 @@ __device__ __forceinline__ void rp_job(const RpJob& jb, const RpCtx& c, int wslo
   const RpProgram& P = *c.P;
   const int tid = threadIdx.x, NS = 1 << jb.ns_log2, n0g = c.rank << jb.ns_log2, RS = NS + 8, KG = 64 >> jb.ns_log2;
   const int B = c.args->hp.B;
-  const float* As;
-  int lda;
-  if (jb.a_src < RP_NABUF) { As = smem_raw + P.sm_abuf + jb.a_src * P.abuf_floats; lda = P.lda; }
-  else { As = smem_raw + P.sm_xbuf + (jb.a_src - RPS_XSA) * RP_RB * P.ldx; lda = P.ldx; }
   const float* Bs = smem_raw + P.sm_wslot + wslot_idx * P.wslot_floats;
   const float* eps = Bs + P.wslot_floats - 1024;
   const float* pws = Bs + P.wslot_floats - 512;
   float* red = smem_raw + P.sm_red;
+  const int red_half = KG * 16 * RS;                 // reduction floats of one half of a pair
   RP_TRACE(4500);
-  rp_job_math(jb, rp_saddr(As), lda, rp_saddr(Bs), red);
+#pragma unroll 1
+  for (int h = 0; h <= jb.pair; ++h) {               // the halves of a pair one after the other: the single job's registers
+    const int src = h ? jb.a_src2 : jb.a_src;
+    const float* As;
+    int lda;
+    if (src < RP_NABUF) { As = smem_raw + P.sm_abuf + src * P.abuf_floats; lda = P.lda; }
+    else { As = smem_raw + P.sm_xbuf + (src - RPS_XSA) * RP_RB * P.ldx; lda = P.ldx; }
+    rp_job_math(jb, rp_saddr(As), lda, rp_saddr(Bs + (h ? jb.w2_off : 0)), red + h * red_half);
+  }
   RP_TRACE(4600);
   __syncthreads();
   RP_TRACE(4650);
-  // thread owns outputs (m, n) and (m, n + 1) of the 16 x NS slice; the NS / 2 lanes of a row sit in one warp
+  // thread owns outputs (m, n) and (m, n + 1) of the 16 x NS slice (of each half); the NS / 2 lanes of a row sit in one warp
   const int e = tid * 2, m = e >> jb.ns_log2, n = e & (NS - 1);
+  // (a rolled loop over the halves on purpose: the kernel lives on instruction fetch, and an unrolled second copy of this
+  //  epilogue made every job slower -- DESIGN.md section 4.2, round 5)
   if (e < RP_RB * NS) {               // warp-uniform
-    float2 s = make_float2(0.f, 0.f);
-    for (int q = 0; q < KG; ++q) {
-      const float2 p = *reinterpret_cast<const float2*>(red + (q * 16 + m) * RS + n);
-      s.x += p.x; s.y += p.y;
-    }
-    float2 v;
-    if (!jb.bkm) {
-      const float2 bb = *reinterpret_cast<const float2*>(eps + n);
-      v = make_float2(act_fwd(jb.act, s.x + bb.x), act_fwd(jb.act, s.y + bb.y));
-    } else {
-      const float2 ax = *reinterpret_cast<const float2*>(eps + m * NS + n);
-      v = make_float2(s.x * act_dz(jb.act, ax.x), s.y * act_dz(jb.act, ax.y));
-    }
-    if (c.row0 + m < B && jb.out >= 0) *reinterpret_cast<float2*>(c.base + jb.out + (i64)(c.row0 + m) * jb.out_ld + n0g + n) = v;
-    const int J = jb.proj_J;
-    if (J > 0) {
-      // projection of the row's slice onto J weight vectors: butterfly over the row's lanes (fixed order: deterministic);
-      // share of CTA `rank` goes to [rank][m][j] of the group's scratch, summed in rank order by every reader
-      const int lpr = NS >> 1, r = (tid & 31) & (lpr - 1);
-      float* dst = c.part + P.part_off[jb.proj_slot] + (c.rank * RP_RB + m) * J;
-      if (J == 1) {                    // critic heads: one weight vector, one butterfly
-        const float2 w = *reinterpret_cast<const float2*>(pws + n);
-        float p1 = fmaf(v.x, w.x, v.y * w.y);
-        for (int o = lpr >> 1; o > 0; o >>= 1) p1 += __shfl_xor_sync(0xffffffffu, p1, o);
-        if (r == 0) dst[0] = p1;
-      } else
-      for (int j0 = 0; j0 < J; j0 += 8) {
-        float p[8];
+#pragma unroll 1
+    for (int h = 0; h <= jb.pair; ++h) {
+      const float* rh = red + h * red_half;
+      float2 s = make_float2(0.f, 0.f);
+      for (int q = 0; q < KG; ++q) {
+        const float2 p = *reinterpret_cast<const float2*>(rh + (q * 16 + m) * RS + n);
+        s.x += p.x; s.y += p.y;
+      }
+      float2 v;
+      if (!jb.bkm) {
+        const float2 bb = *reinterpret_cast<const float2*>(eps + (h && jb.w2_off ? 32 : 0) + n);
+        v = make_float2(act_fwd(jb.act, s.x + bb.x), act_fwd(jb.act, s.y + bb.y));
+      } else {
+        const float2 ax = *reinterpret_cast<const float2*>(eps + m * NS + n);
+        v = make_float2(s.x * act_dz(jb.act, ax.x), s.y * act_dz(jb.act, ax.y));
+      }
+      const i64 out = h ? jb.out2 : jb.out;
+      if (c.row0 + m < B && out >= 0) *reinterpret_cast<float2*>(c.base + out + (i64)(c.row0 + m) * jb.out_ld + n0g + n) = v;
+      const int J = jb.proj_J;
+      if (J > 0) {
+        // projection of the row's slice onto J weight vectors: butterfly over the row's lanes (fixed order: deterministic);
+        // share of CTA `rank` goes to [rank][m][j] of the group's scratch, summed in rank order by every reader.
+        // (Both halves of a pair that projects share the weight slice, hence the projection weights.)
+        const int lpr = NS >> 1, r = (tid & 31) & (lpr - 1);
+        float* dst = c.part + P.part_off[h ? jb.proj_slot2 : jb.proj_slot] + (c.rank * RP_RB + m) * J;
+        if (J == 1) {                    // critic heads: one weight vector, one butterfly
+          const float2 w = *reinterpret_cast<const float2*>(pws + n);
+          float p1 = fmaf(v.x, w.x, v.y * w.y);
+          for (int o = lpr >> 1; o > 0; o >>= 1) p1 += __shfl_xor_sync(0xffffffffu, p1, o);
+          if (r == 0) dst[0] = p1;
+        } else
+        for (int j0 = 0; j0 < J; j0 += 8) {
+          float p[8];
 #pragma unroll
-        for (int jj = 0; jj < 8; ++jj) {
-          p[jj] = 0.f;
-          if (j0 + jj < J) {
-            const float2 w = *reinterpret_cast<const float2*>(pws + (j0 + jj) * NS + n);
-            p[jj] = fmaf(v.x, w.x, v.y * w.y);
+          for (int jj = 0; jj < 8; ++jj) {
+            p[jj] = 0.f;
+            if (j0 + jj < J) {
+              const float2 w = *reinterpret_cast<const float2*>(pws + (j0 + jj) * NS + n);
+              p[jj] = fmaf(v.x, w.x, v.y * w.y);
+            }
           }
-        }
-        for (int o = lpr >> 1; o > 0; o >>= 1) {
+          for (int o = lpr >> 1; o > 0; o >>= 1) {
 #pragma unroll
-          for (int jj = 0; jj < 8; ++jj) p[jj] += __shfl_xor_sync(0xffffffffu, p[jj], o);
-        }
+            for (int jj = 0; jj < 8; ++jj) p[jj] += __shfl_xor_sync(0xffffffffu, p[jj], o);
+          }
 #pragma unroll
-        for (int jj = 0; jj < 8; ++jj)
-          if (j0 + jj < J && r == ((j0 + jj) & (lpr - 1))) dst[j0 + jj] = p[jj];
+          for (int jj = 0; jj < 8; ++jj)
+            if (j0 + jj < J && r == ((j0 + jj) & (lpr - 1))) dst[j0 + jj] = p[jj];
+        }
       }
     }
   }
