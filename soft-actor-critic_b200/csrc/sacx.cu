@@ -179,7 +179,7 @@ static int engine_launch(Engine* e, int plan_id, int pb, int pe, int n_steps, co
   if (pe < 0) pe = hp.n_phases;
   RunArgs a = proto;
   a.arena = e->arena; a.agent_stride = e->stride; a.scal_off = e->scal_off; a.hp = e->hp;
-  a.n_agents = e->cfg.n_agents; a.barrier = e->d_barrier; a.ctas_per_agent = e->grid_x; a.barrier_mode = e->barrier_mode;
+  a.n_agents = e->cfg.n_agents; a.barrier = e->d_barrier; a.ctas_per_agent = e->grid_x;
   if (e->ring) {
     Ring* r = e->ring;
     a.ring = r->dev; a.ring_stride = r->stride; a.ring_capacity = r->cap;
@@ -288,7 +288,7 @@ static int engine_launch_rp(Engine* e, int n_steps, const RunArgs& proto) {
   { int rc = per_flush_pending(e); if (rc) return rc; }
   RunArgs a = proto;
   a.arena = e->arena; a.agent_stride = e->stride; a.scal_off = e->scal_off; a.hp = e->hp;
-  a.n_agents = 1; a.barrier = e->d_barrier; a.ctas_per_agent = e->rp_grid; a.barrier_mode = e->rp_barrier_mode;
+  a.n_agents = 1; a.barrier = e->d_barrier; a.ctas_per_agent = e->rp_grid;
   a.n_steps = n_steps; a.phase_begin = 0; a.phase_end = 2;
   if (e->ring) {
     Ring* r = e->ring;
@@ -298,7 +298,8 @@ static int engine_launch_rp(Engine* e, int n_steps, const RunArgs& proto) {
   a.rp_part = e->d_rp_part;
   a.rp_maps = e->d_rp_maps;
   // two counter sets of its own (behind the tile-parallel kernel's region of d_barrier): launch L spins on set L & 1 and zeroes the
-  // other one for launch L + 1; both start zeroed at create. (During stream capture the choice would be frozen into the graph.)
+  // other one for launch L + 1; both start zeroed at create. When the caller captures the stream into a graph, replays would
+  // freeze that alternation: a captured launch uses the first set and zeroes it in front of the kernel instead.
   {
     unsigned* sets = e->d_barrier + 64 * 2048;
     const size_t set_words = 64 * (1 + RP_MAX_GROUPS);
@@ -425,11 +426,11 @@ static int engine_setup_tc(Engine* e) {
             tp.other_ops = true;
             const int ty = pl.ops[i].type;
             const Op& oo = pl.ops[i];
-            const bool small_fwd = ty == OP_GEMM && oo.epi == EPI_FWD && oo.K <= SMALLK_MAX && oo.zout < 0 && oo.mode == 0 && oo.i[4] == 0 &&
-                                   oo.a_sk == 1 && oo.b_sk == 1 && oo.cfg >= 1;      // the light kernel's small_fwd_tile (64x64 tile grid)
+            const bool small_fwd = ty == OP_GEMM && oo.epi == EPI_FWD && oo.K <= SMALLK_MAX && oo.zout < 0 && oo.a_sk == 1 &&
+                                   oo.b_sk == 1 && oo.cfg >= 1;      // the light kernel's small_fwd_tile (64x64 tile grid)
             const bool small_dw = ty == OP_GEMM && oo.epi == EPI_DW && oo.M <= SMALLM_MAX && oo.K <= SMALLDW_MAXK && oo.a_sm == 1 && oo.b_sn == 1 &&
                                   oo.cfg >= 1 && !(oo.flags & DW_ATOMIC) && oo.i[0] <= 1;         // the light kernel's small_dw_tile
-            if ((ty == OP_GEMM && !small_fwd && !small_dw) || ty == OP_DW_HEAD || ty == OP_LOAD_EXT || ty == OP_NONE) tp.light = false;
+            if ((ty == OP_GEMM && !small_fwd && !small_dw) || ty == OP_LOAD_EXT || ty == OP_NONE) tp.light = false;
             if (pass == 1 && id == PLAN_FUSED && ty == OP_GEMM && !small_fwd && !small_dw && getenv("SACX_TC_VERBOSE"))
               fprintf(stderr, "sacx: FFMA leftover in the fused plan: phase %d epi %d M %d N %d K %d a_sm %d a_sk %d b_sk %d b_sn %d\n", ph, oo.epi,
                       oo.M, oo.N, oo.K, oo.a_sm, oo.a_sk, oo.b_sk, oo.b_sn);
@@ -1014,7 +1015,7 @@ int sacx_agent_create(const sacx_config* cfg, float* arena_dev, sacx_agent_t* ou
   if ((rc = engine_setup_rp(&e))) { sacx_agent_destroy(h); return rc; }
   // launch geometry: one CTA per SM; a single agent spreads over the chip, a population gets one CTA per agent
   const size_t gemm_floats = e.large ? CfgLarge::SMEM_FLOATS : CfgSmall::SMEM_FLOATS;
-  e.smem_bytes = (int)(SMEM_OPS * sizeof(Op) + WSM_FLOATS * 4 + gemm_floats * 4 + XSM_FLOATS * 4);
+  e.smem_bytes = (int)(SMEM_OPS * sizeof(Op) + WSM_FLOATS * 4 + gemm_floats * 4);
   const void* fn = e.large ? (const void*)sacx_run_kernel<true> : (const void*)sacx_run_kernel<false>;
   SACX_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, e.smem_bytes));
   int per_sm = 0;
@@ -1052,13 +1053,6 @@ int sacx_agent_create(const sacx_config* cfg, float* arena_dev, sacx_agent_t* ou
   SACX_CUDA(cudaMemcpy(e.d_plans, e.h_plans.data(), sizeof(Plan) * N_PLANS, cudaMemcpyHostToDevice));
   SACX_CUDA(cudaMalloc((void**)&e.d_barrier, sizeof(unsigned) * 64 * 4096));
   SACX_CUDA(cudaMemset(e.d_barrier, 0, sizeof(unsigned) * 64 * 4096));
-  { const char* bm = getenv("SACX_BARRIER"); e.barrier_mode = bm ? atoi(bm) : 1; }
-  // row-parallel kernel: bit 1 = the 8-CTA group barrier polls its arrival counter, bit 2 = so does the grid barrier -- one L2 hop
-  // less than "the last arriver publishes a flag" (measured: 131.7 -> 127.1 us per update with both)
-  { const char* bm = getenv("SACX_RP_BARRIER"); e.rp_barrier_mode = bm ? atoi(bm) : 7; }
-  // graph replay of the host-path step is opt-in (SACX_GRAPH=1): measured on the B200 box it LOSES to four plain stream
-  // operations at this size -- 6186 vs 6444 updates/s end to end (cudaGraphLaunch costs the host more than it saves the device)
-  { const char* gm = getenv("SACX_GRAPH"); e.graph_mode = (gm && atoi(gm) != 0) ? 1 : 0; }
   SACX_CUDA(cudaMallocHost((void**)&e.pinned_metrics, sizeof(sacx_metrics)));
   if ((rc = engine_init_scalars(&e))) { sacx_agent_destroy(h); return rc; }
   *out = h;
@@ -1081,10 +1075,8 @@ int sacx_agent_destroy(sacx_agent_t h) {
   if (e.pinned_io) cudaFreeHost(e.pinned_io);
   if (e.dev_io) cudaFree(e.dev_io);
   for (auto& io : e.slots) {
-    if (io.gexec) cudaGraphExecDestroy(io.gexec);
     if (io.pinned) cudaFreeHost(io.pinned); if (io.dev) cudaFree(io.dev); if (io.done) cudaEventDestroy(io.done); if (io.copied) cudaEventDestroy(io.copied);
   }
-  if (e.cap_stream) cudaStreamDestroy(e.cap_stream);
   if (e.copy_stream) cudaStreamDestroy(e.copy_stream);
   delete h;
   return SACX_OK;
@@ -1260,7 +1252,6 @@ static int host_update_submit(Engine& e, int slot, const int64_t* idx, const flo
   const size_t total = b_idx + (e1 ? b_eps : 0) + (e2 ? b_eps : 0) + sizeof(AgentScalars) + 256;
   if (io.busy) { SACX_CUDA(cudaEventSynchronize(io.done)); io.busy = false; }
   if (total > io.bytes) {
-    if (io.gexec) { cudaGraphExecDestroy(io.gexec); io.gexec = nullptr; }       // its copy nodes point into the old buffers
     if (io.pinned) cudaFreeHost(io.pinned);
     if (io.dev) cudaFree(io.dev);
     io.pinned = io.dev = nullptr; io.bytes = 0;
@@ -1286,65 +1277,20 @@ static int host_update_submit(Engine& e, int slot, const int64_t* idx, const flo
   a.idx_ext = d_idx; a.eps1_ext = d_e1; a.eps2_ext = d_e2;
   const bool direct_metrics = e.rp;          // the row-parallel kernel writes the metrics block into the pinned slot itself
   if (direct_metrics) a.metrics_host = reinterpret_cast<float*>(hp + io.metrics_off);
-  // the stream operations of one step; `st` is the caller's stream, or the capture stream while the graph is recorded
   // The H2D copy goes on its own stream: the slot's device buffer is free (its previous kernel completed: io.done above), so the
   // copy of step t+1 overlaps the kernel of step t instead of sitting between two kernels on one stream (~10 us per step at
-  // batch 256); the kernel waits for io.copied. Inside a captured graph the copy stays an in-stream node.
-  auto enqueue = [&](cudaStream_t st, bool capturing) -> int {
-    const cudaStream_t keep = e.stream;
-    e.stream = st;
-    int r2 = SACX_OK;
-    do {
-      if (off) {
-        const cudaStream_t cs = capturing ? st : e.copy_stream;
-        if (cudaMemcpyAsync(dp, hp, off, cudaMemcpyHostToDevice, cs) != cudaSuccess) { r2 = fail(SACX_ERR_CUDA, "update_host: H2D copy failed"); break; }
-        if (!capturing && (cudaEventRecord(io.copied, cs) != cudaSuccess || cudaStreamWaitEvent(st, io.copied, 0) != cudaSuccess)) {
-          r2 = fail(SACX_ERR_CUDA, "update_host: H2D copy ordering failed"); break;
-        }
-      }
-      r2 = e.rp ? engine_launch_rp(&e, n_steps, a) : engine_launch(&e, PLAN_FUSED, 0, -1, n_steps, a, false);
-      if (r2) break;
-      // the step's result travels back right behind the kernel (metrics block of agent 0)
-      if (!direct_metrics &&
-          cudaMemcpyAsync(hp + io.metrics_off, e.arena + e.scal_off, sizeof(AgentScalars), cudaMemcpyDeviceToHost, st) != cudaSuccess)
-        r2 = fail(SACX_ERR_CUDA, "update_host: metrics D2H copy failed");
-    } while (0);
-    e.stream = keep;
-    return r2;
-  };
-  // graph replay for the single-launch paths (row-parallel kernel, tile-parallel persistent kernel); the tensor-core path is a
-  // sequence of ~40 launches per update whose grouping depends on the plan and stays on plain stream order
-  const bool graphable = e.graph_mode && (e.rp || !e.tc);
-  bool launched = false;
-  if (graphable) {
-    const unsigned long long key = ((unsigned long long)n_steps << 40) ^ ((unsigned long long)off << 8) ^ (idx ? 1ull : 0) ^ (e1 ? 2ull : 0) ^
-                                   (e2 ? 4ull : 0) ^ ((unsigned long long)(uintptr_t)(e.ring ? e.ring->dev : nullptr) << 3) ^
-                                   ((unsigned long long)(uintptr_t)dp << 1) ^ (e.rp ? 0x8000000000000000ull : 0);
-    if (!io.gexec || io.gkey != key) {
-      if (io.gexec) { cudaGraphExecDestroy(io.gexec); io.gexec = nullptr; }
-      bool ok = true;
-      if (!e.cap_stream) ok = cudaStreamCreateWithFlags(&e.cap_stream, cudaStreamNonBlocking) == cudaSuccess;
-      cudaGraph_t g = nullptr;
-      const long long launches_before = e.launches;
-      if (ok) ok = cudaStreamBeginCapture(e.cap_stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
-      if (ok) {
-        const int r2 = enqueue(e.cap_stream, true);
-        const cudaError_t ce = cudaStreamEndCapture(e.cap_stream, &g);
-        ok = (r2 == SACX_OK) && ce == cudaSuccess && g;
-      }
-      if (ok) ok = cudaGraphInstantiate(&io.gexec, g, 0) == cudaSuccess;
-      if (g) cudaGraphDestroy(g);
-      e.launches = launches_before;                      // recording is not launching
-      if (!ok) { cudaGetLastError(); io.gexec = nullptr; e.graph_mode = 0; }
-      else io.gkey = key;
-    }
-    if (io.gexec) {
-      SACX_CUDA(cudaGraphLaunch(io.gexec, e.stream));
-      ++e.launches;                                      // one fused-kernel launch per replay
-      launched = true;
-    }
+  // batch 256); the kernel waits for io.copied.
+  if (off) {
+    if (cudaMemcpyAsync(dp, hp, off, cudaMemcpyHostToDevice, e.copy_stream) != cudaSuccess) return fail(SACX_ERR_CUDA, "update_host: H2D copy failed");
+    if (cudaEventRecord(io.copied, e.copy_stream) != cudaSuccess || cudaStreamWaitEvent(e.stream, io.copied, 0) != cudaSuccess)
+      return fail(SACX_ERR_CUDA, "update_host: H2D copy ordering failed");
   }
-  if (!launched) { rc = enqueue(e.stream, false); if (rc) return rc; }
+  rc = e.rp ? engine_launch_rp(&e, n_steps, a) : engine_launch(&e, PLAN_FUSED, 0, -1, n_steps, a, false);
+  if (rc) return rc;
+  // the step's result travels back right behind the kernel (metrics block of agent 0)
+  if (!direct_metrics &&
+      cudaMemcpyAsync(hp + io.metrics_off, e.arena + e.scal_off, sizeof(AgentScalars), cudaMemcpyDeviceToHost, e.stream) != cudaSuccess)
+    return fail(SACX_ERR_CUDA, "update_host: metrics D2H copy failed");
   SACX_CUDA(cudaEventRecord(io.done, e.stream));
   io.busy = true;
   return SACX_OK;

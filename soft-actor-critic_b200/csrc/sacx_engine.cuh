@@ -51,7 +51,7 @@ struct Engine {
   sacx_config cfg;
   int n_sms = 0, max_ctas = 0;
   bool large = false, grads_atomic = false;
-  int grid_x = 1, grid_y = 1, smem_bytes = 0, barrier_mode = 1, rp_barrier_mode = 7;
+  int grid_x = 1, grid_y = 1, smem_bytes = 0;
   std::vector<sacx_tensor_desc> lay;
   i64 cur = 0, stride = 0;
   NetLayout pi, q1, q2;
@@ -60,9 +60,7 @@ struct Engine {
   // batch / scratch
   int ldx = 0;
   i64 x_sa, x_s2, x_pi, b_r, b_d, b_idx, b_eps1, b_eps2, b_lp2, b_lp, b_y, b_tq[2], b_q[2], b_qa[2], b_dout[2], b_loss[2], b_coef[2],
-      b_ploss, b_tz, b_se, b_mask, b_headz, b_headz_t, b_headz_a, b_dhead, b_part_q[2], b_part_qt[2], b_part_da[2];
-  int ntn_q = 0, ntn_q0 = 0;
-  bool fuse_rows = false;
+      b_ploss, b_tz, b_se, b_mask, b_headz, b_headz_t, b_headz_a, b_dhead;
   ActSet a_pit, a_pia, a_q[2], a_qt[2];
   i64 d_q[2][SACX_MAX_HIDDEN], d_p[SACX_MAX_HIDDEN];
   float* arena = nullptr;
@@ -78,14 +76,8 @@ struct Engine {
   struct IoSlot {
     void* pinned = nullptr; void* dev = nullptr; size_t bytes = 0, metrics_off = 0; cudaEvent_t done = nullptr; bool busy = false;
     cudaEvent_t copied = nullptr;         // the slot's H2D copy (on copy_stream) has landed
-    // the step (H2D of the index stream / normals -> barrier reset -> fused kernel -> metrics D2H) as an instantiated CUDA graph:
-    // every address in it is fixed per slot, so one submission is ONE cudaGraphLaunch instead of four stream operations
-    cudaGraphExec_t gexec = nullptr;
-    unsigned long long gkey = 0;          // what the graph was built for (n_steps, which streams are given, payload, ring identity)
   };
   cudaStream_t copy_stream = nullptr;     // host inputs of step t+1 travel here while the kernel of step t runs on `stream`
-  cudaStream_t cap_stream = nullptr;      // private stream the graphs are captured on (the caller's may be the legacy default stream)
-  int graph_mode = 1;                     // SACX_GRAPH=0 disables; set to 0 when capture / instantiation fails once
   IoSlot slots[2];
   unsigned long long host_calls = 0;
   bool pipelined_pending = false;
@@ -255,14 +247,6 @@ struct Engine {
       b_dout[c] = alloc("scr.dout" + s, B, 1, 4);        // row stride 4: the dW tile reads it as a 16B-aligned [batch][1] operand
       b_loss[c] = alloc("scr.lossrow" + s, 1, B);
       b_coef[c] = alloc("scr.coef" + s, B, 1, 4);         // actor phase: routed dQ coefficient per row (tensor-core plans)
-    }
-    ntn_q = (cfg.hidden_q[cfg.n_hidden_q - 1] + 31) / 32;      // head shares per row: one per 32-wide column tile
-    ntn_q0 = (cfg.hidden_q[0] + 31) / 32;
-    for (int c = 0; c < 2; ++c) {
-      const std::string s = std::to_string(c + 1);
-      b_part_q[c] = alloc("part.q" + s, ntn_q, B);
-      b_part_qt[c] = alloc("part.qt" + s, ntn_q, B);
-      b_part_da[c] = alloc("part.da" + s, ntn_q0 * B, A);
     }
     b_ploss = alloc("scr.plossrow", 1, B);
     b_tz = alloc("scr.tz", B, A);
@@ -662,163 +646,6 @@ struct Engine {
     emit_actor_tail(pb, AD, 1 | 2 | 4 | 8);
   }
 
-  // ---- fused-rows plan (sacx_fused.cuh): row phases folded into the GEMM tiles -------------------------------
-  bool can_fuse_rows() const {
-    // opt-in (SACX_FUSE_ROWS=1): 13 phases instead of 16, but the generating tiles' one-shot prologue/transform code
-    // is instruction-fetch bound today and the plan measures 5% slower than the unfused one (DESIGN.md section 4)
-    const char* env = getenv("SACX_FUSE_ROWS");
-    if (!env || atoi(env) == 0) return false;
-    if (cfg.n_agents != 1 || large || q1.L() < 2 || pi.L() < 2) return false;
-    if (act_needs_z(q1.act_h) || act_needs_z(pi.act_h)) return false;
-    if (cfg.act_dim > 8 || cfg.batch_size > 8192) return false;
-    for (int l = 1; l <= q1.L(); ++l) if (q1.dims[l] % 4) return false;
-    for (int l = 1; l <= pi.L(); ++l) if (pi.dims[l] % 4) return false;
-    if (q1.dims[q1.L()] > XS_WL_CAP || 2 * cfg.act_dim * pi.dims[pi.L()] > XS_WL_CAP) return false;
-    return true;
-  }
-  void add_part_head(Op& o, i64 w_row, int kdim, i64 out) const {   // shares of one output row: part[tn][m]
-    o.i[4] = 1; o.i[5] = 1; o.i[6] = kdim; o.i[7] = 1; o.o[0] = w_row; o.o[1] = out;
-  }
-  void fill_critic_slots(Op& o, int c) const {
-    const int L = q1.L();
-    const NetLayout& n = c ? q2 : q1;
-    o.act_out = q1.act_o;
-    o.i[2] = ntn_q; o.i[3] = c;
-    o.o[2] = b_part_qt[0]; o.o[3] = b_part_qt[1];
-    o.o[4] = q1.b[L] - q1.begin + T0; o.o[5] = q2.b[L] - q1.begin + T0;
-    o.o[6] = b_r; o.o[7] = b_d; o.o[8] = b_lp2; o.o[9] = b_y; o.o[10] = b_tq[0]; o.o[11] = b_tq[1];
-    o.o[12] = b_part_q[c]; o.o[13] = n.b[L]; o.o[14] = b_q[c]; o.o[15] = b_dout[c]; o.o[16] = b_loss[c]; o.o[17] = n.W[L];
-  }
-  Op op_dw_head(int c, int flags) const {
-    Op o = blank(OP_DW_HEAD);
-    const int L = q1.L();
-    const NetLayout& n = c ? q2 : q1;
-    fill_critic_slots(o, c);
-    o.o[18] = a_q[c].h[L - 1]; o.i[0] = a_q[c].ld[L - 1]; o.i[1] = q1.dims[L];
-    o.opt = c ? OPT_Q2 : OPT_Q1; o.flags = flags;
-    o.p = n.W[L]; o.pm = o.p + blk; o.pv = o.p + 2 * blk; o.pg = o.p + 3 * blk; o.pt = o.p - q1.begin + T0;
-    o.pb = n.b[L]; o.pbm = o.pb + blk; o.pbv = o.pb + 2 * blk; o.pbg = o.pb + 3 * blk; o.pbt = o.pb - q1.begin + T0;
-    o.ntiles = (q1.dims[L] + 31) / 32;
-    return o;
-  }
-  void emit_fused_rows(PB& pb) const {
-    const int AD = DW_ADAM, Lq = q1.L(), Lp = pi.L();
-    pb.phase();
-    pb.add(op_prologue(7));
-    pb.add(op_gather());
-    for (int l = 0; l < Lp; ++l) {
-      pb.phase();
-      pb.add(gemm_fwd(pi, l, 0, l ? a_pit.h[l - 1] : x_s2, l ? a_pit.ld[l - 1] : ldx, a_pit));
-      pb.add(gemm_fwd(pi, l, 0, l ? a_pia.h[l - 1] : x_pi, l ? a_pia.ld[l - 1] : ldx, a_pia));
-    }
-    pb.phase();
-    pb.add(gemm_fwd(q1, 0, 0, x_sa, ldx, a_q[0]));
-    pb.add(op_pi_head(false)); pb.add(op_pi_head(true));
-    pb.add(gemm_fwd(q2, 0, 0, x_sa, ldx, a_q[1]));
-    for (int l = 0; l < Lq; ++l) {            // target critics; Q(s,a)'s deeper layers ride along; last layers emit head shares
-      pb.phase();
-      for (int c = 0; c < 2; ++c) {
-        const NetLayout& n = c ? q2 : q1;
-        Op o = gemm_fwd(n, l, T0 - q1.begin, l ? a_qt[c].h[l - 1] : x_s2, l ? a_qt[c].ld[l - 1] : ldx, a_qt[c]);
-        if (l == Lq - 1) add_part_head(o, n.W[Lq] - q1.begin + T0, q1.dims[Lq], b_part_qt[c]);
-        pb.add(o);
-      }
-      if (l + 1 < Lq)
-        for (int c = 0; c < 2; ++c) {
-          const NetLayout& n = c ? q2 : q1;
-          Op o = gemm_fwd(n, l + 1, 0, a_q[c].h[l], a_q[c].ld[l], a_q[c]);
-          if (l + 1 == Lq - 1) add_part_head(o, n.W[Lq], q1.dims[Lq], b_part_q[c]);
-          pb.add(o);
-        }
-    }
-    // critic backward: stage 0 builds delta_{L-1} inside the dA tiles (target y, MSE delta from the shares); the output
-    // layer's gradient + Adam + Polyak is OP_DW_HEAD in the same phase
-    for (int k = 0; k < bwd_stages(q1); ++k) {
-      pb.phase();
-      for (int c = 0; c < 2; ++c) {
-        const NetLayout& n = c ? q2 : q1;
-        if (k == 0) {
-          const int l = Lq - 1;
-          Op o = gemm_da(n, l, a_q[c].aux(l), a_q[c].ld[l], d_q[c][l - 1], rup4(n.dims[l]), a_q[c].aux(l - 1), a_q[c].ld[l - 1]);
-          o.mode = GEN_CRITIC;
-          fill_critic_slots(o, c);
-          o.o[19] = d_q[c][l];
-          pb.add(o);
-        } else {
-          // light output-layer tiles first: the tiles that wrap round to a second wave then land behind them
-          if (k == 1 && c == 0) { pb.add(op_dw_head(0, AD | DW_POLYAK)); pb.add(op_dw_head(1, AD | DW_POLYAK)); }
-          emit_bwd_stage_from(pb, k, n, a_q[c], d_q[c], x_sa, ldx, c ? OPT_Q2 : OPT_Q1, AD | DW_POLYAK, true, /*skip_head_dw=*/true);
-        }
-      }
-    }
-    // actor: critics on (s, a~pi) with head shares; routed dQ built inside the dA tiles; dQ/da shares from the delta_0 tiles
-    for (int l = 0; l < Lq; ++l) {
-      pb.phase();
-      for (int c = 0; c < 2; ++c) {
-        const NetLayout& n = c ? q2 : q1;
-        Op o = gemm_fwd(n, l, 0, l ? a_q[c].h[l - 1] : x_pi, l ? a_q[c].ld[l - 1] : ldx, a_q[c]);
-        if (l == Lq - 1) add_part_head(o, n.W[Lq], q1.dims[Lq], b_part_q[c]);
-        pb.add(o);
-      }
-    }
-    for (int k = 0; k + 1 < Lq; ++k) {
-      pb.phase();
-      for (int c = 0; c < 2; ++c) {
-        const NetLayout& n = c ? q2 : q1;
-        const int l = Lq - 1 - k;
-        Op o = gemm_da(n, l, k == 0 ? a_q[c].aux(l) : d_q[c][l], k == 0 ? a_q[c].ld[l] : rup4(n.dims[l + 1]), d_q[c][l - 1], rup4(n.dims[l]),
-                       a_q[c].aux(l - 1), a_q[c].ld[l - 1]);
-        if (k == 0) {
-          o.mode = GEN_ACTORQ;
-          o.act_out = q1.act_o;
-          o.i[2] = ntn_q; o.i[3] = c;
-          o.o[2] = b_part_q[0]; o.o[3] = b_part_q[1]; o.o[4] = q1.b[Lq]; o.o[5] = q2.b[Lq];
-          o.o[8] = b_lp; o.o[10] = b_qa[0]; o.o[11] = b_qa[1]; o.o[16] = b_ploss; o.o[17] = n.W[Lq]; o.o[19] = -1;
-        }
-        if (l - 1 == 0) {   // this tile produces delta_0: emit the dQ/da shares (action columns of W_0)
-          o.i[4] = 1; o.i[5] = cfg.act_dim; o.i[6] = 1; o.i[7] = n.dims[0]; o.o[0] = n.W[0] + cfg.obs_dim; o.o[1] = b_part_da[c];
-        }
-        pb.add(o);
-      }
-    }
-    // policy backward: head backward + delta_{L-1} built inside the dA tiles
-    for (int k = 0; k <= bwd_stages(pi); ++k) {
-      const int l = Lp - 1;
-      if (k == 0) {
-        pb.phase();
-        Op o = gemm_da(pi, l, a_pia.aux(l), a_pia.ld[l], d_p[l - 1], rup4(pi.dims[l]), a_pia.aux(l - 1), a_pia.ld[l - 1]);
-        o.mode = GEN_PIBWD;
-        o.act_out = pi.act_o;
-        o.i[2] = ntn_q0;
-        o.o[2] = b_part_da[0]; o.o[3] = b_part_da[1]; o.o[4] = b_tz; o.o[5] = b_se; o.o[6] = b_mask; o.o[7] = b_headz; o.o[8] = b_dhead;
-        o.o[17] = pi.W[Lp]; o.o[19] = d_p[l];
-        pb.add(o);
-      } else if (k == 1) {
-        pb.phase();
-        pb.add(gemm_dw(pi, Lp, OPT_PI, AD, b_dhead, 2 * cfg.act_dim, a_pia.h[Lp - 1], a_pia.ld[Lp - 1], false));
-        emit_bwd_stage_from(pb, 1, pi, a_pia, d_p, x_pi, ldx, OPT_PI, AD, false, true);
-        pb.add(op_final(1 | 2 | 4 | 8));
-      } else if (k < bwd_stages(pi)) {
-        pb.phase();
-        emit_bwd_stage_from(pb, k, pi, a_pia, d_p, x_pi, ldx, OPT_PI, AD, false, true);
-      }
-    }
-  }
-  // backward stage k >= 1 of one MLP when delta_{L-1} and delta_{L-2} already exist (stage 0 was a generating tile)
-  void emit_bwd_stage_from(PB& pb, int k, const NetLayout& n, const ActSet& as, const i64* delta, i64 x, int ld_x, int opt,
-                           int flags, bool is_critic, bool skip_head_dw) const {
-    const int L = n.L();
-    auto ldd = [&](int l) { return rup4(n.dims[l + 1]); };
-    if (L - 2 - k >= 0) {
-      const int l = L - 1 - k;
-      pb.add(gemm_da(n, l, delta[l], ldd(l), delta[l - 1], ldd(l - 1), as.aux(l - 1), as.ld[l - 1]));
-    }
-    const int lw = L - k;
-    if (lw >= 1 && !(skip_head_dw && lw == L))
-      pb.add(gemm_dw(n, lw, opt, flags, delta[lw], ldd(lw), as.h[lw - 1], as.ld[lw - 1], is_critic));
-    if (k == bwd_stages(n) - 1) pb.add(gemm_dw(n, 0, opt, flags, delta[0], ldd(0), x, ld_x, is_critic));
-  }
-
   // ---- row-parallel program (sacx_rowpar.cuh) -----------------------------------------------------------------------
   bool rowpar_eligible(std::string& why) const {
     const char* env = getenv("SACX_ROWPAR");
@@ -1076,8 +903,7 @@ struct Engine {
       return SACX_OK;
     };
     int rc;
-    fuse_rows = can_fuse_rows();
-    { PB pb; if (fuse_rows) emit_fused_rows(pb); else emit_fused(pb, true); if ((rc = put(PLAN_FUSED, pb))) return rc; }
+    { PB pb; emit_fused(pb, true); if ((rc = put(PLAN_FUSED, pb))) return rc; }
     { PB pb; emit_fused(pb, false); if ((rc = put(PLAN_FUSED_NOGATHER, pb))) return rc; }
     { PB pb; pb.phase(); pb.add(op_gather()); if ((rc = put(PLAN_SAMPLE, pb))) return rc; }
     { PB pb; emit_target(pb); if ((rc = put(PLAN_TARGET, pb))) return rc; }
@@ -1107,7 +933,7 @@ struct Engine {
 
   // ---- tensor-core path ------------------------------------------------------------------------------------------------
   bool tc_op_eligible(const Op& o) const {
-    if (o.type != OP_GEMM || o.mode != 0 || o.i[4] != 0 || o.zout >= 0) return false;
+    if (o.type != OP_GEMM || o.zout >= 0) return false;
     auto al = [](i64 x) { return x >= 0 && (x & 3) == 0; };
     if (o.N > TC_NMAX) return false;
     if (o.epi == EPI_DACT && (o.N < 16 || (o.N & 3))) return false;

@@ -21,7 +21,6 @@
 // Precision: plain FFMA, fp32 accumulate -- the parity contract is rel 1e-4 against the fp32 reference,
 // which rules out TF32/BF16 tensor-core inputs for this path (SURVEY 2b note).
 #pragma once
-#include "sacx_fused.cuh"
 #include "sacx_math.cuh"
 #include "sacx_types.cuh"
 
@@ -58,8 +57,6 @@ struct EpiCtx {
   const AgentScalars* scal;
   const Hyper* hp;
   unsigned long long* t;        // optional intra-tile timestamps (profiling aid), 8 slots
-  float* xsm;                   // extra shared memory of the fused paths (XSM_FLOATS)
-  const float* w_ext;           // RunArgs::w_ext (critic loss weights)
 };
 // (intra-tile timestamps for tools/phase_profile.py: debug library only, like the row-parallel kernel's event trace)
 #ifdef SACX_DEBUG_HOOKS
@@ -153,9 +150,8 @@ __device__ __forceinline__ void epi_prefetch(const Op& op, const EpiCtx& ctx, in
 
 template <int MODE>
 __device__ __forceinline__ void epilogue_row4(const Op& op, const EpiCtx& ctx, int m, int n, float4 acc, EpiPre& pre,
-                                              bool have_pre, float4& outv) {
+                                              bool have_pre) {
   float* base = ctx.base;
-  outv = make_float4(0.f, 0.f, 0.f, 0.f);
   if (m >= op.M || n >= op.N) return;
   if (!have_pre) epi_prefetch<MODE>(op, ctx, m, n, pre);
   const bool vec = pre.valid;
@@ -166,8 +162,7 @@ __device__ __forceinline__ void epilogue_row4(const Op& op, const EpiCtx& ctx, i
     if (vec) {
       const float4 zz = make_float4(v[0] + pre.a.x, v[1] + pre.a.y, v[2] + pre.a.z, v[3] + pre.a.w);
       if (z) *reinterpret_cast<float4*>(z) = zz;
-      outv = make_float4(act_fwd(op.act, zz.x), act_fwd(op.act, zz.y), act_fwd(op.act, zz.z), act_fwd(op.act, zz.w));
-      *reinterpret_cast<float4*>(c) = outv;
+      *reinterpret_cast<float4*>(c) = make_float4(act_fwd(op.act, zz.x), act_fwd(op.act, zz.y), act_fwd(op.act, zz.z), act_fwd(op.act, zz.w));
     } else {
       const float* bias = base + op.bias + n;
 #pragma unroll
@@ -176,20 +171,18 @@ __device__ __forceinline__ void epilogue_row4(const Op& op, const EpiCtx& ctx, i
           const float zz = v[j] + __ldcg(bias + j);
           if (z) z[j] = zz;
           c[j] = act_fwd(op.act, zz);
-          (&outv.x)[j] = c[j];
         }
     }
   } else if (MODE == 1) {
     float* c = base + op.c + (i64)m * op.ldc + n;
     if (vec) {
-      outv = make_float4(v[0] * act_dz(op.act, pre.a.x), v[1] * act_dz(op.act, pre.a.y), v[2] * act_dz(op.act, pre.a.z),
-                         v[3] * act_dz(op.act, pre.a.w));
-      *reinterpret_cast<float4*>(c) = outv;
+      *reinterpret_cast<float4*>(c) = make_float4(v[0] * act_dz(op.act, pre.a.x), v[1] * act_dz(op.act, pre.a.y),
+                                                  v[2] * act_dz(op.act, pre.a.z), v[3] * act_dz(op.act, pre.a.w));
     } else {
       const float* aux = base + op.aux + (i64)m * op.ld_aux + n;
 #pragma unroll
       for (int j = 0; j < 4; ++j)
-        if (n + j < op.N) { c[j] = v[j] * act_dz(op.act, __ldcg(aux + j)); (&outv.x)[j] = c[j]; }
+        if (n + j < op.N) c[j] = v[j] * act_dz(op.act, __ldcg(aux + j));
     }
   } else {  // EPI_DW: (m, n) = (out neuron, in feature); parameter leading dim = N (= K_in)
     const i64 e = (i64)m * op.N + n;
@@ -403,10 +396,6 @@ __device__ __noinline__ void gemm_tile_impl(const Op& op, const EpiCtx& ctx, int
   const bool bias_tile = BSUM && (tn == 0) && (op.pb >= 0);
   const int nk = (K + GEMM_BK - 1) / GEMM_BK;
   SACX_TSTAMP(0);
-  const FusedCtx fc{ctx.base, ctx.scal, ctx.hp, ctx.xsm, ctx.w_ext};
-  const bool gen = (MODE == 1) && (op.mode != GEN_NONE);
-  const bool part = (MODE <= 1) && (op.i[4] != 0);
-  if (part) part_stage(op, fc, n0, BN);
 
   const int kg = tid / C::TPG, t = tid % C::TPG;
   const int ty = t / C::TX, tx = t % C::TX;
@@ -437,39 +426,12 @@ __device__ __noinline__ void gemm_tile_impl(const Op& op, const EpiCtx& ctx, int
   // NS-deep cp.async ring as ONE rolled loop (one copy of the load and math code per variant keeps the
   // instruction footprint small: instruction-fetch stalls were 30% of this kernel's samples). Iteration j issues
   // stage j and consumes stage j-(NS-1); for K <= 192 the whole K range is in flight before the first wait.
-  if (MODE == 1) {
-    if (gen) {
-      SACX_TSTAMP(5);
-      gen_prologue(op, fc, m0, tn, BM);      // per-row scalars and W_L into shared memory while the ring fills
-      SACX_TSTAMP(6);
-      __syncthreads();
-      SACX_TSTAMP(7);
-    }
-  }
   float a_cur[8][4];
 #pragma unroll 1
   for (int j = 0; j < nk + GEMM_NS - 1; ++j) {
     const int it = j - (GEMM_NS - 1);
     if (it >= 0) {
       cp_async_wait<GEMM_NS - 3>();          // stages it and it+1 have landed
-      if (MODE == 1) {
-        if (gen) {
-          // this thread's own chunks of the freshly landed stage(s): saved activations -> delta, in place
-          for (int s2 = (it == 0 ? 0 : it + 1); s2 <= it + 1 && s2 < nk; ++s2) {
-            float* st = smem + (s2 % GEMM_NS) * C::STAGE_FLOATS;
-#pragma unroll
-            for (int i = 0; i < BM / 16; ++i) {
-              const int id = tid + i * 256, row = id >> 4, k = (id & 15) << 2;
-              float4* p4 = reinterpret_cast<float4*>(st + row * GEMM_LDK + k);
-              const bool ok = (m0 + row < M) && (s2 * GEMM_BK + k < K);
-              const float4 dv = gen_transform(op, fc, *p4, row, s2 * GEMM_BK + k, ok);
-              *p4 = dv;
-              if (tn == 0 && ok && op.o[19] >= 0)      // delta of the last hidden layer, needed by that layer's dW
-                *reinterpret_cast<float4*>(ctx.base + op.o[19] + (i64)(m0 + row) * op.a_sm + s2 * GEMM_BK + k) = dv;
-            }
-          }
-        }
-      }
       __syncthreads();                       // ... for everyone; slot (it-1) % NS is free again
       if (it == 0) SACX_TSTAMP(1);
     }
@@ -517,9 +479,7 @@ __device__ __noinline__ void gemm_tile_impl(const Op& op, const EpiCtx& ctx, int
       const float4 p = *reinterpret_cast<const float4*>(&red[q * C::RBLK + row * RS + c4]);
       s.x += p.x; s.y += p.y; s.z += p.z; s.w += p.w;
     }
-    float4 outv;
-    epilogue_row4<MODE>(op, ctx, m0 + row, n0 + c4, s, pre, C::NV == 1, outv);
-    if (MODE <= 1) { if (part) part_emit(op, fc, outv, m0 + row, c4, tn, BN); }
+    epilogue_row4<MODE>(op, ctx, m0 + row, n0 + c4, s, pre, C::NV == 1);
   }
   if (BSUM) {
     if (bias_tile && tid < BM) {

@@ -9,35 +9,42 @@ namespace sacx {
 constexpr int SMEM_OPS = 64;                                   // ops of the active phase range cached in smem
 constexpr int WSM_FLOATS = 8 * 4 * SACX_MAX_ACT;               // per-warp scratch for the row ops
 
-// Barrier among the gridDim.x CTAs that work on the same agent (cooperative launch => co-resident).
-// Monotonic counter, release/acquire at gpu scope; thread 0's fences make the CTA's global writes
-// visible and drop stale L1 lines before the other threads continue.
-__device__ __forceinline__ void group_barrier(unsigned* counter, unsigned& epoch, int mode) {
+// Barriers among the gridDim.x CTAs that work on the same agent (cooperative launch => co-resident), on a monotonic
+// arrival counter with release/acquire at gpu scope.
+// Flag form (tile-parallel kernel): arrivals on one line, release flag on another, so pollers do not queue behind the atomics.
+__device__ __forceinline__ void group_barrier_flag(unsigned* counter, unsigned& epoch) {
+  __syncthreads();
+  if (gridDim.x > 1) {
+    if (threadIdx.x == 0) {
+      epoch += gridDim.x;
+      unsigned v, old;
+      unsigned* flag = counter + 32;
+      asm volatile("atom.add.release.gpu.global.u32 %0, [%1], 1;" : "=r"(old) : "l"(counter) : "memory");
+      if (old + 1 == epoch) {
+        asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(flag), "r"(epoch) : "memory");
+      } else {
+        do {
+          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
+        } while ((int)(v - epoch) < 0);
+      }
+    }
+    __syncthreads();
+  }
+}
+// Counter form (row-parallel kernel's grid barrier): every CTA polls the arrival counter itself, one L2 hop less than waiting
+// for a flag. Thread 0's fences make the CTA's global writes visible and drop stale L1 lines before the other threads continue.
+__device__ __forceinline__ void group_barrier_counter(unsigned* counter, unsigned& epoch) {
   __syncthreads();
   if (gridDim.x > 1) {
     if (threadIdx.x == 0) {
       epoch += gridDim.x;
       unsigned v;
-      if (mode == 0) {
-        __threadfence();
-        atomicAdd(counter, 1u);
-        do {
-          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
-        } while (v < epoch);
-        __threadfence();
-      } else {
-        // arrivals on one line, release flag on another: pollers do not queue behind the atomics
-        unsigned* flag = counter + 32;
-        unsigned old;
-        asm volatile("atom.add.release.gpu.global.u32 %0, [%1], 1;" : "=r"(old) : "l"(counter) : "memory");
-        if (old + 1 == epoch) {
-          asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(flag), "r"(epoch) : "memory");
-        } else {
-          do {
-            asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
-          } while ((int)(v - epoch) < 0);
-        }
-      }
+      __threadfence();
+      atomicAdd(counter, 1u);
+      do {
+        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
+      } while (v < epoch);
+      __threadfence();
     }
     __syncthreads();
   }
@@ -79,8 +86,7 @@ __global__ void __launch_bounds__(256, 1) sacx_run_kernel(const Plan* __restrict
     AgentScalars* scal = reinterpret_cast<AgentScalars*>(base + args.scal_off);
     RowCtx rc{base, scal, &sargs, agent, 0, wsm + warp * 4 * SACX_MAX_ACT, gsm, C::SMEM_FLOATS, nullptr};
     rc.gcache = gcache + warp * GCACHE_WORDS;
-    EpiCtx ec{base, scal, &sargs.hp, nullptr, gsm + C::SMEM_FLOATS, sargs.w_ext};
-    const FusedCtx fcx{base, scal, &sargs.hp, gsm + C::SMEM_FLOATS, sargs.w_ext};
+    EpiCtx ec{base, scal, &sargs.hp, nullptr};
     const bool last_agent = (agent + (int)gridDim.y >= args.n_agents);
     for (int step = 0; step < args.n_steps; ++step) {
       rc.step = step;
@@ -104,7 +110,6 @@ __global__ void __launch_bounds__(256, 1) sacx_run_kernel(const Plan* __restrict
             case OP_ACTOR_BWD: tile_actor_bwd<0>(op, rc, lt); __syncthreads(); break;
             case OP_PROLOGUE: if (tid < 3) op_prologue(op, rc, tid); break;
             case OP_FINAL: if (warp == 0) op_final(op, rc, lane); break;
-            case OP_DW_HEAD: tile_dw_head(op, fcx, lt, gsm); break;
             case OP_POLYAK: op_polyak(op, rc, lt); break;
             case OP_ADAM_FLAT: op_adam_flat(op, rc, lt); break;
             default: break;
@@ -116,7 +121,7 @@ __global__ void __launch_bounds__(256, 1) sacx_run_kernel(const Plan* __restrict
           dbg = args.dbg + (((size_t)step * (args.phase_end - args.phase_begin) + (p - args.phase_begin)) * gridDim.x + blockIdx.x) * 2;
           dbg[0] = clock64();
         }
-        if (!very_last) group_barrier(counter, epoch, args.barrier_mode);
+        if (!very_last) group_barrier_flag(counter, epoch);
         if (dbg) dbg[1] = clock64();
       }
     }
@@ -132,8 +137,7 @@ __global__ void __launch_bounds__(256, 1) sacx_run_kernel(const Plan* __restrict
 // in registers, the input rows as warp-wide broadcast loads. Memory-bound on the output write.
 constexpr int SMALLK_MAX = 32;
 __device__ __forceinline__ bool small_fwd_ok(const Op& o) {
-  return o.type == OP_GEMM && o.epi == EPI_FWD && o.K <= SMALLK_MAX && o.zout < 0 && o.mode == 0 && o.i[4] == 0 && o.a_sk == 1 && o.b_sk == 1 &&
-         o.cfg >= 1;
+  return o.type == OP_GEMM && o.epi == EPI_FWD && o.K <= SMALLK_MAX && o.zout < 0 && o.a_sk == 1 && o.b_sk == 1 && o.cfg >= 1;
 }
 // K <= KB: the reduction is unrolled over KB register-resident weights; the tile's 64 input rows are staged (zero-padded to
 // KB) in shared memory first, so the inner loop has no global load and no predicate. (Profile history: one 32-wide bucket

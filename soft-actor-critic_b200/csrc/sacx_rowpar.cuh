@@ -7,7 +7,7 @@
 //   * every layer's output columns are split 8 ways: CTA `rank` computes the 16 x (N/8) slice with 3xTF32
 //     mma.sync.m16n8k8 tensor-core tiles (hi/lo split of both operands, fp32 accumulate: fp32-level accuracy),
 //   * slices are exchanged through L2: each CTA stores its slice, the 8 CTAs meet at a group barrier (one L2 atomic
-//     per CTA + a release flag) and pull the full 16 x N rows back with cp.async,
+//     per CTA, polled by all eight) and pull the full 16 x N rows back with cp.async,
 //   * the narrow heads (policy 2A outputs, critic 1 output, dQ/da) never travel as activations: the producing tile
 //     projects its slice onto the head weights and only the 8 partial sums per row are exchanged,
 //   * weight slices stream from L2 into a 3-slot shared-memory ring two jobs ahead (they do not depend on data),
@@ -104,7 +104,7 @@ struct RpCtx {
   const RpProgram* P;
   RpRows* R;
   float* part;            // this group's partial scratch (global)
-  unsigned* gbar;         // this group's barrier counter (flag at +32)
+  unsigned* gbar;         // this group's barrier counter
   int rank, step, row0;
   RpTrace* tr;
   uint64_t* wbar;         // one mbarrier per weight slot (TMA-staged slices)
@@ -175,34 +175,19 @@ __device__ __forceinline__ void rp_mma3(float (&c0)[4], float (&c1)[4], float (&
   rp_mma(c2, ah, bh);
 }
 
-// ---- group barrier: 8 CTAs, arrivals on one L2 line, release flag on another ----------------------------------------
-__device__ __forceinline__ void rp_group_barrier(unsigned* counter, unsigned& epoch, int mode) {
+// ---- group barrier: 8 CTAs poll the arrival counter itself -- one L2 hop less than "last arriver publishes a flag" ---------
+__device__ __forceinline__ void rp_group_barrier(unsigned* counter, unsigned& epoch) {
   __syncthreads();
-#ifdef SACX_DEBUG_HOOKS      // timing experiment (libsacx_debug.so only): what would the update cost without the group barriers? (results are garbage)
-  if (mode & 16) return;
-#endif
   if (threadIdx.x == 0) {
     epoch += RP_CS;
     unsigned old, v;
     asm volatile("atom.add.release.gpu.global.u32 %0, [%1], 1;" : "=r"(old) : "l"(counter) : "memory");
-    if (mode & 2) {
-      // eight CTAs: poll the arrival counter itself -- one L2 hop less than "last arriver publishes a flag"
-      if (old + 1 != epoch) {
-        do {
-          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
-        } while ((int)(v - epoch) < 0);
-      } else {
-        asm volatile("fence.acq_rel.gpu;" ::: "memory");
-      }
+    if (old + 1 != epoch) {
+      do {
+        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
+      } while ((int)(v - epoch) < 0);
     } else {
-      unsigned* flag = counter + 32;
-      if (old + 1 == epoch) {
-        asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(flag), "r"(epoch) : "memory");
-      } else {
-        do {
-          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
-        } while ((int)(v - epoch) < 0);
-      }
+      asm volatile("fence.acq_rel.gpu;" ::: "memory");
     }
   }
   __syncthreads();
@@ -1067,8 +1052,7 @@ __device__ __noinline__ void rp_dw_tile_tc(const Op& op, const EpiCtx& ctx, int 
     } else if (!adam) {
       pre.valid = (m0 + erow < M) && epi_vec_ok(op, n0 + ec4);          // gradient store only: nothing to prefetch
     }
-    float4 outv;
-    epilogue_row4<2>(op, ctx, m0 + erow, n0 + ec4, s, pre, true, outv);
+    epilogue_row4<2>(op, ctx, m0 + erow, n0 + ec4, s, pre, true);
   }
   if (bias_tile && tid < 32) {
     float s = 0.f;
@@ -1133,8 +1117,7 @@ __device__ __noinline__ void rp_dw_vec_tile(const Op& op, const EpiCtx& ctx, int
                                  red[4 * tid + 3] + red[128 + 4 * tid + 3]);
     EpiPre pre;
     pre.valid = false;
-    float4 outv;
-    if (n0 + 4 * tid < N) epilogue_row4<2>(op, ctx, 0, n0 + 4 * tid, g, pre, false, outv);
+    if (n0 + 4 * tid < N) epilogue_row4<2>(op, ctx, 0, n0 + 4 * tid, g, pre, false);
   }
   if (tile == 0 && op.pb >= 0 && warp == 1) {                        // bias gradient = sum of dout (lane-strided, then butterfly)
     float sacc = 0.f;
@@ -1210,7 +1193,7 @@ __device__ __forceinline__ void rp_run_steps(const RpCtx& c, int s0, int s1, RpS
       rp_job(jb, c, sl);
       RP_TRACE(5000 + j);
     }
-    if (s + 1 < s1) rp_group_barrier(c.gbar, sy.gepoch, c.args->barrier_mode);
+    if (s + 1 < s1) rp_group_barrier(c.gbar, sy.gepoch);
     RP_TRACE(6000 + s);
   }
   cp_async_wait<0>();
@@ -1287,7 +1270,7 @@ __global__ void __launch_bounds__(256, 1) sacx_rp_kernel(const Plan* __restrict_
   if (tid == 32) {            // (another warp than the launch constants' thread)
     sargs = args;             // a plain struct copy: &args would bring the stack copy back
     float* b0 = args.arena;
-    sec = EpiCtx{b0, reinterpret_cast<AgentScalars*>(b0 + args.scal_off), &sargs.hp, nullptr, rp_dyn_smem + WSM_FLOATS + CfgSmall::SMEM_FLOATS};
+    sec = EpiCtx{b0, reinterpret_cast<AgentScalars*>(b0 + args.scal_off), &sargs.hp, nullptr};
   }
   __syncthreads();
   const int rank = blockIdx.x % RP_CS, gid = blockIdx.x / RP_CS, ngr = sprog.n_row_groups;
@@ -1341,7 +1324,7 @@ __global__ void __launch_bounds__(256, 1) sacx_rp_kernel(const Plan* __restrict_
           const int lt = t - op.tile0;
           if (op.type == OP_GEMM) {                 // only dW tiles live in these phases
             if (op.i[5] == 1) rp_dw_vec_tile(op, ec, lt, dwstage, args.rp_maps, dwbar, dwparity);      // one-row layer: 128 columns per tile
-            else if (!(args.barrier_mode & 8) && rp_dw_tc_ok(op, args.rp_maps)) rp_dw_tile_tc(op, ec, lt, dwstage, args.rp_maps, dwbar, dwparity);
+            else if (rp_dw_tc_ok(op, args.rp_maps)) rp_dw_tile_tc(op, ec, lt, dwstage, args.rp_maps, dwbar, dwparity);
             else gemm_tile_impl<CfgSmall, 2>(op, ec, lt, gsm);
           }
           else if (op.type == OP_FINAL) {
@@ -1363,7 +1346,7 @@ __global__ void __launch_bounds__(256, 1) sacx_rp_kernel(const Plan* __restrict_
       const bool very_last = (ph == 3) && (step + 1 == args.n_steps);
       RP_TRACE(7000 + ph);
       if (dbg) dbg[ph * dstride] = clock64();
-      if (!very_last) group_barrier(counter, epoch, (args.barrier_mode & 4) ? 0 : 1);
+      if (!very_last) group_barrier_counter(counter, epoch);
       if (dbg) dbg[ph * dstride + 1] = clock64();
     }
   }

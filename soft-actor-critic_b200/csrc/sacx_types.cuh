@@ -20,7 +20,6 @@ enum OpType : int {
   OP_POLYAK,      // standalone soft target update (a10)
   OP_ADAM_FLAT,   // Adam over a packed gradient block (data-parallel apply)
   OP_LOAD_EXT,    // copy external y / logpi into arena buffers
-  OP_DW_HEAD,     // fused plan: gradient + Adam of the critics' output layer from the head shares
   OP_PI_TAIL,     // large batch: rsample / tanh squash / log_prob from head pre-activations a tensor-core GEMM produced (one thread per row)
   OP_Q_TAIL,      // large batch: Bellman target / critic loss gradient / actor routing from head values the GEMM epilogue projected (one thread per row)
   OP_DELTA,       // large batch: delta of the critics' last hidden layer, coef[b] * W_L[k] * act'(h[b][k]) (element-wise stream)
@@ -124,7 +123,6 @@ struct RunArgs {
   i64 scal_off;
   unsigned long long* dbg;   // optional [n_steps][n_phases][gridDim.x][2] clock64 at barrier arrive / release
   unsigned long long* dbg2;  // optional [n_steps][n_phases][gridDim.x][8] intra-tile timestamps of the CTA's last GEMM tile
-  int barrier_mode;
   int tc_skip;               // 1: GEMM ops marked for the tensor-core path (op.cfg & 2) are run by sacx_tc_kernel, skip them here
   float* rp_part;            // row-parallel kernel: partial-sum scratch [groups][part_stride]
   const void* rp_maps;       // row-parallel kernel: device array of CUtensorMap (128 B each) for the TMA-staged weight slices, or null

@@ -322,7 +322,7 @@ def test_population_agents_are_independent_and_match_single_agent():
         assert pop.metrics(ag)["updates"] == K
 
 
-# ----------------------------------------------------------------------------- edge shapes and the fused-rows plan
+# ----------------------------------------------------------------------------- edge shapes
 def _random_nets(obs, act, hidden_pi, hidden_q, seed=0, scale=0.3):
     rng = np.random.default_rng(seed)
     sds = {}
@@ -373,34 +373,6 @@ def test_update_edge_shapes_vs_oracle(obs, act, hp, hq, B, actfn):
         for l, (w, b) in enumerate(zip(net.W, net.b)):
             assert_close(f"{tag}.W{l}", eng.view(f"{tag}.W{l}").cpu().numpy(), w, 3e-4)
             assert_close(f"{tag}.b{l}", eng.view(f"{tag}.b{l}").cpu().numpy().ravel(), b, 3e-4)
-
-
-@pytest.mark.parametrize("name", ["tiny_auto", "acts_tanh", "acts_leaky_relu", "bipedal", "pendulum128"])
-def test_fused_rows_plan_vs_reference(name, monkeypatch):
-    """SACX_FUSE_ROWS=1: row phases folded into the GEMM tiles (13 phases instead of 16). Same reference vectors."""
-    from sac.replay_buffer import ReplayBuffer
-    monkeypatch.setenv("SACX_FUSE_ROWS", "1")
-    g = Golden(name)
-    eng = engine_from_golden(g)
-    rb = ReplayBuffer(g.cfg["buffer"]["capacity"], g.obs, g.act)
-    fill_ring(rb, g.n_fill, g.obs, g.act)
-    eng.attach_ring(rb)
-    nl_pi, nl_q = len(g.cfg["policy_net"]["hidden_sizes"]) + 1, len(g.cfg["q_net"]["hidden_sizes"]) + 1
-    for k in range(g.K):
-        m = eng.update_host(g[f"step{k}/idx"], g[f"step{k}/eps1"], g[f"step{k}/eps2"], 1)
-        tol = 3e-5 * (3 ** k)
-        assert_close(f"step{k} y", eng.view("out.y").cpu().numpy().ravel(), g[f"step{k}/y"], tol)
-        assert_close(f"step{k} logpi", eng.view("out.logpi").cpu().numpy().ravel(), g[f"step{k}/lp"], tol)
-        assert abs(m["q1_loss"] - float(g[f"step{k}/q1_loss"])) <= 10 * tol * abs(float(g[f"step{k}/q1_loss"])) + 1e-7
-        if g.cfg["sac"]["auto_entropy_tuning"]:
-            assert abs(m["log_alpha"] - float(g[f"step{k}/log_alpha"])) < 2e-6
-        for tag, nl in (("pi", nl_pi), ("q1", nl_q), ("q2", nl_q), ("q1t", nl_q), ("q2t", nl_q)):
-            for nm, v in read_net(eng, tag, nl).items():
-                key = f"step{k}/{tag}/{nm}"
-                if g.full:
-                    assert_close(key, v, g[key], 1e-4 * (2 ** k))
-                else:
-                    assert_close(key + "#smp", v.ravel()[::97], g[key + "#smp"], 1e-4 * (2 ** k))
 
 
 def test_full_size_ring_properties():

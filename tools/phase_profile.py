@@ -71,10 +71,5 @@ for p in range(P):
     if ok.sum() == 0:
         continue
     d = lambda a, b: int(np.median((x[..., a] - x[..., b])[ok]))
-    extra = ""
-    okg = ok & (x[..., 7] > x[..., 5]) & (x[..., 5] > x[..., 0])
-    if okg.sum() > 0:
-        dg = lambda a, b: int(np.median((x[..., a] - x[..., b])[okg]))
-        extra = f"   gen: pre {dg(5,0)} prologue {dg(6,5)} sync {dg(7,6)} first-wait {dg(1,7)}"
-    print(f"{p:5d} {d(1,0):7d} {d(2,1):7d} {d(3,2):7d} {d(4,3):7d} {d(4,0):7d}{extra}")
+    print(f"{p:5d} {d(1,0):7d} {d(2,1):7d} {d(3,2):7d} {d(4,3):7d} {d(4,0):7d}")
 
