@@ -38,6 +38,32 @@ def philox_uniforms(seed, update, which, row, j, agent):
     return f(u1), f(u2)
 
 
+def per_uniform(seed, counter, k, agent):
+    """U[0, 1) of row k of prioritized-replay draw `counter` (``per_uniform`` in csrc/sacx_per.cuh): the Philox stream tagged
+    0x7E in counter word 3, top 24 bits of word 0 times 2^-24 (exact in float32)."""
+    seed, counter = int(seed), int(counter)
+    o = philox4x32_10((counter & _M32, (counter >> 32) & _M32, k, 0x7E000000),
+                      ((seed & _M32) ^ ((agent * 0x9E3779B9) & _M32), ((seed >> 32) & _M32) ^ 0x5AC5AC5A))
+    return np.float32(o[0] >> 8) * np.float32(5.9604644775390625e-8)
+
+
+def per_uniforms(seed, counter, B, agent):
+    """per_uniform(seed, counter, k, agent) for k = 0 .. B-1 as a float32 array: the same rounds on uint64 lanes."""
+    seed, counter = int(seed), int(counter)
+    m32 = np.uint64(_M32)
+    u = lambda x: np.uint64(int(x) & _M32)
+    c0 = np.full(B, u(counter), np.uint64)
+    c1 = np.full(B, u(counter >> 32), np.uint64)
+    c2 = np.arange(B, dtype=np.uint64)
+    c3 = np.full(B, np.uint64(0x7E000000), np.uint64)
+    k0, k1 = (seed & _M32) ^ ((agent * 0x9E3779B9) & _M32), ((seed >> 32) & _M32) ^ 0x5AC5AC5A
+    for _ in range(10):
+        p0, p1 = np.uint64(_M0) * c0, np.uint64(_M1) * c2
+        c0, c1, c2, c3 = (p1 >> np.uint64(32)) ^ c1 ^ u(k0), p1 & m32, (p0 >> np.uint64(32)) ^ c3 ^ u(k1), p0 & m32
+        k0, k1 = (k0 + _W0) & _M32, (k1 + _W1) & _M32
+    return (c0 >> np.uint64(8)).astype(np.float32) * np.float32(5.9604644775390625e-8)
+
+
 def philox_normal(seed, update, which, row, j, agent):
     """N(0, 1) draw of element (update, which, row, j): Box-Muller in float64 on the device's float32 uniforms."""
     u1, u2 = philox_uniforms(seed, update, which, row, j, agent)

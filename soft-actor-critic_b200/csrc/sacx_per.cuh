@@ -8,7 +8,8 @@
 //      ring's worth of pushes, or a push counter that went backwards (ring image loaded), resets every leaf;
 //   3. one level per barrier: every touched internal node is recomputed from its 32 children in a fixed order (xor butterfly).
 //      No atomicAdd deltas: a node is a pure function of its children, so replicas, bursts and a rebuilt tree are bit-identical;
-//   4. sampling: one warp per row walks root -> leaf, 32 children (one 128-byte read) per level.
+//   4. sampling: one warp per row walks root -> leaf, 32 children (one 128-byte read) per level; a slot with p = 0 is never
+//      taken (oracle/per_numpy.py walk_f32 restates the walk bit for bit).
 // Leaves are the priorities themselves ([cap] floats, 0 = empty slot); level l >= 1 holds (sum, min) of groups of 32 nodes of
 // level l - 1 as two arrays; an empty leaf counts as (0, +inf) in the min.
 #pragma once
@@ -198,7 +199,10 @@ __global__ void __launch_bounds__(256) per_refresh_kernel(PerArgs a) {
         const float t = __shfl_up_sync(0xffffffffu, sc, off);
         if (lane >= off) sc += t;
       }
-      const unsigned hit = __ballot_sync(0xffffffffu, sc > u);
+      // first child with p > 0 whose prefix sum exceeds u. Without `v > 0` rounding could take an empty slot (p = 0, weight
+      // inf): an empty child's scanned sum can round above its left neighbour's (a draw at the end of a partly filled ring),
+      // and u - before below can round below 0 (a draw at the start of a child whose first slots are empty)
+      const unsigned hit = __ballot_sync(0xffffffffu, v > 0.f && sc > u);
       int f;
       if (hit) f = __ffs(hit) - 1;
       else {                                                  // u within rounding of the node's sum: last child with p > 0

@@ -21,6 +21,14 @@ Why the comparisons are built the way they are:
 with grads_only, no apply in between): the same comparisons on the gradients the engine stores in `g.*`, without the optimiser,
 Polyak and temperature checks.
 
+`case(..., per={...})` runs prioritized replay (test_gpu_per_oracle.py): a PrioritizedReplayBuffer with loaded priorities is
+attached and `update(None, eps1, eps2, 1)` lets the tree draw the batch. Every ring row on a discontinuity gets priority 0, which
+the walk never takes; batch.idx must equal oracle/per_numpy.py's walk_f32 on the loaded leaves with per_uniform's stream, bit
+for bit. The critic oracle weighs row k by float64 w = (p / p_min)^-beta(t) (dout, loss rows, q losses, gradients), the actor
+and temperature stay unweighted, and duplicate rows are expected (sampling with replacement). The write-back, applied by the
+next read of the priorities, must give each sampled slot (delta + eps)^alpha of its highest row at rel 2e-6 and leave every
+other leaf's bits alone.
+
 Bars (DESIGN.md section 2): rel-L2 2e-5 on per-row outputs, 5e-5 on gradients (with the bias bar of
 test_gpu_baseline_configs._check_layer_grads), 2e-6 on the Adam arithmetic, 1e-6 absolute on log_alpha, bits on the gather
 and on Polyak. Callers print the largest error per quantity (`report`), so the margin is visible.
@@ -47,9 +55,11 @@ T = (0, 1, 39886)                           # Adam step counts before the update
 
 # ----------------------------------------------------------------------------------------------------------------- cases
 def case(obs, act, hp, hq, B, actfn="relu", out_act="identity", t=0, wrap=False, auto=True, lo=-20.0, hi=2.0, scale=1.0,
-         ties=False, device_rng=False, env=None):
+         ties=False, device_rng=False, env=None, per=None):
+    """per: prioritized replay, a dict of alpha, beta (beta0), beta_steps, eps, profile ("spread" or "peaked") and optionally
+    updates (start value of scal.updates: the draw counter and the beta schedule's t)."""
     return dict(obs=obs, act=act, hp=hp, hq=hq, B=B, actfn=actfn, out_act=out_act, t=t, wrap=wrap, auto=auto, lo=lo, hi=hi,
-                scale=scale, ties=ties, device_rng=device_rng, env=dict(env or {}))
+                scale=scale, ties=ties, device_rng=device_rng, env=dict(env or {}), per=dict(per) if per else None)
 
 
 # ------------------------------------------------------------------------------------------------------------ helpers
@@ -183,13 +193,36 @@ def setup(c, monkeypatch, seed):
     a = rng.uniform(-1, 1, (n_push, A)).astype(F32)
     r = rng.standard_normal(n_push).astype(F32)
     d = (rng.random(n_push) < 0.4).astype(F32)
-    rb = ReplayBuffer(cap, O, A)
+    per = c.get("per")
+    if per:
+        from sac.replay_buffer import PrioritizedReplayBuffer
+        rb = PrioritizedReplayBuffer(cap, O, A, alpha=per["alpha"], beta=per["beta"], beta_steps=per["beta_steps"], eps=per["eps"])
+    else:
+        rb = ReplayBuffer(cap, O, A)
     for lo in range(0, n_push, cap // 2):
         rb.push_batch(s[lo: lo + cap // 2], a[lo: lo + cap // 2], r[lo: lo + cap // 2], s2[lo: lo + cap // 2], d[lo: lo + cap // 2])
     eng.attach_ring(rb)
+    if per:
+        eng.attach_per(rb)
+        eng.view("scal.updates").fill_(int(per.get("updates", 0)))
+        n = min(n_push, cap)
+        if per["profile"] == "peaked":                # a few slots hold most of the mass: many duplicate rows
+            p = np.full(n, 1e-3)
+            p[rng.choice(n, 6, replace=False)] = 10.0
+        else:                                         # (delta + eps)^alpha, delta over four decades
+            p = (10.0 ** rng.uniform(-3, 1, n) + per["eps"]) ** per["alpha"]
+        leaves = np.zeros(cap, F32)
+        leaves[per_slots(n_push, cap, n)] = p
+        rb.load_slot_priorities(torch.as_tensor(leaves), float(leaves.max()))
     first = max(n_push - cap, 0)                      # logical position j of the ring = push number first + j
     ring = tuple(x[first:] for x in (s, a, r, s2, d))
     return eng, rb, ring, rng
+
+
+def per_slots(pushes, cap, n):
+    """Ring slot of logical positions 0 .. n-1."""
+    from oracle import per_numpy as P
+    return P.logical_to_slot(np.arange(n), pushes, cap)
 
 
 def _state(eng, c):
@@ -226,7 +259,21 @@ def one_update(eng, c, ring, rng, worst, grads=False):
     st = _state(eng, c)
     pre = _pre_flags(st, c, ring)
     n_ring = len(ring[0])
-    if c["device_rng"]:
+    per = c.get("per")
+    if per:
+        # the tree draws the batch: every ring row on a discontinuity gets p = 0, which the walk never takes
+        from oracle import per_numpy as P
+        assert not grads and not c["device_rng"]
+        buf = eng.per
+        cap, pushes = buf.capacity, int(buf._lib.sacx_ring_pushes(buf.handle, 0))
+        leaves, pmax = buf.slot_priorities()                 # applies the previous update's write-back
+        leaves = leaves.cpu().numpy()
+        leaves[per_slots(pushes, cap, n_ring)[pre]] = 0
+        assert (leaves > 0).any()
+        buf.load_slot_priorities(torch.as_tensor(leaves), pmax)
+        e1 = rng.standard_normal((B, A)).astype(F32)
+        e2 = rng.standard_normal((B, A)).astype(F32)
+    elif c["device_rng"]:
         assert not grads
         idx = None
     else:
@@ -262,6 +309,25 @@ def one_update(eng, c, ring, rng, worst, grads=False):
             worst["eps (float32 ulps of max(1,|x|))"] = max(worst.get("eps (float32 ulps of max(1,|x|))", 0.0), float(ulps.max()))
             assert ulps.max() <= 4, f"eps{which}: {ulps.max():.1f} ulps from philox_normal"
         assert not pre[idx].any(), f"device batch meets {int(pre[idx].sum())} rows on a discontinuity: pick another seed"
+    elif per:
+        dev = lambda x: torch.as_tensor(x).cuda()
+        eng.update(None, dev(e1), dev(e2), 1)
+        eng.sync()
+        m = eng.metrics()
+        idx = _np(eng.view("batch.idx")).ravel()
+        seed = int(eng.view("scal.rng_seed").item())
+        agent = int(eng.view("scal.rng_agent").view(torch.int32).item())
+        slots = P.walk_f32(P.tree_f32(leaves), device_rng.per_uniforms(seed, st["updates"], B, agent))
+        oldest = pushes % cap if pushes > cap else 0
+        assert np.array_equal(idx, (slots - oldest) % cap), \
+            f"{int((idx != (slots - oldest) % cap).sum())} of {B} sampled slots differ from walk_f32"
+        assert (leaves[slots] > 0).all() and not pre[idx].any()
+        p64 = leaves.astype(np.float64)
+        beta = P.beta_at(st["updates"], float(F32(per["beta"])), per["beta_steps"])
+        w = (p64[slots] / p64[p64 > 0].min()) ** -beta
+        n_dup = B - len(np.unique(slots))
+        print(f"    per: t {st['updates']} beta {beta:.6f} w in [{w.min():.3g}, {w.max():.3g}]; duplicate rows {n_dup}; "
+              f"zero-priority (flagged) ring rows {int(pre.sum())}")
     else:
         m = eng.update_host(idx, e1, e2, 1)
     if not grads:
@@ -292,19 +358,22 @@ def one_update(eng, c, ring, rng, worst, grads=False):
         _bar(name, rel_l2(got if isinstance(got, np.ndarray) else _np(got), ref), 2e-5, worst)
 
     # ---- critics
+    # prioritized replay: loss (1/B) sum w diff^2 (w = (p / p_min)^-beta(t)); uniform: w = 1
     x = np.concatenate([f64(s), f64(a)], axis=1)
+    wt = w if per else np.ones(B)
     for cc, tag in ((1, "q1"), (2, "q2")):
         q = _mlp(st[tag], c["actfn"], c["out_act"])
         qv, cache = q.forward(x)
         diff = qv[:, 0] - y
-        _, cache, deltas, _ = oracle_forward_backward(q, x, (2 * diff / B)[:, None])
+        _, cache, deltas, _ = oracle_forward_backward(q, x, (2 * wt * diff / B)[:, None])
         _bar("q", rel_l2(_np(eng.view(f"out.q{cc}")), qv[:, 0]), 2e-5, worst)
         _bar("dout", rel_l2(_np(eng.view(f"scr.dout{cc}"))[:, 0], deltas[-1][:, 0]), 2e-5, worst)
-        _bar("q loss rows", rel_l2(_np(eng.view(f"scr.lossrow{cc}")), diff * diff), 2e-5, worst)
+        _bar("q loss rows", rel_l2(_np(eng.view(f"scr.lossrow{cc}")), wt * diff * diff), 2e-5, worst)
         if not grads:
-            _bar("q loss", abs(m[f"q{cc}_loss"] - np.mean(diff * diff)) / np.mean(diff * diff), 2e-5, worst)
+            ql = np.mean(wt * diff * diff)
+            _bar("q loss", abs(m[f"q{cc}_loss"] - ql) / ql, 2e-5, worst)
         g = _engine_grads(eng, tag, nq, grads)
-        ref = q.backward(cache, (2 * diff / B)[:, None])
+        ref = q.backward(cache, (2 * wt * diff / B)[:, None])
         no = np.zeros(B, bool)
         _check_grads(tag, [g[f"net.{2 * l}.weight"] for l in range(nq)], [g[f"net.{2 * l}.bias"] for l in range(nq)], ref[0], ref[1],
                      deltas, cache["h"][:nq], deltas, cache["h"][:nq], no, worst)
@@ -369,6 +438,8 @@ def one_update(eng, c, ring, rng, worst, grads=False):
     if grads:
         return int(pre.sum()), int(flags.sum())
     _check_adam(eng, "pi", npi, st["pi"], st["v"]["pi"], st["step"][0], 3e-4, g, worst)
+    if per:
+        _check_write_back(eng, per, slots, leaves, pmax, worst)
 
     # ---- temperature
     la = float(eng.view("scal.log_alpha").item())
@@ -385,6 +456,27 @@ def one_update(eng, c, ring, rng, worst, grads=False):
     else:
         assert la == st["log_alpha"], "fixed temperature: log_alpha moved"
     return int(pre.sum()), int(flags.sum())
+
+
+def _check_write_back(eng, per, slots, leaves, pmax, worst):
+    """The update's deferred write-back, applied by the read: each sampled slot holds (delta + eps)^alpha of its highest row
+    (delta in float64 from the engine's own out.q1 / q2 / y; rel 2e-6 for float32 powf), every other leaf keeps its bits,
+    p_max is the float32 max."""
+    from oracle import per_numpy as P
+    q1, q2, y = (_np(eng.view(v)).ravel() for v in ("out.q1", "out.q2", "out.y"))
+    pr = P.priority(P.td_delta(q1, q2, y), float(F32(per["alpha"])), float(F32(per["eps"])))
+    after, pmax_after = eng.per.slot_priorities()
+    after = after.cpu().numpy()
+    last = {}
+    for k, s in enumerate(slots.tolist()):
+        last[s] = k                                   # the highest row wins a slot drawn more than once
+    ss, ks = np.array(list(last)), np.array(list(last.values()))
+    _bar("priority (rel)", float(np.max(np.abs(after[ss] - pr[ks]) / pr[ks])), 2e-6, worst)
+    rest = np.ones(len(after), bool)
+    rest[ss] = False
+    assert np.array_equal(after[rest], leaves[rest]), "write-back changed a leaf it did not sample"
+    assert pmax_after >= max(pmax, float(after.max()))
+    _bar("p_max (rel)", abs(pmax_after - max(pmax, pr.max())) / max(pmax, pr.max()), 2e-6, worst)
 
 
 def run_updates(eng, c, ring, rng, n=2, grads=False):
