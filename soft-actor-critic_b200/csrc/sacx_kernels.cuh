@@ -591,10 +591,9 @@ __global__ void act_kernel(const float* __restrict__ base, NetRef net, int maxw,
     if (deterministic) {
       v = tanhf(mu) * scale;                                     // models.py:89-92
     } else {
-      const float ls = fminf(fmaxf(head[A + j], lo), hi);
       const float e = eps ? eps[(i64)row * A + j]
                           : philox_normal(scal->rng_seed, counter, 3, (uint32_t)blockIdx.x, (uint32_t)j, scal->rng_agent);
-      v = tanhf(mu + e * expf(ls)) * scale;                      // models.py:79-84
+      v = sac_rsample(mu, head[A + j], e, lo, hi).tz * scale;     // models.py:79-84
     }
     a_out[(i64)row * A + j] = v;
   }

@@ -1,6 +1,7 @@
 // Elementwise math of the SAC update: the seven activations of the reference's _ACTIVATIONS table
-// (sac/models.py:104-112) with the derivative forms torch's backward uses, torch's softplus, and the
-// counter-based RNGs of the throughput mode (Philox4x32-10 normals, keyed Feistel index bijection).
+// (sac/models.py:104-112) with the derivative forms torch's backward uses, torch's softplus, the per-row formulas of
+// the losses and their gradients that every kernel path calls, and the counter-based RNGs of the throughput mode
+// (Philox4x32-10 normals, keyed Feistel index bijection).
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
@@ -65,6 +66,73 @@ __device__ __forceinline__ float act_dz2(int act, float z, float h) { return act
 
 // F.softplus(beta=1, threshold=20)
 __device__ __forceinline__ float softplus20(float x) { return x > 20.f ? x : log1pf(expf(x)); }
+
+// ---------------------------------------------------------------- per-row SAC formulas
+// Each per-row formula of the update, stated once for the tile row ops, the tensor-core tails, the row-parallel kernel and
+// act_kernel; loads, stores and the work split stay with the callers. Fixed operation order: equal inputs, equal bits on every path.
+
+// tanh-squashed Gaussian rsample and its log-prob for one action dimension (models.py:79-87). The caller scales tz by
+// action_scale and stores se = sd * e; in_clamp is the mask of the log_std clamp's gradient, bad flags a non-finite head.
+struct SacSample { float tz, sd, lp; bool in_clamp, bad; };
+__device__ __forceinline__ SacSample sac_rsample(float mu, float ls_raw, float e, float lo, float hi) {
+  const float sd = expf(fminf(fmaxf(ls_raw, lo), hi));
+  const float z = mu + e * sd;                       // Normal.rsample: loc + eps * scale
+  const float dzm = z - mu;
+  // Normal.log_prob: -(z-mu)^2 / (2 var) - log(std) - log(sqrt(2 pi))
+  float lp = -(dzm * dzm) / (2.f * (sd * sd)) - logf(sd) - 0.91893853320467274178f;
+  // tanh Jacobian, softplus form: 2 (log 2 - z - softplus(-2 z))   (F7: no -log(action_scale))
+  lp -= 2.f * (0.69314718055994530942f - z - softplus20(-2.f * z));
+  return {tanhf(z), sd, lp, ls_raw >= lo && ls_raw <= hi, !(isfinite(mu) && isfinite(sd))};
+}
+
+// soft Bellman target y = r + gamma (1 - d) (min(Q1t, Q2t) - alpha logpi')      (agent.py:208-210)
+__device__ __forceinline__ float sac_target(float r, float d, float gamma, float alpha, float tq1, float tq2, float lp2) {
+  return r + (gamma * (1.f - d)) * (fminf(tq1, tq2) - alpha * lp2);
+}
+
+// one critic's row of the weighted mse (agent.py:213-236, DESIGN §8): q = act(z), loss w diff^2, and d loss / d z =
+// 2 w diff / B through the output activation. w is the importance weight of prioritized replay, 1.f (exact) without it.
+struct SacCriticRow { float q, dout, loss; };
+__device__ __forceinline__ SacCriticRow sac_critic_row(int act_out, float z, float y, float w, int B_global) {
+  const float q = act_fwd(act_out, z), dq = act_dz2(act_out, z, q), diff = q - y;
+  return {q, (2.f * (w * diff) / (float)B_global) * dq, w * (diff * diff)};
+}
+
+// torch.min backward of the policy loss (agent.py:238-260): gradient to the smaller critic, ties split 1/2 - 1/2, through
+// each critic's output activation
+struct SacRoute { float c1, c2; };
+__device__ __forceinline__ SacRoute sac_actor_route(int act_out, float z1, float q1, float z2, float q2, int B_global) {
+  const float w1 = q1 < q2 ? 1.f : (q1 == q2 ? 0.5f : 0.f);
+  const float g1 = -w1 / (float)B_global, g2 = -(1.f - w1) / (float)B_global;
+  return {g1 * act_dz2(act_out, z1, q1), g2 * act_dz2(act_out, z2, q2)};
+}
+__device__ __forceinline__ float sac_policy_loss_row(float alpha, float lp, float q1, float q2) { return alpha * lp - fminf(q1, q2); }
+
+// closed-form head backward (SURVEY a8), da = dQ/da of both critics, ab = alpha / B: dL/dz = ab 2 tanh z + da c (1 - tanh^2 z),
+// dL/dmu = dL/dz, dL/dlogstd_raw = (sigma eps dL/dz - ab) mask; then through the head's activation (zm, zl: pre-activations)
+struct SacHeadGrad { float dmu, dls; };
+__device__ __forceinline__ SacHeadGrad sac_head_bwd(int act_out, float tz, float se, float mk, float da, float ab,
+                                                    float action_scale, float zm, float zl) {
+  const float dz = ab * (2.f * tz) + da * (action_scale * (1.f - tz * tz));
+  float dmu = dz, dls = (se * dz - ab) * mk;
+  if (act_out != SACX_ACT_IDENTITY) {
+    dmu *= act_dz2(act_out, zm, act_fwd(act_out, zm));
+    dls *= act_dz2(act_out, zl, act_fwd(act_out, zl));
+  }
+  return {dmu, dls};
+}
+
+// delta of a hidden layer: s act'(h), or c w act'(h) behind an output layer of width 1; h is the saved activation. act by
+// reference, so a caller's op.act is read per element: by value, nvcc merges a float4's four act_dz tests into one branch
+// and copies the products into both sides (+28 FMUL per tile kernel)
+__device__ __forceinline__ float sac_dact(float s, float h, const int& act) { return s * act_dz(act, h); }
+__device__ __forceinline__ float4 sac_dact(float4 s, float4 h, const int& act) {
+  return make_float4(s.x * act_dz(act, h.x), s.y * act_dz(act, h.y), s.z * act_dz(act, h.z), s.w * act_dz(act, h.w));
+}
+__device__ __forceinline__ float sac_delta(float c, float w, float h, const int& act) { return c * w * act_dz(act, h); }
+__device__ __forceinline__ float4 sac_delta(float c, float4 w, float4 h, const int& act) {
+  return make_float4(c * w.x * act_dz(act, h.x), c * w.y * act_dz(act, h.y), c * w.z * act_dz(act, h.z), c * w.w * act_dz(act, h.w));
+}
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

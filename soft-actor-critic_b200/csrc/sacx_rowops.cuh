@@ -204,25 +204,16 @@ __device__ __noinline__ void tile_pi_head(const Op& op, const RowCtx& c, int til
   float lp_part = 0.f;
   bool bad = false;
   for (int j = lane; j < A; j += 32) {
-    const float mu = hs[j], ls_raw = hs[A + j];
-    const float ls = fminf(fmaxf(ls_raw, hp.log_std_min), hp.log_std_max);
-    const float sd = expf(ls);
     const float e = e_pre;
     base[op.o[5] + (i64)row * A + j] = e;
-    const float z = mu + e * sd;                       // Normal.rsample: loc + eps * scale
-    const float tz = tanhf(z);
-    base[op.o[3] + (i64)row * op.i[2] + hp.obs + j] = tz * hp.action_scale;
-    const float dzm = z - mu;
-    // Normal.log_prob: -(z-mu)^2 / (2 var) - log(std) - log(sqrt(2 pi))
-    float lp = -(dzm * dzm) / (2.f * (sd * sd)) - logf(sd) - 0.91893853320467274178f;
-    // tanh Jacobian, softplus form: 2 (log 2 - z - softplus(-2 z))   (F7: no -log(action_scale))
-    lp -= 2.f * (0.69314718055994530942f - z - softplus20(-2.f * z));
-    lp_part += lp;
-    bad |= !(isfinite(mu) && isfinite(sd));
+    const SacSample s = sac_rsample(hs[j], hs[A + j], e, hp.log_std_min, hp.log_std_max);
+    base[op.o[3] + (i64)row * op.i[2] + hp.obs + j] = s.tz * hp.action_scale;
+    lp_part += s.lp;
+    bad |= s.bad;
     if (op.o[6] >= 0) {
-      base[op.o[6] + (i64)row * A + j] = tz;
-      base[op.o[7] + (i64)row * A + j] = sd * e;
-      base[op.o[8] + (i64)row * A + j] = (ls_raw >= hp.log_std_min && ls_raw <= hp.log_std_max) ? 1.f : 0.f;
+      base[op.o[6] + (i64)row * A + j] = s.tz;
+      base[op.o[7] + (i64)row * A + j] = s.sd * e;
+      base[op.o[8] + (i64)row * A + j] = s.in_clamp ? 1.f : 0.f;
     }
   }
   if (op.o[9] >= 0)
@@ -237,7 +228,7 @@ __device__ __noinline__ void tile_pi_head(const Op& op, const RowCtx& c, int til
 // ---------------------------------------------------------------- OP_PI_TAIL (large batch, tensor-core path)
 // The policy's output layer is a skinny GEMM (N = 2A) that the tensor-core kernel runs like any other layer; what is left of
 // OP_PI_HEAD is per-row scalar work, so ONE THREAD owns a row (256 rows per tile) instead of one warp: ~30x fewer warp
-// instructions per row than the shuffle-reduced head. Same arithmetic as tile_pi_head (models.py:79-87).
+// instructions per row than the shuffle-reduced head. Same sac_rsample as tile_pi_head.
 // o[0]=z (head pre-activations [B][i[3]]) o[3]=X(dest) o[4]=lp o[5]=eps buf o[6]=tz o[7]=se o[8]=mask o[9]=compact z copy (-1: not saved)
 // i[2]=ldx i[3]=row stride of z   mode 1/2
 constexpr int TAIL_ROWS = 256;
@@ -258,23 +249,17 @@ __device__ __forceinline__ void tile_pi_tail(const Op& op, const RowCtx& c, int 
     const float zm = __ldcg(z + j), zl = __ldcg(z + A + j);
     if (op.o[9] >= 0) { base[op.o[9] + (i64)row * 2 * A + j] = zm; base[op.o[9] + (i64)row * 2 * A + A + j] = zl; }
     const float mu = act_fwd(op.act_out, zm), ls_raw = act_fwd(op.act_out, zl);
-    const float ls = fminf(fmaxf(ls_raw, hp.log_std_min), hp.log_std_max);
-    const float sd = expf(ls);
     const float e = eps_ext ? eps_ext[(((i64)c.step * a.n_agents + c.agent) * hp.B + row) * A + j]
                             : philox_normal(rng_seed, upd, op.mode, (uint32_t)(hp.row0_global + row), (uint32_t)j, rng_agent);
     base[op.o[5] + (i64)row * A + j] = e;
-    const float zz = mu + e * sd;                      // Normal.rsample: loc + eps * scale
-    const float tz = tanhf(zz);
-    base[op.o[3] + (i64)row * op.i[2] + hp.obs + j] = tz * hp.action_scale;
-    const float dzm = zz - mu;
-    float l = -(dzm * dzm) / (2.f * (sd * sd)) - logf(sd) - 0.91893853320467274178f;
-    l -= 2.f * (0.69314718055994530942f - zz - softplus20(-2.f * zz));
-    lp += l;
-    bad |= !(isfinite(mu) && isfinite(sd));
+    const SacSample s = sac_rsample(mu, ls_raw, e, hp.log_std_min, hp.log_std_max);
+    base[op.o[3] + (i64)row * op.i[2] + hp.obs + j] = s.tz * hp.action_scale;
+    lp += s.lp;
+    bad |= s.bad;
     if (op.o[6] >= 0) {
-      base[op.o[6] + (i64)row * A + j] = tz;
-      base[op.o[7] + (i64)row * A + j] = sd * e;
-      base[op.o[8] + (i64)row * A + j] = (ls_raw >= hp.log_std_min && ls_raw <= hp.log_std_max) ? 1.f : 0.f;
+      base[op.o[6] + (i64)row * A + j] = s.tz;
+      base[op.o[7] + (i64)row * A + j] = s.sd * e;
+      base[op.o[8] + (i64)row * A + j] = s.in_clamp ? 1.f : 0.f;
     }
   }
   base[op.o[4] + row] = lp;
@@ -298,7 +283,7 @@ __device__ __forceinline__ void tile_q_tail(const Op& op, const RowCtx& c, int t
   if (op.mode & 1) {
     const float t0 = act_fwd(op.act_out, __ldcg(base + op.o[0] + row)), t1 = act_fwd(op.act_out, __ldcg(base + op.o[1] + row));
     const float r = __ldcg(base + op.o[6] + row), d = __ldcg(base + op.o[7] + row), lp2 = __ldcg(base + op.o[8] + row);
-    y = r + (__ldcg(&c.scal->gamma) * (1.f - d)) * (fminf(t0, t1) - alpha * lp2);
+    y = sac_target(r, d, __ldcg(&c.scal->gamma), alpha, t0, t1, lp2);
     base[op.o[0] + row] = t0; base[op.o[1] + row] = t1; base[op.o[9] + row] = y;
   }
   if (op.mode & 2) {
@@ -306,20 +291,20 @@ __device__ __forceinline__ void tile_q_tail(const Op& op, const RowCtx& c, int t
     const float w = c.args->w_ext ? __ldcg(c.args->w_ext + row) : 1.f;     // importance weight; 1 multiplies exactly
 #pragma unroll
     for (int cc = 0; cc < 2; ++cc) {
-      const float z = __ldcg(base + op.o[2 + cc] + row), q = act_fwd(op.act_out, z), diff = q - y;
-      base[op.o[2 + cc] + row] = q;
-      base[op.o[10 + cc] + (i64)row * 4] = (2.f * (w * diff) / (float)hp.B_global) * act_dz2(op.act_out, z, q);
-      base[op.o[12 + cc] + row] = w * (diff * diff);
+      const SacCriticRow cr = sac_critic_row(op.act_out, __ldcg(base + op.o[2 + cc] + row), y, w, hp.B_global);
+      base[op.o[2 + cc] + row] = cr.q;
+      base[op.o[10 + cc] + (i64)row * 4] = cr.dout;
+      base[op.o[12 + cc] + row] = cr.loss;
     }
   }
   if (op.mode & 4) {
     const float z0 = __ldcg(base + op.o[4] + row), z1 = __ldcg(base + op.o[5] + row);
     const float q0 = act_fwd(op.act_out, z0), q1 = act_fwd(op.act_out, z1);
-    const float w1 = q0 < q1 ? 1.f : (q0 == q1 ? 0.5f : 0.f);            // torch.min backward, ties split
+    const SacRoute g = sac_actor_route(op.act_out, z0, q0, z1, q1, hp.B_global);
     base[op.o[4] + row] = q0; base[op.o[5] + row] = q1;
-    base[op.o[10] + (i64)row * 4] = (-w1 / (float)hp.B_global) * act_dz2(op.act_out, z0, q0);
-    base[op.o[11] + (i64)row * 4] = (-(1.f - w1) / (float)hp.B_global) * act_dz2(op.act_out, z1, q1);
-    base[op.o[15] + row] = alpha * __ldcg(base + op.o[14] + row) - fminf(q0, q1);
+    base[op.o[10] + (i64)row * 4] = g.c1;
+    base[op.o[11] + (i64)row * 4] = g.c2;
+    base[op.o[15] + row] = sac_policy_loss_row(alpha, __ldcg(base + op.o[14] + row), q0, q1);
   }
 }
 
@@ -352,9 +337,7 @@ __device__ __forceinline__ void tile_delta(const Op& op, const RowCtx& c, int ti
     for (int u = 0; u < U; ++u) {
       const int r = rbase + u * rstep, row = rb + r;
       if (r < DELTA_ROWS && row < hp.B)
-        *reinterpret_cast<float4*>(base + op.o[6 + cc] + (i64)row * ld + k) =
-            make_float4(co[u] * w.x * act_dz(op.act, h[u].x), co[u] * w.y * act_dz(op.act, h[u].y), co[u] * w.z * act_dz(op.act, h[u].z),
-                        co[u] * w.w * act_dz(op.act, h[u].w));
+        *reinterpret_cast<float4*>(base + op.o[6 + cc] + (i64)row * ld + k) = sac_delta(co[u], w, h[u], op.act);
     }
   }
 }
@@ -430,9 +413,7 @@ __device__ __noinline__ void tile_q_row(const Op& op, const RowCtx& c, int tile)
       const float part = fast ? row_dot_partial(ht[n], W, K, lane) : warp_dot_any(hp_t[n], W, K, lane);
       tq[n] = act_fwd(op.act_out, warp_sum(part) + bt[n]);
     }
-    const float r = r_, d = d_, lp2 = lp2_;
-    // y = r + gamma * (1 - d) * (min(Q1t, Q2t) - alpha * logpi')      (agent.py:208-210)
-    y = r + (__ldcg(&c.scal->gamma) * (1.f - d)) * (fminf(tq[0], tq[1]) - alpha * lp2);
+    y = sac_target(r_, d_, __ldcg(&c.scal->gamma), alpha, tq[0], tq[1], lp2_);
     if (lane == 0) {
       base[op.o[9] + row] = y;
       base[op.o[10] + row] = tq[0];
@@ -445,15 +426,12 @@ __device__ __noinline__ void tile_q_row(const Op& op, const RowCtx& c, int tile)
     for (int n = 0; n < 2; ++n) {
       const float* W = staged ? Ws + (2 + n) * K : base + op.o[16 + n];
       const float part = fast ? row_dot_partial(hc[n], W, K, lane) : warp_dot_any(hp_c[n], W, K, lane);
-      const float z = warp_sum(part) + bc_[n];
-      const float q = act_fwd(op.act_out, z);
-      const float diff = q - y;
-      // d mse / d q = 2 w (q - y) / B (w: importance weight, 1 without prioritized replay); through the output activation
-      const float dout = (2.f * (w_in * diff) / (float)hp.B_global) * act_dz2(op.act_out, z, q);
+      const SacCriticRow cr = sac_critic_row(op.act_out, warp_sum(part) + bc_[n], y, w_in, hp.B_global);
+      const float dout = cr.dout;
       if (lane == 0) {
-        base[op.o[20 + n] + row] = q;
+        base[op.o[20 + n] + row] = cr.q;
         base[op.o[22 + n] + (i64)row * 4] = dout;
-        base[op.o[26 + n] + row] = w_in * (diff * diff);
+        base[op.o[26 + n] + row] = cr.loss;
       }
       float* dl = base + op.o[24 + n] + (i64)row * ld;
       if (fast) {
@@ -461,15 +439,10 @@ __device__ __noinline__ void tile_q_row(const Op& op, const RowCtx& c, int tile)
 #pragma unroll
         for (int i = 0; i < ROW_KREG; ++i) {
           const int k = (lane + 32 * i) * 4;
-          if (k < K) {
-            const float4 w = *reinterpret_cast<const float4*>(W + k);
-            *reinterpret_cast<float4*>(dl + k) =
-                make_float4(dout * w.x * act_dz(op.act, ar.v[i].x), dout * w.y * act_dz(op.act, ar.v[i].y),
-                            dout * w.z * act_dz(op.act, ar.v[i].z), dout * w.w * act_dz(op.act, ar.v[i].w));
-          }
+          if (k < K) *reinterpret_cast<float4*>(dl + k) = sac_delta(dout, *reinterpret_cast<const float4*>(W + k), ar.v[i], op.act);
         }
       } else {
-        for (int k = lane; k < K; k += 32) dl[k] = dout * W[k] * act_dz(op.act, __ldcg(ax_c[n] + k));
+        for (int k = lane; k < K; k += 32) dl[k] = sac_delta(dout, W[k], __ldcg(ax_c[n] + k), op.act);
       }
     }
   }
@@ -527,17 +500,15 @@ __device__ __noinline__ void tile_actor_q(const Op& op, const RowCtx& c, int til
     z[n] = warp_sum(part) + bq[n];
     q[n] = act_fwd(op.act_out, z[n]);
   }
-  // torch.min backward: gradient to the smaller input, ties split 1/2 - 1/2
-  const float w1 = q[0] < q[1] ? 1.f : (q[0] == q[1] ? 0.5f : 0.f);
-  const float g[2] = {-w1 / (float)hp.B_global, -(1.f - w1) / (float)hp.B_global};
+  const SacRoute g = sac_actor_route(op.act_out, z[0], q[0], z[1], q[1], hp.B_global);
   if (lane == 0) {
     base[op.o[9] + row] = q[0];
     base[op.o[10] + row] = q[1];
-    base[op.o[15] + row] = alpha * lp_ - fminf(q[0], q[1]);
+    base[op.o[15] + row] = sac_policy_loss_row(alpha, lp_, q[0], q[1]);
   }
 #pragma unroll
   for (int n = 0; n < 2; ++n) {
-    const float dout = g[n] * act_dz2(op.act_out, z[n], q[n]);
+    const float dout = n ? g.c2 : g.c1;
     const float* W = staged ? Ws + n * K : base + op.o[4 + n];
     float* dl = base + op.o[13 + n] + (i64)row * ld;
     if (fast) {
@@ -545,15 +516,10 @@ __device__ __noinline__ void tile_actor_q(const Op& op, const RowCtx& c, int til
 #pragma unroll
       for (int i = 0; i < ROW_KREG; ++i) {
         const int k = (lane + 32 * i) * 4;
-        if (k < K) {
-          const float4 w = *reinterpret_cast<const float4*>(W + k);
-          *reinterpret_cast<float4*>(dl + k) =
-              make_float4(dout * w.x * act_dz(op.act, a2.v[i].x), dout * w.y * act_dz(op.act, a2.v[i].y),
-                          dout * w.z * act_dz(op.act, a2.v[i].z), dout * w.w * act_dz(op.act, a2.v[i].w));
-        }
+        if (k < K) *reinterpret_cast<float4*>(dl + k) = sac_delta(dout, *reinterpret_cast<const float4*>(W + k), a2.v[i], op.act);
       }
     } else {
-      for (int k = lane; k < K; k += 32) dl[k] = dout * W[k] * act_dz(op.act, __ldcg(ax[n] + k));
+      for (int k = lane; k < K; k += 32) dl[k] = sac_delta(dout, W[k], __ldcg(ax[n] + k), op.act);
     }
   }
   SACX_RSTAMP(4);
@@ -630,20 +596,11 @@ __device__ __noinline__ void tile_actor_bwd(const Op& op, const RowCtx& c, int t
   __syncwarp();
   const float ab = alpha / (float)hp.B_global;
   for (int j = lane; j < A; j += 32) {
-    const float tz = tz_, se = se_, mk = mk_;
-    // dL/dz = (alpha/B) 2 tanh z + dL/da * c (1 - tanh^2 z);  dL/dmu = dL/dz;
-    // dL/dlogstd_raw = (sigma eps dL/dz - alpha/B) * 1[lo <= raw <= hi]
-    const float dz = ab * (2.f * tz) + da[j] * (hp.action_scale * (1.f - tz * tz));
-    float dmu = dz, dls = (se * dz - ab) * mk;
-    if (op.act_out != SACX_ACT_IDENTITY) {
-      const float zm = zm_, zl = zl_;
-      dmu *= act_dz2(op.act_out, zm, act_fwd(op.act_out, zm));
-      dls *= act_dz2(op.act_out, zl, act_fwd(op.act_out, zl));
-    }
-    dh[j] = dmu;
-    dh[A + j] = dls;
-    base[op.o[8] + (i64)row * 2 * A + j] = dmu;
-    base[op.o[8] + (i64)row * 2 * A + A + j] = dls;
+    const SacHeadGrad g = sac_head_bwd(op.act_out, tz_, se_, mk_, da[j], ab, hp.action_scale, zm_, zl_);
+    dh[j] = g.dmu;
+    dh[A + j] = g.dls;
+    base[op.o[8] + (i64)row * 2 * A + j] = g.dmu;
+    base[op.o[8] + (i64)row * 2 * A + A + j] = g.dls;
   }
   __syncwarp();
   // delta of the policy's last hidden layer: (dhead . Wpi_L) * act'(.)
@@ -659,8 +616,7 @@ __device__ __noinline__ void tile_actor_bwd(const Op& op, const RowCtx& c, int t
           const float g = dh[j];
           s.x = fmaf(g, w.x, s.x); s.y = fmaf(g, w.y, s.y); s.z = fmaf(g, w.z, s.z); s.w = fmaf(g, w.w, s.w);
         }
-        *reinterpret_cast<float4*>(dl + k) = make_float4(s.x * act_dz(op.act, ap.v[i].x), s.y * act_dz(op.act, ap.v[i].y),
-                                                         s.z * act_dz(op.act, ap.v[i].z), s.w * act_dz(op.act, ap.v[i].w));
+        *reinterpret_cast<float4*>(dl + k) = sac_dact(s, ap.v[i], op.act);
       }
     }
   } else {
@@ -668,7 +624,7 @@ __device__ __noinline__ void tile_actor_bwd(const Op& op, const RowCtx& c, int t
     for (int k = lane; k < Kp; k += 32) {
       float s = 0.f;
       for (int j = 0; j < 2 * A; ++j) s = fmaf(dh[j], staged ? W[j * Kp + k] : __ldcg(W + (i64)j * Kp + k), s);
-      dl[k] = s * act_dz(op.act, __ldcg(auxp + k));
+      dl[k] = sac_dact(s, __ldcg(auxp + k), op.act);
     }
   }
   __syncwarp();

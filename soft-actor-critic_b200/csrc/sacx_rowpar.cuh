@@ -632,28 +632,21 @@ __device__ __noinline__ void rp_pi_heads(const RpCtx& c) {
     const float bm = __ldcg(c.base + P.pi_bL + j), bl = __ldcg(c.base + P.pi_bL + A + j);
     const float zm = rp_add_parts(pm) + bm;
     const float zl = rp_add_parts(pl) + bl;
-    const float mu = act_fwd(P.act_opi, zm), ls_raw = act_fwd(P.act_opi, zl);
-    const float ls = fminf(fmaxf(ls_raw, hp.log_std_min), hp.log_std_max);
-    const float sd = expf(ls);
     const float e = which ? R.eps2[mm][j] : R.eps1[mm][j];
-    const float z = mu + e * sd;
-    const float tz = tanhf(z);
-    const float av = tz * hp.action_scale;
-    const float dzm = z - mu;
-    lp = -(dzm * dzm) / (2.f * (sd * sd)) - logf(sd) - 0.91893853320467274178f;
-    lp -= 2.f * (0.69314718055994530942f - z - softplus20(-2.f * z));
-    bad = ok && !(isfinite(mu) && isfinite(sd));
+    const SacSample s = sac_rsample(act_fwd(P.act_opi, zm), act_fwd(P.act_opi, zl), e, hp.log_std_min, hp.log_std_max);
+    const float av = s.tz * hp.action_scale;
+    lp = s.lp;
+    bad = ok && s.bad;
     if (!which) {
       xs2[mm * ldx + O + j] = ok ? av : 0.f;
       if (w0 && ok) c.base[P.x_s2 + (i64)row * P.gldx + O + j] = av;
     } else {
       xpi[mm * ldx + O + j] = ok ? av : 0.f;
-      const float mk = (ls_raw >= hp.log_std_min && ls_raw <= hp.log_std_max) ? 1.f : 0.f;
       if (w0 && ok) {
         c.base[P.x_pi + (i64)row * P.gldx + O + j] = av;
-        c.base[P.b_tz + (i64)row * A + j] = tz;
-        c.base[P.b_se + (i64)row * A + j] = sd * e;
-        c.base[P.b_mask + (i64)row * A + j] = mk;
+        c.base[P.b_tz + (i64)row * A + j] = s.tz;
+        c.base[P.b_se + (i64)row * A + j] = s.sd * e;
+        c.base[P.b_mask + (i64)row * A + j] = s.in_clamp ? 1.f : 0.f;
         c.base[P.b_headz + (i64)row * J + j] = zm;
         c.base[P.b_headz + (i64)row * J + A + j] = zl;
       }
@@ -687,10 +680,7 @@ __device__ __forceinline__ void rp_delta_critics(const RpCtx& c, const float4 (&
     const float4 w = wl[cc];
     for (int mm = m0; mm < RP_RB; mm += mstep) {
       float4* p = reinterpret_cast<float4*>(ab + mm * lda + k);
-      const float4 h = *p;
-      const float co = coef[mm];
-      const float4 dv = make_float4(co * w.x * act_dz(act, h.x), co * w.y * act_dz(act, h.y), co * w.z * act_dz(act, h.z),
-                                    co * w.w * act_dz(act, h.w));
+      const float4 dv = sac_delta(coef[mm], w, *p, act);
       *p = dv;
       if (mine && mm < nrows) *reinterpret_cast<float4*>(dq + (i64)mm * ld) = dv;
     }
@@ -727,18 +717,14 @@ __device__ __noinline__ void rp_target_critic(const RpCtx& c) {
     const float st[2] = {rp_add_parts(pt[0]), rp_add_parts(pt[1])};
     const float sq[2] = {rp_add_parts(pq[0]), rp_add_parts(pq[1])};
     const float tq[2] = {act_fwd(P.act_oq, st[0] + bt[0]), act_fwd(P.act_oq, st[1] + bt[1])};
-    const float y = R.r[mm] + (__ldcg(&c.scal->gamma) * (1.f - R.d[mm])) * (fminf(tq[0], tq[1]) - alpha * R.lp2[mm]);
+    const float y = sac_target(R.r[mm], R.d[mm], __ldcg(&c.scal->gamma), alpha, tq[0], tq[1], R.lp2[mm]);
     const float wr = (WEIGHTED && ok) ? __ldcg(c.args->w_ext + row) : 1.f;
     if (w0 && ok) { c.base[P.b_y + row] = y; c.base[P.b_tq[0] + row] = tq[0]; c.base[P.b_tq[1] + row] = tq[1]; }
 #pragma unroll
     for (int cc = 0; cc < 2; ++cc) {
-      const float z = sq[cc] + bq[cc];
-      const float q = act_fwd(P.act_oq, z);
-      const float diff = q - y;
-      // importance weight w (prioritized replay): loss w diff^2, gradient 2 w diff / B; w = 1 multiplies exactly
-      const float dout = (2.f * (wr * diff) / (float)hp.B_global) * act_dz2(P.act_oq, z, q);
-      R.coef[cc][mm] = ok ? dout : 0.f;
-      if (w0 && ok) { c.base[P.b_q[cc] + row] = q; c.base[P.b_dout[cc] + (i64)row * 4] = dout; c.base[P.b_loss[cc] + row] = wr * (diff * diff); }
+      const SacCriticRow cr = sac_critic_row(P.act_oq, sq[cc] + bq[cc], y, wr, hp.B_global);
+      R.coef[cc][mm] = ok ? cr.dout : 0.f;
+      if (w0 && ok) { c.base[P.b_q[cc] + row] = cr.q; c.base[P.b_dout[cc] + (i64)row * 4] = cr.dout; c.base[P.b_loss[cc] + row] = cr.loss; }
     }
   }
   RP_TRACE(2902);
@@ -822,13 +808,12 @@ __device__ __noinline__ void rp_actor_q(const RpCtx& c) {
     const float sq[2] = {rp_add_parts(pq[0]), rp_add_parts(pq[1])};
     const float z[2] = {sq[0] + bq[0], sq[1] + bq[1]};
     const float q[2] = {act_fwd(P.act_oq, z[0]), act_fwd(P.act_oq, z[1])};
-    const float w1 = q[0] < q[1] ? 1.f : (q[0] == q[1] ? 0.5f : 0.f);      // torch.min backward, ties split
-    const float g[2] = {-w1 / (float)hp.B_global, -(1.f - w1) / (float)hp.B_global};
-#pragma unroll
-    for (int cc = 0; cc < 2; ++cc) R.coef[cc][mm] = ok ? g[cc] * act_dz2(P.act_oq, z[cc], q[cc]) : 0.f;
+    const SacRoute g = sac_actor_route(P.act_oq, z[0], q[0], z[1], q[1], hp.B_global);
+    R.coef[0][mm] = ok ? g.c1 : 0.f;
+    R.coef[1][mm] = ok ? g.c2 : 0.f;
     if (w0 && ok) {
       c.base[P.b_qa[0] + row] = q[0]; c.base[P.b_qa[1] + row] = q[1];
-      c.base[P.b_ploss + row] = alpha * R.lp[mm] - fminf(q[0], q[1]);
+      c.base[P.b_ploss + row] = sac_policy_loss_row(alpha, R.lp[mm], q[0], q[1]);
     }
   }
   __syncthreads();
@@ -859,16 +844,9 @@ __device__ __forceinline__ void rp_pi_bwd_impl(const RpCtx& c) {
       rp_load_parts(c, RPP_DA1, A, mm, j, d1); rp_load_parts(c, RPP_DA2, A, mm, j, d2);
       const float alpha = __ldcg(&c.scal->alpha_f32);
       const float da = rp_add_parts(d1) + rp_add_parts(d2);
-      const float ab = alpha / (float)hp.B_global;
-      const float tz = R.tz[mm][j], se = R.se[mm][j], mk = R.mk[mm][j];
-      const float dz = ab * (2.f * tz) + da * (hp.action_scale * (1.f - tz * tz));
-      float dmu = dz, dls = (se * dz - ab) * mk;
-      if (P.act_opi != SACX_ACT_IDENTITY) {
-        const float zm = R.hz[mm][j], zl = R.hz[mm][A + j];
-        dmu *= act_dz2(P.act_opi, zm, act_fwd(P.act_opi, zm));
-        dls *= act_dz2(P.act_opi, zl, act_fwd(P.act_opi, zl));
-      }
-      if (!ok) { dmu = 0.f; dls = 0.f; }
+      const SacHeadGrad g = sac_head_bwd(P.act_opi, R.tz[mm][j], R.se[mm][j], R.mk[mm][j], da, alpha / (float)hp.B_global,
+                                         hp.action_scale, R.hz[mm][j], R.hz[mm][A + j]);
+      const float dmu = ok ? g.dmu : 0.f, dls = ok ? g.dls : 0.f;
       R.dh[mm][j] = dmu; R.dh[mm][A + j] = dls;
       if (c.rank == 0 && ok) { c.base[P.b_dhead + (i64)row * J + j] = dmu; c.base[P.b_dhead + (i64)row * J + A + j] = dls; }
     }
@@ -889,8 +867,7 @@ __device__ __forceinline__ void rp_pi_bwd_impl(const RpCtx& c) {
       }
     }
     float4* p = reinterpret_cast<float4*>(ab + mm * lda + k);
-    const float4 h = *p;
-    const float4 dv = make_float4(s.x * act_dz(act, h.x), s.y * act_dz(act, h.y), s.z * act_dz(act, h.z), s.w * act_dz(act, h.w));
+    const float4 dv = sac_dact(s, *p, act);
     *p = dv;
     if (mine && mm < nrows) *reinterpret_cast<float4*>(dp + (i64)mm * ld) = dv;
   }
