@@ -66,7 +66,10 @@ typedef struct sacx_config {
   uint64_t seed;                                              /* device RNG key (train.seed)   */
   int32_t dp_world, dp_rank;                                  /* large-batch data parallel: batch_size is per rank */
   int32_t agent_id_base;                                      /* population sharded over ranks: global id of local agent 0 (keys the device RNG streams) */
-  int32_t reserved_i;
+  int32_t n_step;                                             /* buffer.n_step: 1..16, 0 = 1 (one-step returns). Every
+                                                               * update folds R = sum_{i<m} gamma^i r[j+i] (cut at a terminal, at
+                                                               * n and at the newest record) into the gathered row; assumes a ring
+                                                               * holds one environment's transitions in time order */
 } sacx_config;
 
 typedef struct sacx_ring_s*  sacx_ring_t;    /* replaces sac.replay_buffer.ReplayBuffer        */

@@ -628,6 +628,7 @@ static int validate(const sacx_config* c) {
   const int acts[4] = {c->act_hidden_pi, c->act_out_pi, c->act_hidden_q, c->act_out_q};
   for (int a : acts) if (a < 0 || a > SACX_ACT_SELU) return fail(SACX_ERR_ACTIVATION, "unknown activation id");
   if (!(c->alpha > 0.0)) return fail(SACX_ERR_INVALID, "alpha must be positive");
+  if (c->n_step < 0 || c->n_step > 16) return fail(SACX_ERR_INVALID, "n_step out of range (0..16, 0 = 1)");
   return SACX_OK;
 }
 
@@ -1010,6 +1011,7 @@ int sacx_agent_create(const sacx_config* cfg, float* arena_dev, sacx_agent_t* ou
   hp.auto_alpha = cfg->auto_entropy_tuning;
   hp.obs = cfg->obs_dim; hp.act = cfg->act_dim; hp.B = cfg->batch_size;
   hp.B_global = cfg->batch_size * e.cfg.dp_world; hp.row0_global = cfg->batch_size * e.cfg.dp_rank;
+  hp.n_step = cfg->n_step > 0 ? cfg->n_step : 1;
   hp.seed = cfg->seed;
   if ((rc = e.build_plans())) { sacx_agent_destroy(h); return rc; }
   if ((rc = engine_setup_rp(&e))) { sacx_agent_destroy(h); return rc; }

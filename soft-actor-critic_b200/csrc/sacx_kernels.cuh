@@ -100,7 +100,10 @@ __global__ void __launch_bounds__(256, 1) sacx_run_kernel(const Plan* __restrict
           const int lt = t - op.tile0;
           switch (op.type) {
             case OP_GEMM: if (!(args.tc_skip && (op.cfg & 2))) gemm_tile<C>(op, ec, lt, gsm); break;
-            case OP_GATHER: op_gather(op, rc, lt * ROWS_PER_TILE + warp, lane); break;
+            case OP_GATHER:
+              if (sargs.hp.n_step > 1) op_gather<true>(op, rc, lt * ROWS_PER_TILE + warp, lane);
+              else op_gather<false>(op, rc, lt * ROWS_PER_TILE + warp, lane);
+              break;
             case OP_PI_HEAD: tile_pi_head<0>(op, rc, lt); __syncthreads(); break;
             case OP_PI_TAIL: tile_pi_tail(op, rc, lt); break;
             case OP_Q_TAIL: tile_q_tail(op, rc, lt); break;
@@ -322,7 +325,10 @@ __global__ void __launch_bounds__(256, 3) sacx_rows_kernel(const Plan* __restric
           }
           else if (small_dw_ok(op)) { small_dw_tile(op, base, scal, sargs.hp, lt, tsm); last_oi = -2; }
           break;
-        case OP_GATHER: op_gather(op, rc, lt * ROWS_PER_TILE + warp, lane); break;
+        case OP_GATHER:
+          if (sargs.hp.n_step > 1) op_gather<true>(op, rc, lt * ROWS_PER_TILE + warp, lane);
+          else op_gather<false>(op, rc, lt * ROWS_PER_TILE + warp, lane);
+          break;
         case OP_PI_HEAD: tile_pi_head<1>(op, rc, lt); break;
         case OP_PI_TAIL: tile_pi_tail(op, rc, lt); break;
         case OP_Q_TAIL: tile_q_tail(op, rc, lt); break;

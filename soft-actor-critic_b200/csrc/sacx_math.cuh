@@ -90,6 +90,30 @@ __device__ __forceinline__ float sac_target(float r, float d, float gamma, float
   return r + (gamma * (1.f - d)) * (fminf(tq1, tq2) - alpha * lp2);
 }
 
+// n-step returns, folded into the gathered row so that sac_target stays as it is (DESIGN.md §9). For the window of n records
+// starting at logical position j of a ring holding len transitions, the return ends at the first offset i with a terminal,
+// i = n - 1, or the newest record (pos = j + i = len - 1).
+__device__ __forceinline__ bool nstep_stop(float d, int i, int n, long long pos, long long len) {
+  return d != 0.f || i == n - 1 || pos == len - 1;
+}
+// Across the `width` lanes of a segment, lane i holding r[j+i] and d[j+i] (i < n) and e = m - 1 the offset of the window's
+// last record: R = sum_{i<m} gamma^i r[j+i] and the done column d_eff = 1 for a terminal end, else 1 - gamma^(m-1), so that
+// sac_target(R, d_eff) = R + gamma^m (1 - d_end) (min Qt - alpha logpi'). One fixed order of _rn operations (no contraction):
+// the same bits on every path and in oracle/nstep_numpy.py. Every lane of the warp calls it; every lane gets the result.
+struct NstepFold { float r, d; };
+__device__ __forceinline__ NstepFold nstep_fold(float ri, float di, int e, int n, float gamma, int width) {
+  float acc = __shfl_sync(0xffffffffu, ri, 0, width), g = 1.f;
+  for (int i = 1; i < n; ++i) {
+    const float x = __shfl_sync(0xffffffffu, ri, i, width);
+    if (i <= e) {
+      g = __fmul_rn(g, gamma);
+      acc = __fadd_rn(acc, __fmul_rn(g, x));
+    }
+  }
+  const float de = __shfl_sync(0xffffffffu, di, e, width);
+  return {acc, de != 0.f ? 1.f : __fsub_rn(1.f, g)};
+}
+
 // one critic's row of the weighted mse (agent.py:213-236, DESIGN §8): q = act(z), loss w diff^2, and d loss / d z =
 // 2 w diff / B through the output activation. w is the importance weight of prioritized replay, 1.f (exact) without it.
 struct SacCriticRow { float q, dout, loss; };

@@ -95,6 +95,9 @@ __device__ __noinline__ float warp_dot_any(const float* __restrict__ h, const fl
 
 // ---------------------------------------------------------------- OP_GATHER
 // o[0]=X_sa o[1]=X_s2 o[2]=X_pi o[3]=r o[4]=d o[5]=idx(i64)  i[0]=ldx
+// NSTEP (hp.n_step > 1): the row keeps s[j], a[j]; r becomes the n-step return R, s2 the next state of the window's last
+// record j + m - 1, d the encoded d_eff (nstep_fold in sacx_math.cuh). Lanes i < n load r, d of logical j + i.
+template <bool NSTEP>
 __device__ __forceinline__ void op_gather(const Op& op, RowCtx& c, int row, int lane) {
   const RunArgs& a = *c.args;
   const Hyper& hp = a.hp;
@@ -135,6 +138,27 @@ __device__ __forceinline__ void op_gather(const Op& op, RowCtx& c, int row, int 
   const float* rec = ring + slot * a.ring_rs;            // packed record [s | s2 | a | r | d]
   const float* rs = rec + a.ring_s;
   const float* rs2 = rec + a.ring_s2;
+  float nr = 0.f, nd = 0.f;
+  if (NSTEP) {
+    const int ns = hp.n_step;
+    i64 si = slot + lane;                                      // lane < ns <= 16 and slot < cap: valid lanes need one subtraction
+    if (si >= cap) si -= cap;
+    float ri = 0.f, di = 0.f;
+    bool stop = false;
+    if (lane < ns && j + lane < n) {
+      const float* ri_rec = ring + si * a.ring_rs;
+      ri = __ldcg(ri_rec + a.ring_r);
+      di = __ldcg(ri_rec + a.ring_d);
+      stop = nstep_stop(di, lane, ns, j + lane, n);
+    }
+    const unsigned bits = __ballot_sync(0xffffffffu, stop);
+    const int e = bits ? __ffs(bits) - 1 : 0;
+    const NstepFold f = nstep_fold(ri, di, e, ns, __ldcg(&c.scal->gamma), 32);
+    nr = f.r; nd = f.d;
+    i64 se = slot + e;
+    if (se >= cap) se -= cap;
+    rs2 = ring + se * a.ring_rs + a.ring_s2;
+  }
   float* xsa = base + op.o[0] + (i64)row * ldx;
   float* xs2 = base + op.o[1] + (i64)row * ldx;
   float* xpi = base + op.o[2] + (i64)row * ldx;
@@ -147,8 +171,8 @@ __device__ __forceinline__ void op_gather(const Op& op, RowCtx& c, int row, int 
   const float* ra = rec + a.ring_a;
   for (int k = lane; k < A; k += 32) xsa[O + k] = __ldcs(ra + k);
   if (lane == 0) {
-    base[op.o[3] + row] = __ldcs(rec + a.ring_r);
-    base[op.o[4] + row] = __ldcs(rec + a.ring_d);
+    base[op.o[3] + row] = NSTEP ? nr : __ldcs(rec + a.ring_r);
+    base[op.o[4] + row] = NSTEP ? nd : __ldcs(rec + a.ring_d);
   }
 }
 

@@ -502,8 +502,10 @@ __device__ __forceinline__ float rp_sum8(float v) {     // sum over the 8 lanes 
 // before the first is used. Per-launch constants (push count, stream keys, update counter at launch) come from RpLaunch.
 struct RpLaunch { i64 pushes, upd0, oldest_slot; unsigned long long rng_seed; unsigned rng_agent, pad; };
 
-template <int MAXE>
-__device__ __forceinline__ void rp_gather_rows(const RpCtx& c, const i64* __restrict__ slots, const float* __restrict__ ring) {
+// NSTEP: the s2 columns come from the window's last record (slot2), r and d are the folded nr / nd (rp_nstep_fold)
+template <int MAXE, bool NSTEP>
+__device__ __forceinline__ void rp_gather_rows(const RpCtx& c, const i64* __restrict__ slots, const float* __restrict__ ring,
+                                               i64 slot2 = 0, float nr = 0.f, float nd = 0.f) {
   RP_SMEM;
   const RunArgs& a = *c.args;
   const RpProgram& P = *c.P;
@@ -514,11 +516,13 @@ __device__ __forceinline__ void rp_gather_rows(const RpCtx& c, const i64* __rest
   const int W = 2 * O + A + 2, mm = tid >> 4, c0 = tid & 15, row = c.row0 + mm;
   const i64 slot = slots[mm];
   const float* __restrict__ rec = ring + a.ring_s + (slot >= 0 ? slot : 0) * a.ring_rs;      // record = [s | s2 | a | r | d]: ring_s is its first field
+  const float* __restrict__ rec2 = NSTEP ? ring + a.ring_s + (slot >= 0 ? slot2 : 0) * a.ring_rs : rec;
   float v[MAXE];
 #pragma unroll
   for (int u = 0; u < MAXE; ++u) {
     const int col = c0 + 16 * u;
-    v[u] = (col < W && slot >= 0) ? __ldcs(rec + col) : 0.f;
+    if (NSTEP) v[u] = (col < 2 * O + A && slot >= 0) ? __ldcs((col >= O && col < 2 * O ? rec2 : rec) + col) : 0.f;
+    else v[u] = (col < W && slot >= 0) ? __ldcs(rec + col) : 0.f;
   }
   // padding columns (finite zeros: they meet zero-padded weights in the K loop)
   for (int col = O + c0; col < ldx; col += 16) {
@@ -546,14 +550,53 @@ __device__ __forceinline__ void rp_gather_rows(const RpCtx& c, const i64* __rest
         xsa[mm * ldx + col - O] = x;                       // action columns sit behind the state in X_sa
         if (ok) gsa[col - O] = x;
       } else if (col == 2 * O + A) {
-        R.r[mm] = x;
-        if (ok) *gr = x;
+        const float y = NSTEP ? nr : x;
+        R.r[mm] = y;
+        if (ok) *gr = y;
       } else {
-        R.d[mm] = x;
-        if (ok) *gd = x;
+        const float y = NSTEP ? nd : x;
+        R.d[mm] = y;
+        if (ok) *gd = y;
       }
     }
   }
+}
+
+// n-step fold of the row block (hp.n_step > 1): thread (row mm = tid >> 4, offset i = tid & 15) loads r, d of logical
+// j + i, a 16-lane ballot finds the window's end e = m - 1, and every thread of the row gets R, d_eff and the end slot --
+// the same threads then gather the row (rp_gather_rows<.., true>), so nothing goes through shared memory. Out of line:
+// the one-step gather keeps its code and its registers.
+struct RpFold { i64 slot2; float r, d; };
+__device__ __noinline__ RpFold rp_nstep_fold(const RpCtx& c, i64 slot) {
+  const RunArgs& a = *c.args;
+  const RpLaunch& L = *c.L;
+  const int i = threadIdx.x & 15, ns = a.hp.n_step;
+  const i64 cap = a.ring_capacity, len = L.pushes < cap ? L.pushes : cap;
+  i64 j = slot - L.oldest_slot;                      // logical position of the row's first record
+  if (j < 0) j += cap;
+  i64 si = slot + i;
+  if (si >= cap) si -= cap;
+  float ri = 0.f, di = 0.f;
+  bool stop = false;
+  if (slot >= 0 && i < ns && j + i < len) {
+    const float* rec = a.ring + si * a.ring_rs;
+    ri = __ldcg(rec + a.ring_r);
+    di = __ldcg(rec + a.ring_d);
+    stop = nstep_stop(di, i, ns, j + i, len);
+  }
+  const unsigned bits = (__ballot_sync(0xffffffffu, stop) >> (threadIdx.x & 16)) & 0xffffu;
+  const int e = bits ? __ffs(bits) - 1 : 0;
+  const NstepFold f = nstep_fold(ri, di, e, ns, __ldcg(&c.scal->gamma), 16);
+  i64 s2 = slot + e;
+  if (s2 >= cap) s2 -= cap;
+  return {s2, f.r, f.d};
+}
+
+__device__ __noinline__ void rp_gather_nstep(const RpCtx& c, const i64* __restrict__ slots, const float* __restrict__ ring, int W) {
+  const RpFold f = rp_nstep_fold(c, slots[threadIdx.x >> 4]);
+  if (W <= 64) rp_gather_rows<4, true>(c, slots, ring, f.slot2, f.r, f.d);
+  else if (W <= 128) rp_gather_rows<8, true>(c, slots, ring, f.slot2, f.r, f.d);
+  else rp_gather_rows<16, true>(c, slots, ring, f.slot2, f.r, f.d);
 }
 
 __device__ __noinline__ void rp_gather(const RpCtx& c, const RpLaunch& L, i64* __restrict__ slots) {
@@ -603,9 +646,10 @@ __device__ __noinline__ void rp_gather(const RpCtx& c, const RpLaunch& L, i64* _
   // body is instantiated for 4 / 8 / 16 columns per thread: with one 16-column body every update walked twelve predicated-off
   // copies of the scatter at BipedalWalker shape, all instruction-cache misses (`no_instruction` at this line in the ncu source view)
   const int W = 2 * O + A + 2;
-  if (W <= 64) rp_gather_rows<4>(c, slots, ring);
-  else if (W <= 128) rp_gather_rows<8>(c, slots, ring);
-  else rp_gather_rows<16>(c, slots, ring);
+  if (hp.n_step > 1) rp_gather_nstep(c, slots, ring, W);
+  else if (W <= 64) rp_gather_rows<4, false>(c, slots, ring);
+  else if (W <= 128) rp_gather_rows<8, false>(c, slots, ring);
+  else rp_gather_rows<16, false>(c, slots, ring);
   RP_TRACE(2103);
   __syncthreads();
 }

@@ -96,6 +96,7 @@ struct Hyper {
   float target_entropy;
   int auto_alpha;
   int obs, act, B, B_global, row0_global;            // data-parallel: this rank's rows are [row0, row0+B)
+  int n_step;                                        // buffer.n_step in 1..16: returns folded into the gathered batch
   unsigned long long seed;
 };
 

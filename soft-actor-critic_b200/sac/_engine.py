@@ -7,6 +7,7 @@ that needs the engine raises ``RuntimeError``.  Nothing here imports ``oracle/``
 from __future__ import annotations
 
 import ctypes as C
+import numbers
 import os
 from typing import Dict, Optional
 
@@ -39,7 +40,8 @@ class SacxConfig(C.Structure):
         ("alpha", C.c_double), ("actor_lr", C.c_double), ("critic_lr", C.c_double), ("alpha_lr", C.c_double),
         ("seed", C.c_uint64),
         ("dp_world", C.c_int32), ("dp_rank", C.c_int32),
-        ("agent_id_base", C.c_int32), ("reserved_i", C.c_int32),
+        ("agent_id_base", C.c_int32),
+        ("n_step", C.c_int32),            # buffer.n_step: 1..16 (0 = 1); see n_step_config
     ]
 
 
@@ -224,6 +226,25 @@ def per_config(config: dict) -> Optional[dict]:
     return {"alpha": alpha, "beta": beta, "beta_steps": int(beta_steps), "eps": eps}
 
 
+N_STEP_MAX = 16
+
+
+def n_step_config(config: dict) -> int:
+    """``buffer.n_step`` of a YAML config: an integer in 1..16, 1 (one-step returns) when absent or null. Needs no device.
+
+    With n > 1 every update's batch row j carries the n-step return R = sum_{i<m} gamma^i r[j+i], where m <= n stops at the
+    first terminal and at the newest record, the next state of record j+m-1, and the done column 1 (terminal end) or
+    1 - gamma^(m-1); the unchanged soft target r + gamma (1 - d)(min Qt - alpha log pi) then equals R + gamma^m (1 - d_end)(...).
+    The intermediate steps carry no entropy terms (they would need the policy at states outside the batch). A ring must
+    receive one environment's transitions in time order, as the training loop, SACPopulation and the DonkeyVae assembler do."""
+    n = (config.get("buffer") or {}).get("n_step")
+    if n is None:
+        return 1
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 1 <= int(n) <= N_STEP_MAX:
+        raise ValueError(f"buffer.n_step must be an integer in 1..{N_STEP_MAX}, got {n!r}")
+    return int(n)
+
+
 def make_config(obs_dim: int, act_dim: int, config: dict, n_agents: int = 1, ctas_per_agent: int = 0,
                 dp_world: int = 1, dp_rank: int = 0, batch_size: Optional[int] = None, agent_id_base: int = 0) -> SacxConfig:
     """YAML dict (reference: configs/example_config_env.yaml, sac/agent.py:22-115) -> sacx_config."""
@@ -256,4 +277,5 @@ def make_config(obs_dim: int, act_dim: int, config: dict, n_agents: int = 1, cta
     c.seed = int(tr.get("seed", 0)) & 0xFFFFFFFFFFFFFFFF
     c.dp_world, c.dp_rank = int(dp_world), int(dp_rank)
     c.agent_id_base = int(agent_id_base)
+    c.n_step = n_step_config(config)
     return c

@@ -255,8 +255,23 @@ class SAC:
         return len(self.replay_buffer) >= self.config["train"]["warming_steps"]
 
     def sample_batch(self) -> Transition:
-        """reference: agent.py:166-193 -- float32 device tensors for a ``random.sample`` index draw."""
-        return ReplayBuffer.sample_tensors(self.replay_buffer, self.config["train"]["batch_size"])
+        """reference: agent.py:166-193 -- float32 device tensors for a ``random.sample`` index draw.
+
+        With ``buffer.n_step`` > 1 the batch is gathered by the engine, so the per-phase methods see the folded batch
+        ``training_step`` trains on (n-step return, next state at the window's end, encoded done column): indices from the
+        reference's stream in host-RNG mode, else the device draw the next ``training_step`` would make."""
+        B = self.config["train"]["batch_size"]
+        if self.engine.cfg.n_step <= 1:
+            return ReplayBuffer.sample_tensors(self.replay_buffer, B)
+        idx = None
+        if self.rng_mode == "host":
+            idx = torch.as_tensor(np.asarray(self.replay_buffer.draw_indices(B), dtype=np.int64)).to(self.device)
+        else:
+            self.replay_buffer._require(B)
+        self.engine.sample_batch(idx)
+        sa, s2a, O = self._views["batch.sa"], self._views["batch.s2a"], self.obs_size
+        return Transition(sa[:, :O].clone(), sa[:, O:].clone(), self._views["batch.r"].reshape(-1).clone(),
+                          s2a[:, :O].clone(), self._views["batch.d"].reshape(-1).clone())
 
     # ------------------------------------------------------------------ acting
     def select_action(self, state: Any, deterministic: bool = False) -> Any:
