@@ -21,6 +21,10 @@ Why the comparisons are built the way they are:
 with grads_only, no apply in between): the same comparisons on the gradients the engine stores in `g.*`, without the optimiser,
 Polyak and temperature checks.
 
+A population engine (test_gpu_population_oracle.py) launches once for all agents, so the pieces are separate: `prepare` before
+the launch, `_poison` and `check_update` per agent after it. Each reads only the views of its `agent` (default 0), and the
+oracle takes gamma, the three learning rates and the temperature's from that agent's scalar block (`hyper`), as the kernels do.
+
 `case(..., per={...})` runs prioritized replay (test_gpu_per_oracle.py): a PrioritizedReplayBuffer with loaded priorities is
 attached and `update(None, eps1, eps2, 1)` lets the tree draw the batch. Every ring row on a discontinuity gets priority 0, which
 the walk never takes; batch.idx must equal oracle/per_numpy.py's walk_f32 on the loaded leaves with per_uniform's stream, bit
@@ -93,11 +97,14 @@ def _clamp_rows(head, A, lo, hi):
     return ((np.abs(ls - lo) < THR * max(1.0, abs(lo))) | (np.abs(ls - hi) < THR * max(1.0, abs(hi)))).any(axis=1)
 
 
-def _poison(eng):
-    """NaN over every per-update float buffer, padding columns included (batch.idx too: its words become a huge index)."""
+def _poison(eng, agent=0):
+    """NaN over every per-update float buffer of `agent`, padding columns included (batch.idx too: its words become a huge
+    index), and over its g.* (the fused update must leave them NaN, the gradient-only entry points must write all of them)."""
     for name, (off, rows, cols, ld, dtype) in eng.layout.items():
         if name.startswith(POISON):
-            eng.arena[off: off + rows * ld * (1 if dtype == 0 else 2)].fill_(float("nan"))
+            base = agent * eng.stride + off
+            eng.arena[base: base + rows * ld * (1 if dtype == 0 else 2)].fill_(float("nan"))
+    eng.view("block.g", agent).fill_(float("nan"))
 
 
 def _bar(what, e, bar, worst):
@@ -118,22 +125,22 @@ def _check_grads(what, eng_gW, eng_gb, ref_gW, ref_gb, g_deltas, g_inputs, o_del
         assert err < lim, f"{what}.b{l} grad: |err| {err:.3e} >= {lim:.3e}"
 
 
-def _engine_grads(eng, tag, n_lin, grads):
+def _engine_grads(eng, tag, n_lin, grads, agent=0):
     """The gradient the engine computed: g.* after the gradient-only entry points, else m / 0.1f (m = 0 before the update)."""
     if grads:
-        return read_net(eng, tag, n_lin, prefix="g.")
-    m = read_net(eng, tag, n_lin, prefix="m.")
+        return read_net(eng, tag, n_lin, prefix="g.", agent=agent)
+    m = read_net(eng, tag, n_lin, prefix="m.", agent=agent)
     return {k: v / F32(0.1) for k, v in m.items()}
 
 
-def _check_adam(eng, tag, n_lin, before, v_before, step, lr, grads, worst):
+def _check_adam(eng, tag, n_lin, before, v_before, step, lr, grads, worst, agent=0):
     """float32 torch Adam (m = 0 before the step) on the recovered gradient reproduces the new parameters and v."""
     from oracle.sac_numpy import AdamState
     names = list(before.keys())
     params = [before[nm].copy() for nm in names]
     st = AdamState(lr, [np.zeros_like(p) for p in params], [v_before[nm].copy() for nm in names], step=step)
     st.apply(params, [grads[nm] for nm in names])
-    got, got_v = read_net(eng, tag, n_lin), read_net(eng, tag, n_lin, prefix="v.")
+    got, got_v = read_net(eng, tag, n_lin, agent=agent), read_net(eng, tag, n_lin, prefix="v.", agent=agent)
     for i, nm in enumerate(names):
         _bar(f"{tag} adam param", rel_l2(got[nm], params[i]), 2e-6, worst)
         _bar(f"{tag} adam v", rel_l2(got_v[nm], st.v[i]), 2e-6, worst)
@@ -225,15 +232,27 @@ def per_slots(pushes, cap, n):
     return P.logical_to_slot(np.arange(n), pushes, cap)
 
 
-def _state(eng, c):
+def hyper(eng, agent=0):
+    """The agent's hyper-parameters as the kernels read them from its scalar block: gamma as float32 (sac_target), the
+    learning rates of pi / q1 / q2 and the temperature's as python doubles, where a value <= 0 means the config's
+    (op_prologue: lr[o] > 0 ? lr[o] : Hyper.lr[o]; final_tail: the same for alpha_lr, whose sign < 0 freezes the temperature)."""
+    cfg_lr = (eng.cfg.actor_lr, eng.cfg.critic_lr, eng.cfg.critic_lr)
+    lr = [float(v) if v > 0 else float(cfg_lr[o]) for o, v in enumerate(_np(eng.view("scal.lr", agent)).ravel())]
+    alr = float(eng.view("scal.alpha_lr", agent).item())
+    return {"gamma": float(F32(eng.view("scal.gamma", agent).item())), "lr": lr, "alpha_frozen": alr < 0,
+            "alpha_lr": alr if alr > 0 else float(eng.cfg.alpha_lr)}
+
+
+def _state(eng, c, agent=0):
     nq, npi = len(c["hq"]) + 1, len(c["hp"]) + 1
-    st = {tag: read_net(eng, tag, n) for tag, n in (("pi", npi), ("q1", nq), ("q2", nq), ("q1t", nq), ("q2t", nq))}
-    st["v"] = {tag: read_net(eng, tag, n, prefix="v.") for tag, n in (("pi", npi), ("q1", nq), ("q2", nq))}
-    st["step"] = _np(eng.view("scal.step")).tolist()
-    st["log_alpha"] = float(eng.view("scal.log_alpha").item())
-    st["alpha_m"], st["alpha_v"] = float(eng.view("scal.alpha_m").item()), float(eng.view("scal.alpha_v").item())
-    st["alpha_f32"] = float(eng.view("scal.alpha_f32").item())
-    st["updates"] = int(eng.view("scal.updates").item())
+    st = {tag: read_net(eng, tag, n, agent=agent) for tag, n in (("pi", npi), ("q1", nq), ("q2", nq), ("q1t", nq), ("q2t", nq))}
+    st["v"] = {tag: read_net(eng, tag, n, prefix="v.", agent=agent) for tag, n in (("pi", npi), ("q1", nq), ("q2", nq))}
+    st["step"] = _np(eng.view("scal.step", agent)).tolist()
+    st["log_alpha"] = float(eng.view("scal.log_alpha", agent).item())
+    st["alpha_m"], st["alpha_v"] = float(eng.view("scal.alpha_m", agent).item()), float(eng.view("scal.alpha_v", agent).item())
+    st["alpha_f32"] = float(eng.view("scal.alpha_f32", agent).item())
+    st["updates"] = int(eng.view("scal.updates", agent).item())
+    st["hyper"] = hyper(eng, agent)
     return st
 
 
@@ -251,73 +270,94 @@ def _pre_flags(st, c, ring):
 
 
 # ---------------------------------------------------------------------------------------------------------------- one update
-def one_update(eng, c, ring, rng, worst, grads=False):
-    from oracle import device_rng
-    from oracle.sac_numpy import squash_sample
-    O, A, B = c["obs"], c["act"], c["B"]
-    nq, npi = len(c["hq"]) + 1, len(c["hp"]) + 1
-    st = _state(eng, c)
-    pre = _pre_flags(st, c, ring)
-    n_ring = len(ring[0])
+def prepare(eng, c, ring, rng, agent=0, grads=False):
+    """Before a launch: `agent`'s state, its ring rows on a discontinuity, and the batch the host draws off them (indices into
+    the agent's logical ring positions, normals); prioritized replay: the loaded leaves with every flagged row at p = 0."""
+    B, A = c["B"], c["act"]
+    u = {"st": _state(eng, c, agent)}
+    u["pre"] = pre = _pre_flags(u["st"], c, ring)
+    u["idx"] = u["e1"] = u["e2"] = None
     per = c.get("per")
     if per:
         # the tree draws the batch: every ring row on a discontinuity gets p = 0, which the walk never takes
-        from oracle import per_numpy as P
-        assert not grads and not c["device_rng"]
+        assert not grads and not c["device_rng"] and agent == 0
         buf = eng.per
-        cap, pushes = buf.capacity, int(buf._lib.sacx_ring_pushes(buf.handle, 0))
-        leaves, pmax = buf.slot_priorities()                 # applies the previous update's write-back
-        leaves = leaves.cpu().numpy()
-        leaves[per_slots(pushes, cap, n_ring)[pre]] = 0
+        u["cap"], u["pushes"] = cap, pushes = buf.capacity, int(buf._lib.sacx_ring_pushes(buf.handle, 0))
+        leaves, u["pmax"] = buf.slot_priorities()           # applies the previous update's write-back
+        u["leaves"] = leaves = leaves.cpu().numpy()
+        leaves[per_slots(pushes, cap, len(ring[0]))[pre]] = 0
         assert (leaves > 0).any()
-        buf.load_slot_priorities(torch.as_tensor(leaves), pmax)
-        e1 = rng.standard_normal((B, A)).astype(F32)
-        e2 = rng.standard_normal((B, A)).astype(F32)
+        buf.load_slot_priorities(torch.as_tensor(leaves), u["pmax"])
     elif c["device_rng"]:
         assert not grads
-        idx = None
+        return u
     else:
         good = np.flatnonzero(~pre)
         assert len(good) >= B
-        idx = rng.choice(good, B, replace=False).astype(np.int64)
-        e1 = rng.standard_normal((B, A)).astype(F32)
-        e2 = rng.standard_normal((B, A)).astype(F32)
+        u["idx"] = rng.choice(good, B, replace=False).astype(np.int64)
+    u["e1"] = rng.standard_normal((B, A)).astype(F32)
+    u["e2"] = rng.standard_normal((B, A)).astype(F32)
+    return u
+
+
+def one_update(eng, c, ring, rng, worst, grads=False):
+    """One update of a single-agent engine (prepare, poison, launch, check)."""
+    u = prepare(eng, c, ring, rng, grads=grads)
     _poison(eng)
-    eng.view("block.g").fill_(float("nan"))          # fused: must stay NaN; gradient-only: every element must be written
+    dev = lambda x: torch.as_tensor(x).cuda()
     if grads:
-        dev = lambda x: torch.as_tensor(x).cuda()
-        eng.sample_batch(dev(idx))
-        eng.target(dev(e1))
+        eng.sample_batch(dev(u["idx"]))
+        eng.target(dev(u["e1"]))
         eng.critic_step(None, grads_only=True)
-        eng.actor_step(dev(e2), None, grads_only=True)
+        eng.actor_step(dev(u["e2"]), None, grads_only=True)
         eng.sync()
         m = eng.metrics()
-        assert m["nonfinite"] == 0 and m["updates"] == st["updates"]
     elif c["device_rng"]:
         eng.update(None, None, None, 1)
         eng.sync()
         m = eng.metrics()
-        idx = _np(eng.view("batch.idx")).ravel()
-        seed = int(eng.view("scal.rng_seed").item())
-        agent = int(eng.view("scal.rng_agent").view(torch.int32).item())
-        want = device_rng.feistel_indices(B, n_ring, seed, st["updates"], agent)
+    elif c.get("per"):
+        eng.update(None, dev(u["e1"]), dev(u["e2"]), 1)
+        eng.sync()
+        m = eng.metrics()
+    else:
+        m = eng.update_host(u["idx"], u["e1"], u["e2"], 1)
+    return check_update(eng, c, ring, u, m, worst, grads=grads)
+
+
+def check_update(eng, c, ring, u, m, worst, grads=False, agent=0):
+    """After the launch: `agent`'s update against the float64 oracle on its pre-launch state `u` (prepare); m its metrics."""
+    from oracle import device_rng
+    from oracle.sac_numpy import squash_sample
+    O, A, B = c["obs"], c["act"], c["B"]
+    nq, npi = len(c["hq"]) + 1, len(c["hp"]) + 1
+    st, pre, idx, e1, e2 = u["st"], u["pre"], u["idx"], u["e1"], u["e2"]
+    hy = st["hyper"]
+    n_ring = len(ring[0])
+    per = c.get("per")
+    if grads:
+        assert m["nonfinite"] == 0 and m["updates"] == st["updates"]
+    elif c["device_rng"]:
+        idx = _np(eng.view("batch.idx", agent)).ravel()
+        seed = int(eng.view("scal.rng_seed", agent).item())
+        rng_agent = int(eng.view("scal.rng_agent", agent).view(torch.int32).item())
+        want = device_rng.feistel_indices(B, n_ring, seed, st["updates"], rng_agent)
         assert np.array_equal(idx, want), "device index stream != feistel_index"
-        e1, e2 = _np(eng.view("batch.eps1")), _np(eng.view("batch.eps2"))
+        e1, e2 = _np(eng.view("batch.eps1", agent)), _np(eng.view("batch.eps2", agent))
         for which, e in ((1, e1), (2, e2)):
-            ref = np.array([[device_rng.philox_normal(seed, st["updates"], which, row, j, agent) for j in range(A)] for row in range(B)])
+            ref = np.array([[device_rng.philox_normal(seed, st["updates"], which, row, j, rng_agent) for j in range(A)]
+                            for row in range(B)])
             ulps = np.abs(e - ref) / (np.spacing(F32(1)) * np.maximum(1.0, np.abs(ref)))
             worst["eps (float32 ulps of max(1,|x|))"] = max(worst.get("eps (float32 ulps of max(1,|x|))", 0.0), float(ulps.max()))
             assert ulps.max() <= 4, f"eps{which}: {ulps.max():.1f} ulps from philox_normal"
         assert not pre[idx].any(), f"device batch meets {int(pre[idx].sum())} rows on a discontinuity: pick another seed"
     elif per:
-        dev = lambda x: torch.as_tensor(x).cuda()
-        eng.update(None, dev(e1), dev(e2), 1)
-        eng.sync()
-        m = eng.metrics()
+        from oracle import per_numpy as P
+        leaves, cap, pushes = u["leaves"], u["cap"], u["pushes"]
         idx = _np(eng.view("batch.idx")).ravel()
         seed = int(eng.view("scal.rng_seed").item())
-        agent = int(eng.view("scal.rng_agent").view(torch.int32).item())
-        slots = P.walk_f32(P.tree_f32(leaves), device_rng.per_uniforms(seed, st["updates"], B, agent))
+        rng_agent = int(eng.view("scal.rng_agent").view(torch.int32).item())
+        slots = P.walk_f32(P.tree_f32(leaves), device_rng.per_uniforms(seed, st["updates"], B, rng_agent))
         oldest = pushes % cap if pushes > cap else 0
         assert np.array_equal(idx, (slots - oldest) % cap), \
             f"{int((idx != (slots - oldest) % cap).sum())} of {B} sampled slots differ from walk_f32"
@@ -328,20 +368,18 @@ def one_update(eng, c, ring, rng, worst, grads=False):
         n_dup = B - len(np.unique(slots))
         print(f"    per: t {st['updates']} beta {beta:.6f} w in [{w.min():.3g}, {w.max():.3g}]; duplicate rows {n_dup}; "
               f"zero-priority (flagged) ring rows {int(pre.sum())}")
-    else:
-        m = eng.update_host(idx, e1, e2, 1)
     if not grads:
         assert m["nonfinite"] == 0 and m["updates"] == st["updates"] + 1
-        assert torch.isnan(eng.view("block.g")).all(), "the fused update stored gradients in g.*"
+        assert torch.isnan(eng.view("block.g", agent)).all(), "the fused update stored gradients in g.*"
     s, a, r, s2, d = (x[idx] for x in ring)
 
     # ---- gather: bits
-    sa = _np(eng.view("batch.sa"))
+    sa = _np(eng.view("batch.sa", agent))
     assert np.array_equal(sa, np.concatenate([s, a], axis=1)), "batch.sa"
-    s2a = _np(eng.view("batch.s2a"))
+    s2a = _np(eng.view("batch.s2a", agent))
     assert np.array_equal(s2a[:, :O], s2), "batch.s2a[:, :O]"
-    assert np.array_equal(_np(eng.view("batch.r")).ravel(), r) and np.array_equal(_np(eng.view("batch.d")).ravel(), d)
-    assert np.array_equal(_np(eng.view("batch.idx")).ravel(), idx)
+    assert np.array_equal(_np(eng.view("batch.r", agent)).ravel(), r) and np.array_equal(_np(eng.view("batch.d", agent)).ravel(), d)
+    assert np.array_equal(_np(eng.view("batch.idx", agent)).ravel(), idx)
 
     # ---- target, float64 on the pre-update state
     f64 = lambda x: np.asarray(x, np.float64)
@@ -352,9 +390,9 @@ def one_update(eng, c, ring, rng, worst, grads=False):
     a2, lp2, _ = squash_sample(head2, f64(e1), c["lo"], c["hi"], c["scale"])
     x2 = np.concatenate([f64(s2), a2], axis=1)
     tq1, tq2 = q1t.forward(x2)[0][:, 0], q2t.forward(x2)[0][:, 0]
-    y = f64(r) + 0.99 * (1 - f64(d)) * (np.minimum(tq1, tq2) - alpha * lp2)
-    for name, got, ref in (("a'", s2a[:, O:], a2), ("logpi_next", eng.view("out.logpi_next"), lp2), ("tq1", eng.view("out.tq1"), tq1),
-                           ("tq2", eng.view("out.tq2"), tq2), ("y", eng.view("out.y"), y)):
+    y = f64(r) + hy["gamma"] * (1 - f64(d)) * (np.minimum(tq1, tq2) - alpha * lp2)
+    for name, got, ref in (("a'", s2a[:, O:], a2), ("logpi_next", eng.view("out.logpi_next", agent), lp2), ("tq1", eng.view("out.tq1", agent), tq1),
+                           ("tq2", eng.view("out.tq2", agent), tq2), ("y", eng.view("out.y", agent), y)):
         _bar(name, rel_l2(got if isinstance(got, np.ndarray) else _np(got), ref), 2e-5, worst)
 
     # ---- critics
@@ -366,33 +404,33 @@ def one_update(eng, c, ring, rng, worst, grads=False):
         qv, cache = q.forward(x)
         diff = qv[:, 0] - y
         _, cache, deltas, _ = oracle_forward_backward(q, x, (2 * wt * diff / B)[:, None])
-        _bar("q", rel_l2(_np(eng.view(f"out.q{cc}")), qv[:, 0]), 2e-5, worst)
-        _bar("dout", rel_l2(_np(eng.view(f"scr.dout{cc}"))[:, 0], deltas[-1][:, 0]), 2e-5, worst)
-        _bar("q loss rows", rel_l2(_np(eng.view(f"scr.lossrow{cc}")), wt * diff * diff), 2e-5, worst)
+        _bar("q", rel_l2(_np(eng.view(f"out.q{cc}", agent)), qv[:, 0]), 2e-5, worst)
+        _bar("dout", rel_l2(_np(eng.view(f"scr.dout{cc}", agent))[:, 0], deltas[-1][:, 0]), 2e-5, worst)
+        _bar("q loss rows", rel_l2(_np(eng.view(f"scr.lossrow{cc}", agent)), wt * diff * diff), 2e-5, worst)
         if not grads:
             ql = np.mean(wt * diff * diff)
             _bar("q loss", abs(m[f"q{cc}_loss"] - ql) / ql, 2e-5, worst)
-        g = _engine_grads(eng, tag, nq, grads)
+        g = _engine_grads(eng, tag, nq, grads, agent)
         ref = q.backward(cache, (2 * wt * diff / B)[:, None])
         no = np.zeros(B, bool)
         _check_grads(tag, [g[f"net.{2 * l}.weight"] for l in range(nq)], [g[f"net.{2 * l}.bias"] for l in range(nq)], ref[0], ref[1],
                      deltas, cache["h"][:nq], deltas, cache["h"][:nq], no, worst)
         if not grads:
-            _check_adam(eng, tag, nq, st[tag], st["v"][tag], st["step"][cc], 3e-4, g, worst)
+            _check_adam(eng, tag, nq, st[tag], st["v"][tag], st["step"][cc], hy["lr"][cc], g, worst, agent)
 
     # ---- Polyak: bits, from the engine's post-step critics
     if not grads:
-        tau, omt = (F32(v) for v in _np(eng.view("scal.tau")).ravel())
+        tau, omt = (F32(v) for v in _np(eng.view("scal.tau", agent)).ravel())
         for tag in ("q1", "q2"):
-            new, tnew = read_net(eng, tag, nq), read_net(eng, tag + "t", nq)
+            new, tnew = read_net(eng, tag, nq, agent=agent), read_net(eng, tag + "t", nq, agent=agent)
             for nm in new:
                 assert np.array_equal(tnew[nm], tau * new[nm] + omt * st[tag + "t"][nm]), f"polyak {tag}t.{nm}"
     if c["ties"]:
-        for nm, v in read_net(eng, "q1", nq).items():
-            assert np.array_equal(v, read_net(eng, "q2", nq)[nm]), "tied critics diverged"
+        for nm, v in read_net(eng, "q1", nq, agent=agent).items():
+            assert np.array_equal(v, read_net(eng, "q2", nq, agent=agent)[nm]), "tied critics diverged"
 
     # ---- actor: post-step critics (read exactly; unchanged by the gradient-only calls), pre-update policy and alpha
-    post = {tag: _mlp(read_net(eng, tag, nq), c["actfn"], c["out_act"]) for tag in ("q1", "q2")}
+    post = {tag: _mlp(read_net(eng, tag, nq, agent=agent), c["actfn"], c["out_act"]) for tag in ("q1", "q2")}
     head, pcache = pi0.forward(f64(s))
     act_, lp, aux = squash_sample(head, f64(e2), c["lo"], c["hi"], c["scale"])
     xa = np.concatenate([f64(s), act_], axis=1)
@@ -412,49 +450,49 @@ def one_update(eng, c, ring, rng, worst, grads=False):
     d_head = np.concatenate([dz, (se * dz - alpha / B) * mask], axis=1)
     _, pcache, pdeltas, _ = oracle_forward_backward(pi0, f64(s), d_head)
     keep = ~flags
-    spi = _np(eng.view("batch.spi"))
+    spi = _np(eng.view("batch.spi", agent))
     assert np.array_equal(spi[:, :O], s)
     _bar("a~", rel_l2(spi[:, O:], act_), 2e-5, worst)
-    _bar("logpi", rel_l2(_np(eng.view("out.logpi")), lp), 2e-5, worst)
-    q1_pi, q2_pi = _np(eng.view("out.q1_pi")).ravel(), _np(eng.view("out.q2_pi")).ravel()
+    _bar("logpi", rel_l2(_np(eng.view("out.logpi", agent)), lp), 2e-5, worst)
+    q1_pi, q2_pi = _np(eng.view("out.q1_pi", agent)).ravel(), _np(eng.view("out.q2_pi", agent)).ravel()
     _bar("q_pi", max(rel_l2(q1_pi, qa[0]), rel_l2(q2_pi, qa[1])), 2e-5, worst)
     if c["ties"]:
         assert np.array_equal(q1_pi, q2_pi) and (qa[0] == qa[1]).all()
-    dhead = _np(eng.view("scr.dhead"))
+    dhead = _np(eng.view("scr.dhead", agent))
     _bar("dhead (unflagged rows)", rel_l2(dhead[keep], pdeltas[-1][keep]), 2e-5, worst)
-    g_deltas = [_np(eng.view(f"delta.pi.{l}")) for l in range(npi - 1)] + [dhead]
-    g_inputs = [spi[:, :O]] + [_np(eng.view(f"act.pia.h{l}")) for l in range(npi - 1)]
+    g_deltas = [_np(eng.view(f"delta.pi.{l}", agent)) for l in range(npi - 1)] + [dhead]
+    g_inputs = [spi[:, :O]] + [_np(eng.view(f"act.pia.h{l}", agent)) for l in range(npi - 1)]
     for l in range(npi - 1):
         _bar("delta.pi (unflagged rows)", rel_l2(g_deltas[l][keep], pdeltas[l][keep]), 2e-5, worst)
     prow = alpha * lp - np.minimum(qa[0], qa[1])
-    _bar("policy loss rows", rel_l2(_np(eng.view("scr.plossrow")), prow), 2e-5, worst)
+    _bar("policy loss rows", rel_l2(_np(eng.view("scr.plossrow", agent)), prow), 2e-5, worst)
     if not grads:
         # a mean of signed rows: relative to the mean of their magnitudes, which is what rounding of the rows adds up to
         _bar("policy loss (of mean |row|)", abs(m["policy_loss"] - prow.mean()) / np.abs(prow).mean(), 2e-5, worst)
-    g = _engine_grads(eng, "pi", npi, grads)
+    g = _engine_grads(eng, "pi", npi, grads, agent)
     ref = pi0.backward(pcache, d_head)
     _check_grads("pi", [g[f"net.{2 * l}.weight"] for l in range(npi)], [g[f"net.{2 * l}.bias"] for l in range(npi)], ref[0], ref[1],
                  g_deltas, g_inputs, pdeltas, pcache["h"][:npi], flags, worst)
     if grads:
         return int(pre.sum()), int(flags.sum())
-    _check_adam(eng, "pi", npi, st["pi"], st["v"]["pi"], st["step"][0], 3e-4, g, worst)
+    _check_adam(eng, "pi", npi, st["pi"], st["v"]["pi"], st["step"][0], hy["lr"][0], g, worst, agent)
     if per:
-        _check_write_back(eng, per, slots, leaves, pmax, worst)
+        _check_write_back(eng, per, slots, leaves, u["pmax"], worst)
 
     # ---- temperature
-    la = float(eng.view("scal.log_alpha").item())
-    if c["auto"]:
-        lp_e = f64(_np(eng.view("out.logpi")).ravel())
+    la = float(eng.view("scal.log_alpha", agent).item())
+    if c["auto"] and not hy["alpha_frozen"]:
+        lp_e = f64(_np(eng.view("out.logpi", agent)).ravel())
         grad = -np.mean(lp_e - A)
         tt = st["step"][3] + 1
         am = st["alpha_m"] + 0.1 * (grad - st["alpha_m"])
         av = st["alpha_v"] * 0.999 + 0.001 * grad * grad
-        la_ref = st["log_alpha"] - (3e-4 / (1 - 0.9 ** tt)) * (am / (np.sqrt(av) / np.sqrt(1 - 0.999 ** tt) + 1e-8))
+        la_ref = st["log_alpha"] - (hy["alpha_lr"] / (1 - 0.9 ** tt)) * (am / (np.sqrt(av) / np.sqrt(1 - 0.999 ** tt) + 1e-8))
         _bar("log_alpha (abs)", abs(la - la_ref), 1e-6, worst)
-        _bar("alpha_m (abs)", abs(float(eng.view("scal.alpha_m").item()) - am), 1e-6, worst)
-        _bar("alpha_v (rel)", abs(float(eng.view("scal.alpha_v").item()) - av) / av, 2e-6, worst)
+        _bar("alpha_m (abs)", abs(float(eng.view("scal.alpha_m", agent).item()) - am), 1e-6, worst)
+        _bar("alpha_v (rel)", abs(float(eng.view("scal.alpha_v", agent).item()) - av) / av, 2e-6, worst)
     else:
-        assert la == st["log_alpha"], "fixed temperature: log_alpha moved"
+        assert la == st["log_alpha"], "fixed or frozen temperature: log_alpha moved"
     return int(pre.sum()), int(flags.sum())
 
 
