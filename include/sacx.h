@@ -297,6 +297,41 @@ int sacx_per_load_priorities(sacx_per_t per, const float* leaves_dev, float p_ma
  * per-phase entry points (sacx_critic_step, ...) stay unweighted. */
 int sacx_agent_attach_per(sacx_agent_t h, sacx_per_t per);
 
+/* ---------------------------------------------------------------- population-based training (Jaderberg et al., 2017)
+ * Learner-state copy between agents of a population ("exploit"), optionally followed by new hyper-parameters ("explore").
+ * Copied: online parameters, Adam m and v, target critics, and from the scalar block log_alpha, alpha_m, alpha_v, alpha,
+ * alpha_f32, the Adam step counters and bias corrections, the learning rates, gamma, tau, 1 - tau. Kept from the destination:
+ * the update counter and the RNG keys (its device streams stay its own), metrics, the non-finite flag, the data-parallel
+ * shares, and its replay ring. Each call is one kernel on the agent's stream (behind any queued update); nothing synchronises.
+ * Validated before any device work (SACX_ERR_INVALID): agent ids and slots in range, no repeated destination, no destination
+ * that is also a source of the same call (every copy reads the state from before the call; a source may feed several
+ * destinations), record values positive and finite (tau in (0, 1]), no temperature record with auto_entropy_tuning. */
+#define SACX_PBT_ALPHA      1    /* log_alpha, alpha, alpha_f32 (fixed temperature only)  */
+#define SACX_PBT_ALPHA_LR   2
+#define SACX_PBT_ACTOR_LR   4    /* lr[0]                                                 */
+#define SACX_PBT_CRITIC_LR  8    /* lr[1] and lr[2]                                       */
+#define SACX_PBT_TAU       16    /* tau and one_minus_tau                                 */
+#define SACX_PBT_GAMMA     32
+/* new hyper-parameters of one destination, as the final field values (the caller applies the config's roundings) */
+typedef struct sacx_pbt_record {
+  uint32_t set;                  /* SACX_PBT_* bits of the fields written; 0 = no record */
+  uint32_t reserved;
+  double   log_alpha, alpha;
+  double   alpha_lr, actor_lr, critic_lr;
+  float    alpha_f32, gamma, tau, one_minus_tau;
+} sacx_pbt_record;
+int     sacx_sizeof_pbt_record(void);
+/* float32 words of one packed learner state (a slot of the pack / unpack buffers; 16-byte multiple) */
+int64_t sacx_pbt_state_floats(sacx_agent_t h);
+/* agent dst[i] <- agent src[i] (local ids), then records[i] (records nullable) */
+int sacx_pbt_copy(sacx_agent_t h, const int32_t* src_host, const int32_t* dst_host, int32_t n_pairs,
+                  const sacx_pbt_record* records_host /* nullable */);
+/* slot k of buf_dev [n, sacx_pbt_state_floats] <- agent agents[k] */
+int sacx_pbt_pack(sacx_agent_t h, const int32_t* agents_host, int32_t n, float* buf_dev);
+/* agent dst[i] <- slot slots[i] of buf_dev [n_slots, sacx_pbt_state_floats], then records[i] (records nullable) */
+int sacx_pbt_unpack(sacx_agent_t h, const float* buf_dev, int32_t n_slots, const int32_t* slots_host, const int32_t* dst_host,
+                    int32_t n, const sacx_pbt_record* records_host /* nullable */);
+
 #ifdef __cplusplus
 }
 #endif

@@ -11,6 +11,7 @@
 #include <vector>
 
 #include "sacx_engine.cuh"
+#include "sacx_pbt.cuh"
 #include "sacx_per.cuh"
 
 namespace sacx {
@@ -632,6 +633,92 @@ static int validate(const sacx_config* c) {
   return SACX_OK;
 }
 
+// ------------------------------------------------------------------------------------------ population-based training
+// span 0 starts with the scalar block and runs through Adam v; span 1 holds the target critics (sacx_pbt.cuh)
+static i64 pbt_span0(const Engine& e) { return e.P0 + 3 * e.blk - e.scal_off; }
+static i64 pbt_span1(const Engine& e) { return align4(e.n_critic); }
+static PbtEnd pbt_arena(const Engine& e) { return PbtEnd{e.arena, e.stride, e.scal_off, e.T0}; }
+static PbtEnd pbt_buffer(const Engine& e, const float* buf) {
+  return PbtEnd{const_cast<float*>(buf), pbt_span0(e) + pbt_span1(e), 0, pbt_span0(e)};
+}
+
+static int pbt_check_agents(const Engine& e, const int32_t* ids, int n, const char* what) {
+  for (int i = 0; i < n; ++i)
+    if (ids[i] < 0 || ids[i] >= e.cfg.n_agents)
+      return fail(SACX_ERR_INVALID, std::string("pbt: ") + what + " agent " + std::to_string(ids[i]) + " out of range [0, " +
+                                        std::to_string(e.cfg.n_agents) + ")");
+  return SACX_OK;
+}
+
+static int pbt_check_destinations(const Engine& e, const int32_t* dst, int n, const int32_t* src /* nullable */) {
+  std::vector<char> is_dst((size_t)e.cfg.n_agents, 0);
+  for (int i = 0; i < n; ++i) {
+    if (is_dst[dst[i]]) return fail(SACX_ERR_INVALID, "pbt: agent " + std::to_string(dst[i]) + " is a destination twice");
+    is_dst[dst[i]] = 1;
+  }
+  if (src)
+    for (int i = 0; i < n; ++i)
+      if (is_dst[src[i]])
+        return fail(SACX_ERR_INVALID, "pbt: agent " + std::to_string(src[i]) + " is both a source and a destination");
+  return SACX_OK;
+}
+
+static int pbt_check_record(const Engine& e, const sacx_pbt_record& r) {
+  const unsigned all = SACX_PBT_ALPHA | SACX_PBT_ALPHA_LR | SACX_PBT_ACTOR_LR | SACX_PBT_CRITIC_LR | SACX_PBT_TAU | SACX_PBT_GAMMA;
+  auto pos = [](double x) { return x > 0.0 && std::isfinite(x); };
+  if (r.set & ~all) return fail(SACX_ERR_INVALID, "pbt: unknown record bits");
+  if (r.set & SACX_PBT_ALPHA) {
+    if (e.cfg.auto_entropy_tuning)
+      return fail(SACX_ERR_INVALID, "pbt: with auto_entropy_tuning the temperature is learner state; a record cannot set it");
+    if (!pos(r.alpha) || !pos(r.alpha_f32) || !std::isfinite(r.log_alpha)) return fail(SACX_ERR_INVALID, "pbt: alpha must be positive and finite");
+  }
+  if ((r.set & SACX_PBT_ALPHA_LR) && !pos(r.alpha_lr)) return fail(SACX_ERR_INVALID, "pbt: alpha_lr must be positive and finite");
+  if ((r.set & SACX_PBT_ACTOR_LR) && !pos(r.actor_lr)) return fail(SACX_ERR_INVALID, "pbt: actor_lr must be positive and finite");
+  if ((r.set & SACX_PBT_CRITIC_LR) && !pos(r.critic_lr)) return fail(SACX_ERR_INVALID, "pbt: critic_lr must be positive and finite");
+  if ((r.set & SACX_PBT_TAU) && !(pos(r.tau) && r.tau <= 1.f && r.one_minus_tau >= 0.f && r.one_minus_tau <= 1.f))
+    return fail(SACX_ERR_INVALID, "pbt: tau must be in (0, 1]");
+  if ((r.set & SACX_PBT_GAMMA) && !pos(r.gamma)) return fail(SACX_ERR_INVALID, "pbt: gamma must be positive and finite");
+  return SACX_OK;
+}
+
+// validated pairs -> one pbt_copy_kernel launch on the agent's stream (the pair list goes up through a pinned block)
+static int pbt_launch(Engine& e, const PbtEnd& src, const PbtEnd& dst, bool dst_arena, const int32_t* s, const int32_t* d, int n,
+                      const sacx_pbt_record* rec) {
+  if (n == 0) return SACX_OK;
+  if (e.P0 != e.scal_off + SCAL_WORDS || ((uintptr_t)e.arena & 15))
+    return fail(SACX_ERR_INVALID, "pbt: the arena does not hold the learner state as two 16-byte aligned spans");
+  if (rec)
+    for (int i = 0; i < n; ++i) {
+      int rc = pbt_check_record(e, rec[i]);
+      if (rc) return rc;
+    }
+  const size_t bytes = (size_t)n * sizeof(PbtPair);
+  if (!e.pbt_copied) SACX_CUDA(cudaEventCreateWithFlags(&e.pbt_copied, cudaEventDisableTiming));
+  SACX_CUDA(cudaEventSynchronize(e.pbt_copied));         // the previous pair list has left the pinned block
+  if (bytes > e.pbt_bytes) {
+    if (e.pbt_pinned) { cudaFreeHost(e.pbt_pinned); e.pbt_pinned = nullptr; }
+    if (e.pbt_dev) { SACX_CUDA(cudaStreamSynchronize(e.stream)); cudaFree(e.pbt_dev); e.pbt_dev = nullptr; }
+    e.pbt_bytes = 0;
+    SACX_CUDA(cudaMallocHost(&e.pbt_pinned, bytes));
+    SACX_CUDA(cudaMalloc(&e.pbt_dev, bytes));
+    e.pbt_bytes = bytes;
+  }
+  PbtPair* p = static_cast<PbtPair*>(e.pbt_pinned);
+  for (int i = 0; i < n; ++i) {
+    memset(&p[i], 0, sizeof p[i]);
+    p[i].src = s[i]; p[i].dst = d[i];
+    if (rec) p[i].rec = rec[i];
+  }
+  SACX_CUDA(cudaMemcpyAsync(e.pbt_dev, e.pbt_pinned, bytes, cudaMemcpyHostToDevice, e.stream));
+  SACX_CUDA(cudaEventRecord(e.pbt_copied, e.stream));
+  const i64 n0 = pbt_span0(e) / 4, n1 = pbt_span1(e) / 4;
+  const dim3 grid((unsigned)((n0 + n1 + PBT_CHUNK - 1) / PBT_CHUNK), (unsigned)std::min(n, 65535));
+  pbt_copy_kernel<<<grid, PBT_THREADS, 0, e.stream>>>(src, dst, n0, n1, dst_arena ? 1 : 0, static_cast<const PbtPair*>(e.pbt_dev), n);
+  ++e.launches;
+  SACX_CUDA(cudaGetLastError());
+  return SACX_OK;
+}
+
 }  // namespace sacx
 
 using namespace sacx;
@@ -1080,6 +1167,9 @@ int sacx_agent_destroy(sacx_agent_t h) {
     if (io.pinned) cudaFreeHost(io.pinned); if (io.dev) cudaFree(io.dev); if (io.done) cudaEventDestroy(io.done); if (io.copied) cudaEventDestroy(io.copied);
   }
   if (e.copy_stream) cudaStreamDestroy(e.copy_stream);
+  if (e.pbt_pinned) cudaFreeHost(e.pbt_pinned);
+  if (e.pbt_dev) cudaFree(e.pbt_dev);
+  if (e.pbt_copied) cudaEventDestroy(e.pbt_copied);
   delete h;
   return SACX_OK;
 }
@@ -1567,6 +1657,45 @@ int sacx_sync(sacx_agent_t h) {
 }
 
 int64_t sacx_launch_count(sacx_agent_t h) { return h ? h->e.launches + (h->e.ring ? h->e.ring->launches : 0) : 0; }
+
+// ---------------------------------------------------------------------------------------- population-based training
+int sacx_sizeof_pbt_record(void) { return (int)sizeof(sacx_pbt_record); }
+
+int64_t sacx_pbt_state_floats(sacx_agent_t h) { return h ? pbt_span0(h->e) + pbt_span1(h->e) : 0; }
+
+int sacx_pbt_copy(sacx_agent_t h, const int32_t* src, const int32_t* dst, int32_t n, const sacx_pbt_record* rec) {
+  if (!h || n < 0 || (n > 0 && (!src || !dst))) return fail(SACX_ERR_INVALID, "pbt_copy: bad arguments");
+  Engine& e = h->e;
+  int rc;
+  if ((rc = pbt_check_agents(e, src, n, "source")) || (rc = pbt_check_agents(e, dst, n, "destination")) ||
+      (rc = pbt_check_destinations(e, dst, n, src)))
+    return rc;
+  return pbt_launch(e, pbt_arena(e), pbt_arena(e), true, src, dst, n, rec);
+}
+
+int sacx_pbt_pack(sacx_agent_t h, const int32_t* agents, int32_t n, float* buf) {
+  if (!h || n < 0 || (n > 0 && (!agents || !buf))) return fail(SACX_ERR_INVALID, "pbt_pack: bad arguments");
+  if ((uintptr_t)buf & 15) return fail(SACX_ERR_INVALID, "pbt_pack: buffer not 16-byte aligned");
+  Engine& e = h->e;
+  int rc = pbt_check_agents(e, agents, n, "source");
+  if (rc) return rc;
+  std::vector<int32_t> slots((size_t)n);
+  for (int i = 0; i < n; ++i) slots[i] = i;
+  return pbt_launch(e, pbt_arena(e), pbt_buffer(e, buf), false, agents, slots.data(), n, nullptr);
+}
+
+int sacx_pbt_unpack(sacx_agent_t h, const float* buf, int32_t n_slots, const int32_t* slots, const int32_t* dst, int32_t n,
+                    const sacx_pbt_record* rec) {
+  if (!h || n < 0 || n_slots < 0 || (n > 0 && (!buf || !slots || !dst))) return fail(SACX_ERR_INVALID, "pbt_unpack: bad arguments");
+  if ((uintptr_t)buf & 15) return fail(SACX_ERR_INVALID, "pbt_unpack: buffer not 16-byte aligned");
+  Engine& e = h->e;
+  for (int i = 0; i < n; ++i)
+    if (slots[i] < 0 || slots[i] >= n_slots)
+      return fail(SACX_ERR_INVALID, "pbt_unpack: slot " + std::to_string(slots[i]) + " out of range [0, " + std::to_string(n_slots) + ")");
+  int rc;
+  if ((rc = pbt_check_agents(e, dst, n, "destination")) || (rc = pbt_check_destinations(e, dst, n, nullptr))) return rc;
+  return pbt_launch(e, pbt_buffer(e, buf), pbt_arena(e), true, slots, dst, n, rec);
+}
 
 // ---------------------------------------------------------------------------------------- prioritized replay
 int sacx_per_create(sacx_ring_t ring, float alpha, float beta0, int64_t beta_steps, float eps, int32_t max_batch, sacx_per_t* out) {

@@ -84,6 +84,11 @@ struct Engine {
   cudaStream_t stream = 0;
   Ring* ring = nullptr;
   Per* per = nullptr;                     // prioritized replay tree (sacx_agent_attach_per), or null: uniform sampling
+  // population-based training (sacx_pbt.cuh): the pair list of the latest copy, pinned for its H2D copy and on the device
+  void* pbt_pinned = nullptr;
+  void* pbt_dev = nullptr;
+  size_t pbt_bytes = 0;
+  cudaEvent_t pbt_copied = nullptr;       // the latest pair list has left pbt_pinned
   long long launches = 0;
   unsigned long long act_calls = 0;
   Hyper hp;

@@ -62,6 +62,17 @@ class SacxTensorDesc(C.Structure):
                 ("ld", C.c_int32), ("dtype", C.c_int32)]
 
 
+# SACX_PBT_* bits of sacx_pbt_record.set
+PBT_ALPHA, PBT_ALPHA_LR, PBT_ACTOR_LR, PBT_CRITIC_LR, PBT_TAU, PBT_GAMMA = 1, 2, 4, 8, 16, 32
+
+
+class SacxPbtRecord(C.Structure):
+    _fields_ = [("set", C.c_uint32), ("reserved", C.c_uint32),
+                ("log_alpha", C.c_double), ("alpha", C.c_double),
+                ("alpha_lr", C.c_double), ("actor_lr", C.c_double), ("critic_lr", C.c_double),
+                ("alpha_f32", C.c_float), ("gamma", C.c_float), ("tau", C.c_float), ("one_minus_tau", C.c_float)]
+
+
 # every symbol include/sacx.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 _I32, _I64, _U64, _F = C.c_int32, C.c_int64, C.c_uint64, C.c_float
@@ -138,6 +149,11 @@ SYMBOLS = {
     "sacx_sync": (C.c_int, [_P]),
     "sacx_debug_profile": (C.c_int, [_P, _I32, _P, _I64, C.POINTER(_I32), C.POINTER(_I32)]),
     "sacx_launch_count": (_I64, [_P]),
+    "sacx_sizeof_pbt_record": (C.c_int, []),
+    "sacx_pbt_state_floats": (_I64, [_P]),
+    "sacx_pbt_copy": (C.c_int, [_P, _P, _P, _I32, _P]),
+    "sacx_pbt_pack": (C.c_int, [_P, _P, _I32, _P]),
+    "sacx_pbt_unpack": (C.c_int, [_P, _P, _I32, _P, _P, _I32, _P]),
 }
 
 _LIB: Optional[C.CDLL] = None
@@ -164,7 +180,8 @@ def load() -> C.CDLL:
         fn.restype = res
         fn.argtypes = args
     if (lib.sacx_sizeof_config() != C.sizeof(SacxConfig) or lib.sacx_sizeof_metrics() != C.sizeof(SacxMetrics)
-            or lib.sacx_sizeof_tensor_desc() != C.sizeof(SacxTensorDesc)):
+            or lib.sacx_sizeof_tensor_desc() != C.sizeof(SacxTensorDesc)
+            or lib.sacx_sizeof_pbt_record() != C.sizeof(SacxPbtRecord)):
         raise RuntimeError("libsacx.so struct layout differs from the Python binding (stale build?)")
     _LIB = lib
     return lib

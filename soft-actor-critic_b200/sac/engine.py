@@ -240,6 +240,51 @@ class UpdateEngine:
         E.check(self.lib.sacx_q_values_host(self.h, agent, s.ctypes.data, a.ctypes.data, s.shape[0], q1.ctypes.data, q2.ctypes.data))
         return q1, q2
 
+    # ------------------------------------------------------------------ population-based training (include/sacx.h: sacx_pbt_*)
+    def pbt_state_floats(self) -> int:
+        """float32 words of one packed learner state."""
+        return int(self.lib.sacx_pbt_state_floats(self.h))
+
+    @staticmethod
+    def _ids(ids) -> np.ndarray:
+        return np.ascontiguousarray(np.asarray(ids, dtype=np.int64).reshape(-1).astype(np.int32))
+
+    @staticmethod
+    def _records(records, n: int):
+        if records is None:
+            return None
+        if len(records) != n:
+            raise ValueError("one record per pair expected")
+        return (E.SacxPbtRecord * n)(*records)
+
+    def pbt_copy(self, src, dst, records=None) -> None:
+        """Agent dst[i] takes the learner state of agent src[i] (local ids), then records[i]: one launch on the engine's stream."""
+        self._sync_stream()
+        s, d = self._ids(src), self._ids(dst)
+        if len(s) != len(d):
+            raise ValueError("pbt_copy: src and dst differ in length")
+        E.check(self.lib.sacx_pbt_copy(self.h, s.ctypes.data, d.ctypes.data, len(d), self._records(records, len(d))))
+
+    def pbt_pack(self, agents, buf: torch.Tensor) -> None:
+        """buf[k] <- learner state of agent agents[k]; buf a contiguous float32 device tensor [len(agents), pbt_state_floats()]."""
+        self._sync_stream()
+        a = self._ids(agents)
+        if buf.dtype != torch.float32 or not buf.is_contiguous() or buf.numel() < len(a) * self.pbt_state_floats():
+            raise ValueError("pbt_pack: buffer must be a contiguous float32 tensor of len(agents) packed states")
+        E.check(self.lib.sacx_pbt_pack(self.h, a.ctypes.data, len(a), E.ptr(buf)))
+
+    def pbt_unpack(self, buf: torch.Tensor, slots, dst, records=None) -> None:
+        """Agent dst[i] takes the packed state buf[slots[i]], then records[i]."""
+        self._sync_stream()
+        s, d = self._ids(slots), self._ids(dst)
+        if len(s) != len(d):
+            raise ValueError("pbt_unpack: slots and dst differ in length")
+        if buf.dtype != torch.float32 or not buf.is_contiguous():
+            raise ValueError("pbt_unpack: buffer must be a contiguous float32 tensor")
+        n_slots = buf.numel() // max(self.pbt_state_floats(), 1)
+        E.check(self.lib.sacx_pbt_unpack(self.h, E.ptr(buf), n_slots, s.ctypes.data, d.ctypes.data, len(d),
+                                         self._records(records, len(d))))
+
     def metrics(self, agent: int = 0) -> dict:
         self._sync_stream()
         E.check(self.lib.sacx_get_metrics(self.h, agent, C.byref(self._metrics)))

@@ -175,6 +175,40 @@ class SACPopulation:
                 raise KeyError(f"not a per-agent hyper-parameter: {sorted(unknown)} (per-agent: {self.TRIAL_KEYS})")
             self.set_trial(a, **{k: trials[g].get(k) for k in self.TRIAL_KEYS})
 
+    def exploit(self, pairs: Sequence[Tuple[int, int]], hypers: Optional[Sequence[Optional[Dict[str, float]]]] = None) -> None:
+        """Population-based training's exploit (and explore) step: for every (source, destination) pair of GLOBAL agent ids the
+        destination takes over the source's learner state -- parameters, Adam state, targets, temperature and its optimiser,
+        step counters and hyper-parameters -- and keeps its own replay ring, update counter, RNG streams and metrics; then
+        hypers[i] (a dict over a subset of TRIAL_KEYS, or None) is written into pair i's destination with set_trial's
+        roundings. Every copy reads the state from before the call: a destination may not be a source, a source may feed
+        several destinations. Like set_trials, every rank calls it with the same arguments. Pairs within a rank are one
+        launch; pairs across ranks add a pack launch, ONE all_to_all_single on the engine's stream, and an unpack launch. The
+        result does not depend on the sharding."""
+        from .pbt import pbt_record, route_exploit
+        pairs = [(int(s), int(d)) for s, d in pairs]
+        if hypers is not None and len(hypers) != len(pairs):
+            raise ValueError("one hyper-parameter dict (or None) per pair expected")
+        routes = route_exploit(pairs, self.n_agents_global, self.world)
+        rt = routes[self.rank]
+        records = None
+        if hypers is not None:
+            auto = bool(self.config["sac"]["auto_entropy_tuning"])
+            records = [pbt_record(h, auto) for h in hypers]
+        eng = self.engine
+        if rt.copy_dst:
+            eng.pbt_copy(rt.copy_src, rt.copy_dst, None if records is None else [records[i] for i in rt.copy_pair])
+        if not any(r.pack for r in routes):
+            return
+        d = _dist()
+        if d is None or d.get_world_size() != self.world:
+            raise RuntimeError("exploit: pairs across ranks need the torch.distributed process group the population is sharded over")
+        F = eng.pbt_state_floats()
+        send = torch.empty((len(rt.pack), F), dtype=torch.float32, device=eng.device)
+        recv = torch.empty((sum(rt.recv_counts), F), dtype=torch.float32, device=eng.device)
+        eng.pbt_pack(rt.pack, send)
+        d.all_to_all_single(recv, send, output_split_sizes=rt.recv_counts, input_split_sizes=rt.send_counts)
+        eng.pbt_unpack(recv, rt.unpack_slot, rt.unpack_dst, None if records is None else [records[i] for i in rt.unpack_pair])
+
     def act_all(self, states, deterministic: bool = False, eps=None) -> torch.Tensor:
         """One action per local agent from its own observation (vectorised envs): states [n_local, obs] (numpy or tensor) ->
         device tensor [n_local, act]; one kernel launch for the whole population (reference: select_action per agent,

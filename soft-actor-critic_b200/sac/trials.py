@@ -17,12 +17,13 @@ import copy
 import math
 import random as _random
 from collections import deque
-from typing import Any, Callable, Dict, List, Optional, Sequence
+from typing import Any, Callable, Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
 
-from .population import SACPopulation
+from .pbt import PBTConfig, explore, round_rng, select_pairs
+from .population import SACPopulation, _dist
 
 
 def sample_search_space(search_space: Dict[str, Dict[str, dict]], n_trials: int, seed: int = 0) -> List[Dict[str, Any]]:
@@ -58,9 +59,13 @@ def trial_config(base_config: dict, params: Dict[str, Any]) -> dict:
 
 class PopulationTrials:
     def __init__(self, base_config: dict, trials: Sequence[Dict[str, Any]], env_factory: Callable[[], Any], device=None,
-                 rank: Optional[int] = None, world: Optional[int] = None):
+                 rank: Optional[int] = None, world: Optional[int] = None,
+                 search_space: Optional[Dict[str, Dict[str, dict]]] = None):
+        """search_space (run_search.py format) bounds and redraws the values population-based training explores."""
         self.base_config = base_config
+        self.search_space = search_space
         self.trials = [dict(t) for t in trials]
+        self.lineage: List[List[Tuple[int, int, Dict[str, Any]]]] = [[] for _ in self.trials]     # (step, source, values)
         per_agent = []
         for i, t in enumerate(self.trials):
             pa = {}
@@ -85,11 +90,16 @@ class PopulationTrials:
             env.action_space.seed(s)
             env.observation_space.seed(s)
 
-    def run(self, num_episodes: int, out: Callable[[str], None] = print) -> List[Dict[str, float]]:
+    def run(self, num_episodes: int, out: Callable[[str], None] = print, pbt: Optional[PBTConfig] = None) -> List[Dict[str, float]]:
         """run_training_loop (agent.py:329-418) for every trial in lockstep: one environment step per trial per iteration, one
         update launch for all trials once every ring holds train.warming_steps transitions. Prints, per trial, the lines the
         reference driver prints / scrapes; returns the per-trial metrics dicts (total_episodes, best_avg_return,
-        final_avg_return) in global trial order for this rank's trials."""
+        final_avg_return) in global trial order for this rank's trials.
+
+        With a PBTConfig, population-based training: every pbt.interval_steps environment steps one exploit round (see
+        sac/pbt.py) on the mean return of each trial's episodes since its last exploit (at most the last 100). A receiver
+        takes its source's learner state and explored values (trial dict and lineage updated, return window emptied) and
+        continues its environment episode; one line per pair: ``PBT step {t}: trial {dst} <- trial {src} {params}``."""
         pop, tr = self.pop, self.base_config["train"]
         n = pop.n_local
         update_every, grad_steps = tr.get("update_frequency", 1), tr.get("gradient_steps_per_update", 1)
@@ -101,7 +111,11 @@ class PopulationTrials:
         final: List[Optional[Dict[str, float]]] = [None] * n
         total_steps = 0
         obs_dim = pop.obs_dim
-        while any(f is None for f in final):
+        rounds = 0
+        # with ranks, finishing is decided at the exploit rounds (all ranks agree there), so every rank joins every round
+        lockstep = pbt is not None and pop.world > 1
+        running = True
+        while running if lockstep else any(f is None for f in final):
             actions = pop.act_all(np.asarray(states, np.float32).reshape(n, obs_dim)).cpu().numpy()       # one launch, one D2H
             for a, env in enumerate(self.envs):
                 if final[a] is not None:
@@ -127,8 +141,38 @@ class PopulationTrials:
             total_steps += 1
             if total_steps >= warming and total_steps % update_every == 0:
                 pop.update(grad_steps)
+            if pbt is not None and total_steps % pbt.interval_steps == 0:
+                local = [float(np.mean(window[a])) if final[a] is None and len(window[a]) >= pbt.min_episodes else None
+                         for a in range(n)]
+                scores, running = self._gather_scores(local, [f is None for f in final])
+                rng = round_rng(pbt.seed, rounds)
+                pairs = select_pairs(scores, pbt.fraction, rng)
+                rounds += 1
+                if pairs:
+                    values = [explore(self.trials[s], self.search_space, pbt, rng) for s, _ in pairs]
+                    pop.exploit(pairs, [{k.split(".", 1)[1]: v for k, v in vals.items()} for vals in values])
+                    for (s, d), vals in zip(pairs, values):
+                        self.trials[d] = vals
+                        self.lineage[d].append((total_steps, s, dict(vals)))
+                        if d in pop.agent_ids:
+                            window[pop.local_index(d)].clear()
+                        out(f"PBT step {total_steps}: trial {d} <- trial {s} {vals}")
         torch.cuda.synchronize()
         return [f for f in final if f is not None]
+
+    def _gather_scores(self, local: List[Optional[float]], unfinished: List[bool]) -> Tuple[List[Optional[float]], bool]:
+        """Every rank's scores in global trial order, and whether any trial anywhere is unfinished."""
+        pop = self.pop
+        d = _dist()
+        if d is None or pop.world == 1:
+            return list(local), any(unfinished)
+        parts: List[Any] = [None] * pop.world
+        d.all_gather_object(parts, (list(pop.agent_ids), list(local), any(unfinished)))
+        scores: List[Optional[float]] = [None] * pop.n_agents_global
+        for ids, vals, _ in parts:
+            for g, v in zip(ids, vals):
+                scores[g] = v
+        return scores, any(p[2] for p in parts)
 
 
 def run_population_search(base_config: dict, search_space: Dict[str, Dict[str, dict]], n_trials: int,
@@ -150,3 +194,28 @@ def run_population_search(base_config: dict, search_space: Dict[str, Dict[str, d
     for k, v in trials[best].items():
         out(f"    {k}: {v}")
     return {"trials": trials, "metrics": metrics, "best_trial": best, "best_value": values[best]}
+
+
+def run_population_pbt(base_config: dict, search_space: Dict[str, Dict[str, dict]], n_trials: int, env_factory: Callable[[], Any],
+                       pbt: PBTConfig, num_episodes: Optional[int] = None, seed: int = 0,
+                       out: Callable[[str], None] = print) -> Dict[str, Any]:
+    """run_population_search with population-based training: the same initial draws and printed summary; the best trial's
+    "Best Hyperparameters" are the values in force at its end, followed by every trial's lineage."""
+    trials = sample_search_space(search_space, n_trials, seed)
+    runner = PopulationTrials(base_config, trials, env_factory, search_space=search_space)
+    metrics = runner.run(num_episodes or base_config["train"].get("num_episodes", 1000), out=out, pbt=pbt)
+    values = [m["final_avg_return"] for m in metrics]
+    best = int(np.argmax(values))
+    out("\n\n--- Hyperparameter Search Finished ---")
+    out(f"Number of finished trials: {len(values)}")
+    out("\n--- Best Trial ---")
+    out(f"  Trial Number: {best}")
+    out(f"  Value (Final Avg Return): {values[best]:.4f}")
+    out("\n  Best Hyperparameters:")
+    for k, v in runner.trials[best].items():
+        out(f"    {k}: {v}")
+    out("\n--- PBT Lineage ---")
+    for g, steps in enumerate(runner.lineage):
+        out(f"  Trial {g}: " + ("; ".join(f"step {t} <- trial {s} {vals}" for t, s, vals in steps) if steps else "initial values"))
+    return {"trials": trials, "final_trials": runner.trials, "lineage": runner.lineage, "metrics": metrics, "best_trial": best,
+            "best_value": values[best]}
